@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py - queries/sec of exhaustive multi-field top-100 on synthetic STaRK-shaped corpora.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload scale_10m_all] [--batch 512]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload scale_10m_all] [--batch 512] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
     python bench.py --impl reference ...      # the reference's CPU pipeline on the host cores
 
@@ -40,6 +40,7 @@ NOMINAL_BF16_TFLOPS = 2250.0    # dense bf16, B200 data sheet
 DIM = 768
 TOPK = 100
 GEN_CHUNK = 65536
+DUMP_BYTES = 64_000_000         # --dump-outputs: at most this much in all
 # what rides along with the headline in the default run: (workload, batches) - BASELINE.json configs 2, 3, 4 and the
 # single_ scorer of config 5
 OTHER_WORKLOADS = (("prime_full", (1, 64)), ("mag_full", (1, 512)), ("amazon_full", (64, 512)),
@@ -423,10 +424,12 @@ class Workload:
         extra = 1 + (0 if self.ctx.world == 1 else (1 if self.ctx.exchange is None else (3 if self.piped.pipelined else 2)))
         return out, self.retr.last_launches + extra       # + mixture weights (+ epoch bump + exchange kernels / merge)
 
-    def time_device(self, pool, steps, warmup, graph: bool, profile: bool, sample_clocks=False):
+    def time_device(self, pool, steps, warmup, graph: bool, profile: bool, sample_clocks=False, keep_last=False):
         """K timed steps with device-resident inputs.  Returns (ms total [max over ranks], launches, kernel ms list,
         clocks).  The scoring kernel's own duration comes from the library's CUDA-event pair around it; a graph replay
-        carries no such events, so with `graph` the kernel is timed in a separate eager pass of the same length."""
+        carries no such events, so with `graph` the kernel is timed in a separate eager pass of the same length.
+        With `keep_last`, the (scores, ids) the last timed step returned are copied to the host as `last_outputs`
+        before anything else runs (a graph replay returns static buffers that later steps overwrite)."""
         from mfar_b200 import _native as nv
         ctx = self.ctx
         for i in range(warmup):
@@ -445,11 +448,14 @@ class Workload:
             torch.cuda.profiler.start()
         e0.record()
         for i in range(steps):
-            launches += self.step(pool[i % len(pool)], graph)[1]
+            out, n = self.step(pool[i % len(pool)], graph)
+            launches += n
         e1.record()
         ctx.barrier()
         if ncu_range:
             torch.cuda.profiler.stop()
+        if keep_last:
+            self.last_outputs = tuple(t.cpu() for t in out)
         ms_local = e0.elapsed_time(e1)
         ms = ctx.max_over_ranks(ms_local)
         self.last_per_rank_ms_per_step = [x / steps for x in ctx.per_rank(ms_local)]
@@ -698,7 +704,10 @@ def run_workload(ctx: Ctx, name, batches, steps, warmup, headline=False):
             est = wl.time_device(pool, 3, 2, graph, profile=False)[0] / 3
             st = max(st, min(300, int(math.ceil(100.0 / max(est, 1e-3)))))
             wu = max(wu, min(100, int(math.ceil(40.0 / max(est, 1e-3)))))
-        ms, launches, km, clocks = wl.time_device(pool, st, wu, graph, profile=True, sample_clocks=main)
+        keep = main and a.dump_outputs is not None
+        ms, launches, km, clocks = wl.time_device(pool, st, wu, graph, profile=True, sample_clocks=main, keep_last=keep)
+        if keep:
+            out["last_outputs"] = wl.last_outputs
         k_ms = statistics.mean(km) if km else None
         rec = {"batch": Q, "value": Q * st / (ms * 1e-3), "ms_per_step": ms / st, "steps": st,
                "roofline": wl.roofline(Q, k_ms, len(km), ms, st), "gpu_launches": launches}
@@ -727,6 +736,17 @@ def run_workload(ctx: Ctx, name, batches, steps, warmup, headline=False):
             out["union_rescore"] = {"error": f"{type(e).__name__}: {e}"[:200]}
     wl.release()
     return out
+
+
+def dump_outputs(out_dir, scores, ids):
+    """`--dump-outputs`: DIR/topk_scores.npy (float32 [Q, 100]) and DIR/topk_ids.npy (float64 [Q, 100]; doc ids are
+    exact below 2**53).  Within DUMP_BYTES in all: a larger batch is cut to its first queries, a fixed sample since
+    the batch is one seeded random draw."""
+    import numpy as np
+    n = min(scores.shape[0], (DUMP_BYTES - 4096) // (scores.shape[1] * (4 + 8)))     # 4096: room for the .npy headers
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "topk_scores.npy"), scores[:n].numpy().astype(np.float32))
+    np.save(os.path.join(out_dir, "topk_ids.npy"), ids[:n].numpy().astype(np.float64))
 
 
 def main():
@@ -760,7 +780,15 @@ def main():
                          "rank of the step) or its own (complete)")
     ap.add_argument("--cpu-budget-s", type=float, default=20.0, help="0 skips the cpu_baseline leg of our arm")
     ap.add_argument("--seed", type=int, default=1234)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the headline's last timed step returned (top-k scores "
+                         "and doc ids) as DIR/<name>.npy; the inputs depend only on the arguments, so two builds run "
+                         "with the same arguments can be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None and args.impl != "ours":
+        ap.error("--dump-outputs writes the GPU arm's outputs (--impl ours)")
     args.warmup = max(args.warmup, 3)
 
     from mfar_b200 import synth
@@ -815,6 +843,8 @@ def main():
 
     extra = [int(x) for x in args.extra_batches.split(",") if x and int(x) != Q]
     head = run_workload(ctx, args.workload, [Q] + extra, args.steps, args.warmup, headline=True)
+    if rank == 0 and args.dump_outputs is not None:
+        dump_outputs(args.dump_outputs, *head["last_outputs"])
     others = []
     if args.others != "none":
         spec = OTHER_WORKLOADS if args.others == "default" else tuple(

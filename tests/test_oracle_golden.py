@@ -113,28 +113,3 @@ def test_topk_sorted_tie_break_and_matches_torch():
     tv, _ = torch.topk(s, 50, dim=1)
     np.testing.assert_array_equal(v.numpy(), tv.numpy())
     assert i[:, :3].tolist() == [[5, 10, 20]] * 4
-
-
-def test_cross_check_against_live_reference_if_present():
-    """When /root/reference exists (build container) run the reference classes live on a fresh seed."""
-    import ref_import
-    if not ref_import.available():
-        pytest.skip("reference tree not on this machine (expected on the GPU box)")
-    DenseFlatIndex, _, _, LinearWeights, _ = ref_import.load()
-    rng = np.random.RandomState(99)
-    N, d, Q, k = 500, 64, 6, 25
-    v = O.round_bf16(torch.from_numpy(rng.standard_normal((N, d)).astype(np.float32))).numpy()
-    q = O.round_bf16(torch.from_numpy(rng.standard_normal((Q, d)).astype(np.float32))).numpy()
-    keys = [str(i) for i in range(N)]
-    idx = DenseFlatIndex(None, v, keys, {k_: i for i, k_ in enumerate(keys)}, vector_batch_size=128)
-    hits = idx.retrieve_batch(q, top_k=k)
-    s, r = O.dense_retrieve_batch(torch.from_numpy(q), torch.from_numpy(v), k, 128)
-    np.testing.assert_allclose(s.numpy(), np.array([[h[1] for h in hit] for hit in hits], np.float32), rtol=1e-6)
-    assert r.tolist() == [[int(h[0]) for h in hit] for hit in hits]
-    layer = LinearWeights(d, 3, query_cond=True)
-    W = torch.from_numpy((0.05 * rng.standard_normal((d, 3))).astype(np.float32))
-    with torch.no_grad():
-        layer.weight.copy_(W)
-        x = torch.from_numpy(rng.standard_normal((Q, 40, 3)).astype(np.float32))
-        ref = layer(x, torch.from_numpy(q))
-    np.testing.assert_allclose(O.linear_weights_forward(x, torch.from_numpy(q), W, True).numpy(), ref.numpy(), rtol=1e-6)
