@@ -300,7 +300,7 @@ class DeviceBM25:
         # score once, then peel the ranking off in passes of <= 128 - each pass is the same streaming top-k kernel over
         # the score rows, the docs already taken are sunk to -inf in between.  Passes come out in rank order.
         Q, n = len(query_tokens), self.num_docs
-        ld = (n + 63) // 64 * 64
+        ld = (n + 64) // 64 * 64                        # >= 1 padding column past the docs (see the scatter below)
         rows = torch.full((Q, 1, ld), float("-inf"), dtype=torch.float32, device=self.device)
         rows[:, 0, :n] = self.get_scores_batch(query_tokens)
         r = MultiFieldRetriever(None, LinearWeights(1, 1).to(self.device), n_sparse=1, top_k=nv.MAX_K, n_docs=n,
@@ -312,7 +312,8 @@ class DeviceBM25:
             launches += r.last_launches
             out_s.append(s)
             out_i.append(i)
-            rows[:, 0, :].scatter_(1, i, float("-inf"))
+            # an empty slot (id -1) must not index the row: it lands in the last padding column, outside the docs
+            rows[:, 0, :].scatter_(1, i.remainder(ld), float("-inf"))
             left -= kk
         self.last_launches = launches
         return torch.cat(out_i, dim=1).cpu().numpy(), torch.cat(out_s, dim=1).cpu().numpy()
