@@ -9,9 +9,11 @@ namespace mfar {
 
 // ---------------------------------------------------------------------------------------
 // pack: one warp per source row.  row-major [n_rows, dim] fp32|bf16 -> packed bf16
-// [tile][field][128][dim].  Optional L2 normalisation == torch.nn.functional.normalize
-// (x / max(||x||_2, 1e-12)), what sentence-transformers' Normalize() applies
-// (reference: mfar/modeling/util.py:50-51).
+// [tile][field][128][dim].  Optional L2 normalisation x / max(||x||_2, 1e-12), what
+// sentence-transformers' Normalize() applies (reference: mfar/modeling/util.py:50-51), computed
+// in fp64 and rounded ONCE to bf16: the squares of fp32 values are exact in fp64, the sum cannot
+// overflow (a row of |x| ~ 1e19 packs as itself over its norm, not as zeros), and the quotient
+// goes straight to nearest-even bf16.  Queries go through the same kernel (prepare_queries).
 // ---------------------------------------------------------------------------------------
 template <typename SrcT>
 __global__ void pack_rows_kernel(const SrcT* __restrict__ src, int64_t n_rows, int64_t row_begin,
@@ -21,22 +23,23 @@ __global__ void pack_rows_kernel(const SrcT* __restrict__ src, int64_t n_rows, i
   const int64_t r = (int64_t(blockIdx.x) * blockDim.x + threadIdx.x) >> 5;
   if (r >= n_rows) return;
   const SrcT* s = src + r * dim;
-  float scale = 1.0f;
-  if (normalize) {
-    float ss = 0.f;
-    for (int i = lane; i < dim; i += 32) {
-      float v = float(s[i]);
-      ss += v * v;
-    }
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) ss += __shfl_xor_sync(0xffffffffu, ss, o);
-    scale = 1.0f / fmaxf(sqrtf(ss), 1e-12f);
-  }
   const int64_t doc = row_begin + r;
   const int64_t tile = doc / kTileDocs;
   const int in_tile = int(doc % kTileDocs);
   __nv_bfloat16* d = packed + ((tile * n_fields + field) * kTileDocs + in_tile) * int64_t(dim);
-  for (int i = lane; i < dim; i += 32) d[i] = __float2bfloat16_rn(float(s[i]) * scale);
+  if (!normalize) {
+    for (int i = lane; i < dim; i += 32) d[i] = __float2bfloat16_rn(float(s[i]));
+    return;
+  }
+  double ss = 0.0;
+  for (int i = lane; i < dim; i += 32) {
+    const double v = double(float(s[i]));
+    ss = fma(v, v, ss);
+  }
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) ss += __shfl_xor_sync(0xffffffffu, ss, o);
+  const double norm = fmax(sqrt(ss), double(1e-12f));   // F.normalize's eps on an fp32 tensor
+  for (int i = lane; i < dim; i += 32) d[i] = __double2bfloat16(double(float(s[i])) / norm);
 }
 
 __global__ void unpack_rows_kernel(const __nv_bfloat16* __restrict__ packed, int n_fields, int field, int dim,

@@ -112,14 +112,28 @@ class PackedCorpus:
         return out[:, : self.dim]
 
     def prepare_queries(self, q_vecs) -> torch.Tensor:
-        """[Q, dim] (any float dtype, host or device) -> contiguous bf16 [Q, dim_pad] on the device."""
+        """[Q, dim] (any float dtype, host or device) -> contiguous bf16 [Q, dim_pad] on the device.
+
+        On a cosine corpus the queries are normalised by the kernel that packs the docs, so both sides are rounded to
+        bf16 once, by the same arithmetic: with one field the packed layout [tile][1][128][dim_pad] of Q rows is plain
+        row-major [Q, dim_pad].  Inputs other than fp32 / bf16 are taken to fp32 first, as in ``load_rows``."""
         if not torch.is_tensor(q_vecs):
             q_vecs = torch.from_numpy(np.ascontiguousarray(q_vecs))
         if q_vecs.dim() != 2 or q_vecs.shape[1] != self.dim:
             raise ValueError(f"expected [Q,{self.dim}] query vectors, got {tuple(q_vecs.shape)}")
         q = q_vecs.to(self.device)
         if self.normalize:
-            q = torch.nn.functional.normalize(q.float(), p=2, dim=1)
+            if q.dtype not in (torch.float32, torch.bfloat16):
+                q = q.float()
+            if self.dim_pad != self.dim:
+                q = torch.nn.functional.pad(q, (0, self.dim_pad - self.dim))
+            q = q.contiguous()
+            out = torch.empty((q.shape[0], self.dim_pad), dtype=torch.bfloat16, device=self.device)
+            if q.shape[0]:
+                nv.check(nv.lib().mfar_corpus_pack_rows(nv.ptr(q), nv.F32 if q.dtype == torch.float32 else nv.BF16,
+                                                        q.shape[0], 0, nv.ptr(out), q.shape[0], 1, 0, self.dim_pad, 1,
+                                                        nv.stream()), "corpus_pack_rows (queries)")
+            return out
         q = q.to(torch.bfloat16)
         if self.dim_pad != self.dim:
             q = torch.nn.functional.pad(q, (0, self.dim_pad - self.dim))
@@ -175,6 +189,21 @@ class MultiFieldRetriever:
         self.mask = mask
         if field_names is not None:
             self.masked_fields_string = ",".join(field_names[i] for i in field_idx_list)
+
+    def mixture_input(self, q_vecs, q_emb=None) -> Optional[torch.Tensor]:
+        """The fp32 [Q,E] device input of a query-conditioned mixture (None for static weights).  ``q_emb`` defaults to
+        the query vectors, as in the reference where both come from the same encoder (contrastive.py:688-694); on a
+        cosine corpus that encoder ends in ``Normalize()``, so its output ``x_encoded`` - and the default here - is the
+        unit-normalised query."""
+        if not self.mixture.query_cond:
+            return None
+        if q_emb is not None:
+            return q_emb.to(self.device).float()
+        qv = q_vecs if torch.is_tensor(q_vecs) else torch.from_numpy(np.ascontiguousarray(q_vecs))
+        qe = qv.to(self.device).float()
+        if self.corpus is not None and self.corpus.normalize:
+            qe = torch.nn.functional.normalize(qe, p=2, dim=1)
+        return qe
 
     # ------------------------------------------------------------------ internals
     def _workspace(self, Q: int, k: int, n_sparse: int, n_docs: Optional[int] = None,
@@ -286,8 +315,9 @@ class MultiFieldRetriever:
         """Exhaustive multi-field top-k.
 
         q_vecs [Q,dim]: query vectors for the dense dots (rounded to bf16);
-        q_emb  [Q,E]  : fp32 query embedding for the mixture softmax (defaults to q_vecs, as in the
-                        reference where both come from the same encoder, contrastive.py:688-694);
+        q_emb  [Q,E]  : fp32 query embedding for the mixture softmax (defaults to q_vecs - unit-normalised on a
+                        cosine corpus - as in the reference where both come from the same encoder,
+                        contrastive.py:688-694; ``mixture_input``);
         sparse [Q,Fs,ld>=N]: precomputed per-field BM25 scores of this shard's docs (f16/f32).  With a 32-byte aligned row
                         pitch (``ld`` a multiple of 16 for f16, 8 for f32) the rows are gathered and mixed INSIDE the
                         scoring epilogue; otherwise a pre-mix kernel writes a [Q,N] fp32 block first.
@@ -307,11 +337,7 @@ class MultiFieldRetriever:
                 sparse_tokens is None or torch.is_tensor(sparse_tokens)):
             batch = int(q_emb.shape[0])
         Q = self._batch_size(q_bf16, sparse, sparse_tokens, batch)
-        if self.mixture.query_cond:
-            qe = q_emb if q_emb is not None else (q_vecs if torch.is_tensor(q_vecs) else torch.from_numpy(q_vecs))
-            qe = qe.to(self.device).float()
-        else:
-            qe = None
+        qe = self.mixture_input(q_vecs, q_emb)
         w = self.mixture.field_weights(qe, self.mask, batch=Q)
         if sparse_tokens is not None:
             ent = self._bm25_entries(sparse_tokens)
@@ -372,11 +398,7 @@ class MultiFieldRetriever:
         q_bf16 = self.corpus.prepare_queries(q_vecs) if self.corpus is not None else None
         ent = self._bm25_entries(sparse_tokens) if sparse_tokens is not None else None
         Q = self._batch_size(q_bf16, sparse, sparse_tokens, batch)
-        if self.mixture.query_cond:
-            qe = q_emb if q_emb is not None else (q_vecs if torch.is_tensor(q_vecs) else torch.from_numpy(q_vecs))
-            qe = qe.to(self.device).float()
-        else:
-            qe = None
+        qe = self.mixture_input(q_vecs, q_emb)
         w = self.mixture.field_weights(qe, None, batch=Q)                      # [Q,F] unmasked softmax weights
         M = len(masked_sets)
         masks = torch.ones((M, self.num_fields), dtype=torch.float32, device=self.device)
@@ -563,11 +585,7 @@ class MultiFieldRetriever:
             sparse = self._sparse_from_tokens(None, sparse_tokens, q_bf16, batch)
         _, rows = self.per_field_topk(q_vecs, sparse, k, batch=batch)      # [F,Q,k] local rows, (0.0, row 0) quirk applied
         Q = rows.shape[1]
-        if self.mixture.query_cond:
-            qv = q_vecs if torch.is_tensor(q_vecs) else torch.from_numpy(q_vecs)
-            qe = (q_emb if q_emb is not None else qv).to(self.device).float()
-        else:
-            qe = None
+        qe = self.mixture_input(q_vecs, q_emb)
         w = self.mixture.field_weights(qe, self.mask, batch=Q)             # softmax(q@W) * mask, [Q,F]
         sp, code = self._check_sparse(sparse, Q)
         vals = torch.empty((Q, k), dtype=torch.float32, device=self.device)
@@ -638,7 +656,11 @@ class GraphedSearch:
         self.Q = int(batch)
         self.sparse_kind = sparse
         dim = r.corpus.dim if r.corpus is not None else 1
-        self.q_vecs = torch.zeros((self.Q, dim), dtype=torch.bfloat16, device=dev) if r.corpus is not None else None
+        # a cosine corpus normalises the query it is given: the static buffer keeps fp32 queries unrounded, so the graph
+        # rounds them to bf16 once, after the normalisation, as the eager search does (without normalisation the one
+        # rounding is the copy into a bf16 buffer)
+        q_dtype = torch.float32 if r.corpus is not None and r.corpus.normalize else torch.bfloat16
+        self.q_vecs = torch.zeros((self.Q, dim), dtype=q_dtype, device=dev) if r.corpus is not None else None
         E = r.mixture.weight.shape[0] if r.mixture.query_cond else 0
         self.q_emb = torch.zeros((self.Q, E), dtype=torch.float32, device=dev) if E else None
         self.sparse = self.entries = None
@@ -679,7 +701,7 @@ class GraphedSearch:
         if self.q_vecs is not None:
             self.q_vecs.copy_(q_vecs, non_blocking=True)
         if self.q_emb is not None:
-            self.q_emb.copy_(q_emb if q_emb is not None else q_vecs, non_blocking=True)
+            self.q_emb.copy_(q_emb if q_emb is not None else self.r.mixture_input(q_vecs), non_blocking=True)
         if self.sparse is not None and sparse is not None and sparse.data_ptr() != self.sparse.data_ptr():
             self.sparse[:, :, : sparse.shape[2]].copy_(sparse, non_blocking=True)
         if self.entries is not None:

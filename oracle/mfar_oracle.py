@@ -108,7 +108,8 @@ def sparse_score_batch(score_vecs: torch.Tensor, rows: Sequence[int]) -> torch.T
 # --------------------------------------------------------------------------------------
 def exhaustive_scores(q_vecs: torch.Tensor, dense_fields: Sequence[torch.Tensor],
                       sparse_scores: Optional[torch.Tensor], weights: torch.Tensor,
-                      mask: Optional[torch.Tensor] = None, doc_chunk: int = 65536) -> torch.Tensor:
+                      mask: Optional[torch.Tensor] = None, doc_chunk: int = 65536,
+                      normalize: bool = False) -> torch.Tensor:
     """Mixture score of every doc: ``sum_f w[q,f] * mask[f] * s_f[q,n]`` with
     s_f = q . v_f for dense fields (index.py:197 / 231) followed by the sparse fields'
     precomputed scores (index.py:114-117), field order dense-then-sparse (schema.py:130-134),
@@ -116,7 +117,12 @@ def exhaustive_scores(q_vecs: torch.Tensor, dense_fields: Sequence[torch.Tensor]
     (contrastive.py:686 then weighting.py:28-29).
 
     q_vecs [Q,d]; dense_fields: F_d tensors [N,d]; sparse_scores [Q,F_s,N] or None;
-    weights [Q,F] or [1,F] (already softmaxed).  Returns [Q, N] fp32."""
+    weights [Q,F] or [1,F] (already softmaxed).  With ``normalize`` (cosine: the encoder ends in
+    ``Normalize()``, modeling/util.py:50-51) queries and doc rows first go through
+    ``normalize_rows_bf16``.  Returns [Q, N] fp32."""
+    if normalize:
+        q_vecs = torch.from_numpy(normalize_rows_bf16(q_vecs))
+        dense_fields = [torch.from_numpy(normalize_rows_bf16(f)) for f in dense_fields]
     Q = q_vecs.shape[0]
     Fd = len(dense_fields)
     Fs = 0 if sparse_scores is None else sparse_scores.shape[1]
@@ -222,3 +228,36 @@ def union_rescore(q_vecs: torch.Tensor, dense_fields: Sequence[torch.Tensor],
 # --------------------------------------------------------------------------------------
 def round_bf16(x: torch.Tensor) -> torch.Tensor:
     return x.to(torch.bfloat16).to(torch.float32)
+
+
+# --------------------------------------------------------------------------------------
+# Cosine: L2 normalisation rounded once to bf16                modeling/util.py:50-51
+# --------------------------------------------------------------------------------------
+NORM_EPS = float(np.float32(1e-12))     # F.normalize's eps as it acts on an fp32 tensor
+BF16_MIN_EXP = -133                     # exponent of the bf16 subnormal spacing
+
+
+def round_bf16_rne(y) -> np.ndarray:
+    """float64 -> the nearest bf16 value (ties to even), as float64: ONE rounding, including bf16 subnormals
+    (spacing 2^-133) and overflow to +-inf.  Signs of zeros are kept.  (torch's float64 -> bf16 cast may round twice
+    through fp32, so it is not used here.)"""
+    y = np.asarray(y, dtype=np.float64)
+    _, e = np.frexp(y)                                  # |y| = m 2^e, 0.5 <= m < 1: 8 significant bits -> 2^(e-8)
+    q = np.maximum(e - 8, BF16_MIN_EXP)
+    with np.errstate(over="ignore"):
+        r = np.ldexp(np.rint(np.ldexp(y, -q)), q)       # the scaling is exact; rint rounds half to even
+    big = np.abs(r) >= 2.0 ** 128                       # past the largest bf16 (1 - 2^-8) 2^128
+    return np.where(big, np.copysign(np.inf, y), r)
+
+
+def normalize_rows_bf16(x) -> np.ndarray:
+    """The cosine contract of ``PackedCorpus(normalize=True)`` for docs and queries alike: every row, taken exactly into
+    float64, is divided by ``max(||x||_2, float32(1e-12))`` in float64 and rounded ONCE to nearest-even bf16.  An
+    all-zero row stays zero and keeps the signs of its zeros.  x: [n, d] fp32 / bf16 / f16 (tensor or array).
+    Returns float32 [n, d] holding bf16 values exactly."""
+    if torch.is_tensor(x):
+        x = x.detach().cpu().double().numpy()
+    x = np.asarray(x, dtype=np.float64)
+    norm = np.sqrt(np.sum(x * x, axis=1, keepdims=True))   # squares of fp32 values are exact in float64
+    y = x / np.maximum(norm, NORM_EPS)
+    return round_bf16_rne(y).astype(np.float32)

@@ -73,9 +73,9 @@ def run_case(c: dict) -> None:
     mu = torch.randn(d, generator=g)
     raw = [torch.randn(N, d, generator=g) + 0.5 * mu for _ in range(Fd)]
     qraw = torch.randn(Q, d, generator=g) + 0.5 * mu
-    if c["normalize"]:                              # oracle side of Normalize(): fp32 normalise, then bf16 rounding
-        fields = [O.round_bf16(torch.nn.functional.normalize(f, dim=1)) for f in raw]
-        q = O.round_bf16(torch.nn.functional.normalize(qraw, dim=1))
+    if c["normalize"]:                              # oracle side of Normalize(): float64 normalise, one bf16 rounding
+        fields = [torch.from_numpy(O.normalize_rows_bf16(f)) for f in raw]
+        q = torch.from_numpy(O.normalize_rows_bf16(qraw))
     else:
         fields = [O.round_bf16(f) for f in raw]
         q = O.round_bf16(qraw)
@@ -104,9 +104,8 @@ def run_case(c: dict) -> None:
     torch.cuda.synchronize()
     w = O.mixture_weights(q_emb.float().cpu() if qc else None, W, qc)
     ref = O.exhaustive_scores(q, fields, None if sp is None else sp.float(), w, mask)
-    rtol = 2e-5 if not c["normalize"] else 2e-3     # device-side normalisation rounds to bf16 from a device rsqrt
-    assert_topk_parity(scores.cpu().numpy(), ids.cpu().numpy(), ref.numpy(), k, id_offset=c["base"], rtol=rtol,
-                       tie_rel=1e-5 if not c["normalize"] else 2e-3, scale_floor=_term_scale(c))
+    assert_topk_parity(scores.cpu().numpy(), ids.cpu().numpy(), ref.numpy(), k, id_offset=c["base"], rtol=2e-5,
+                       tie_rel=1e-5, scale_floor=_term_scale(c))
 
 
 def draw_api_case(rng: np.random.RandomState) -> dict:
