@@ -8,7 +8,8 @@ When ``query_cond`` is False the reference constructs it as ``LinearWeights(num_
 
 ``forward`` runs the CUDA kernels behind ``mfar_mixture_weights`` / ``mfar_mixture_apply`` (fp32).  When autograd
 is recording and any of x / q / weight requires grad, it goes through ``MixtureFunction`` whose backward is
-``mfar_mixture_bwd`` (dx, dW, dq) - the training-time use inside the contrastive losses (losses.py:197-202).
+``mfar_mixture_bwd`` (dx, dW, dq) - the training-time use inside the contrastive losses (losses.py:197-202); an [S,F]
+x is expanded to [B,S,F] first, so it stays differentiable as in the reference.
 """
 from __future__ import annotations
 
@@ -102,16 +103,18 @@ class LinearWeights(torch.nn.Module):
 
     def forward(self, x: torch.Tensor, q: Optional[torch.Tensor]) -> torch.Tensor:
         nv.require_device(x, "x")
-        if torch.is_grad_enabled() and x.dim() == 3 and (
+        if torch.is_grad_enabled() and x.dim() in (2, 3) and (
                 x.requires_grad or self.weight.requires_grad or (q is not None and q.requires_grad)):
             nv.require_device(self.weight, "LinearWeights.weight")
-            if x.shape[2] != self.num_fields:
-                raise RuntimeError(f"x has {x.shape[2]} fields, layer has {self.num_fields}")
-            if self.query_cond:
-                if q is None:
-                    raise ValueError("query_cond=True needs the query embedding")
-                if q.shape[0] != x.shape[0]:
-                    raise RuntimeError("batch size of x and q must match (weighting.py:21-23)")
+            if x.shape[-1] != self.num_fields:
+                raise RuntimeError(f"x has {x.shape[-1]} fields, layer has {self.num_fields}")
+            if self.query_cond and q is None:
+                raise ValueError("query_cond=True needs the query embedding")
+            if x.dim() == 2:                         # [S,F] against every query (weighting.py:29); expand's backward
+                B = q.shape[0] if self.query_cond else 1     # sums dx over the queries
+                x = x.unsqueeze(0).expand(B, *x.shape)
+            if self.query_cond and q.shape[0] != x.shape[0]:
+                raise RuntimeError("batch size of x and q must match (weighting.py:21-23)")
             return MixtureFunction.apply(x, q if self.query_cond else None, self.weight, self.query_cond)
         with torch.no_grad():
             return self._forward_nograd(x, q)
