@@ -552,10 +552,11 @@ __global__ void seed_from_keys_kernel(const uint64_t* keys, int Q, int k, unsign
   }
 }
 
-// index.py:192-193 quirk: running top-k starts as (0.0, row 0) entries.
+// index.py:192-193 quirk: running top-k starts as (0.0, row 0) entries.  They replace the negative scores only: a NaN
+// entry outranks them under torch.topk's order (NaN largest) and stays.
 __global__ void zero_init_kernel(float* scores, int64_t* ids, int n) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i < n && !(scores[i] >= 0.0f)) { scores[i] = 0.0f; ids[i] = 0; }
+  if (i < n && scores[i] < 0.0f) { scores[i] = 0.0f; ids[i] = 0; }
 }
 
 // ---------------------------------------------------------------------------------------

@@ -49,15 +49,22 @@ struct PerDeviceOnce {
 //   high 32 bits: float score mapped so that unsigned order == float order
 //   low  32 bits: ~doc_id, so that among equal scores the LOWER doc id is the LARGER key
 // max-key-first order therefore is (score desc, doc id asc): the deterministic tie-break the
-// oracle's topk_sorted() uses.  Key 0 is never produced by a finite score: it marks "empty".
+// oracle's topk_sorted() uses.  Every NaN, whatever its sign or payload, maps to ONE word above +inf's
+// (kNanOrdered, the word of the canonical +NaN 0x7FC00000), so the full order is
+//   NaN > +inf > finite scores (desc) > -inf, then doc id asc inside each class
+// - torch.topk's order (NaN counts as the largest value), which the reference ranks with (contrastive.py:696).
+// A NaN doc reports the canonical NaN.  (-0.0 would rank just below +0.0, but every score is a sum started at +0.0,
+// which never yields -0.0.)  Key 0 is never produced by any score: it marks "empty".
 // ---------------------------------------------------------------------------------------
+constexpr uint32_t kNanOrdered = 0xFFC00000u;
 __host__ __device__ __forceinline__ uint32_t float_to_ordered(float f) {
 #ifdef __CUDA_ARCH__
   uint32_t u = __float_as_uint(f);
 #else
   union { float f; uint32_t u; } c; c.f = f; uint32_t u = c.u;
 #endif
-  return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
+  const uint32_t o = (u & 0x80000000u) ? ~u : (u | 0x80000000u);
+  return f != f ? kNanOrdered : o;
 }
 __host__ __device__ __forceinline__ float ordered_to_float(uint32_t o) {
   uint32_t u = (o & 0x80000000u) ? (o & 0x7FFFFFFFu) : ~o;
@@ -72,6 +79,15 @@ __host__ __device__ __forceinline__ uint64_t make_key(float score, uint32_t doc_
 }
 __host__ __device__ __forceinline__ float key_score(uint64_t key) { return ordered_to_float(uint32_t(key >> 32)); }
 __host__ __device__ __forceinline__ uint32_t key_doc(uint64_t key) { return ~uint32_t(key & 0xFFFFFFFFull); }
+
+// max that PROPAGATES NaN (fmaxf drops it).  The float pre-filters of the scoring kernels take a group maximum and
+// test it with !(m < thr): a NaN anywhere in the group (a NaN score, or -inf - -inf, +inf - +inf in score_tc's
+// differences) then passes to the exact key compare instead of being rejected - the filters stay conservative.
+__device__ __forceinline__ float fmax_nan(float a, float b) {
+  float d;
+  asm("max.NaN.f32 %0, %1, %2;" : "=f"(d) : "f"(a), "f"(b));
+  return d;
+}
 
 // Workspace carve-up shared by the scoring kernels and the merge.
 //   cand_keys [G][Qp][kCandCap] u64 | cand_thr [G][Qp] u64 | cand_cnt [G][Qp] i32 | err flag (256 B) |

@@ -541,12 +541,13 @@ score_qs_kernel(const __grid_constant__ CUtensorMap map_b, const __grid_constant
           // more than the 8 group branches it saves - single_ Q=512 8.2 ms vs 7.5 ms.)
 #pragma unroll
           for (int c0 = 0; c0 < kQsDocs; c0 += 8) {
-            const float m = fmaxf(fmaxf(fmaxf(acc[c0], acc[c0 + 1]), fmaxf(acc[c0 + 2], acc[c0 + 3])),
-                                  fmaxf(fmaxf(acc[c0 + 4], acc[c0 + 5]), fmaxf(acc[c0 + 6], acc[c0 + 7])));
-            if (m >= thr_f) {
+            // NaN-propagating max and !(x < thr_f): a NaN score (or a NaN threshold) reaches the key compare
+            const float m = fmax_nan(fmax_nan(fmax_nan(acc[c0], acc[c0 + 1]), fmax_nan(acc[c0 + 2], acc[c0 + 3])),
+                                     fmax_nan(fmax_nan(acc[c0 + 4], acc[c0 + 5]), fmax_nan(acc[c0 + 6], acc[c0 + 7])));
+            if (!(m < thr_f)) {
 #pragma unroll
               for (int c = c0; c < c0 + 8; ++c) {
-                if (c < nd && acc[c] >= thr_f) {
+                if (c < nd && !(acc[c] < thr_f)) {
                   const uint64_t key = make_key(acc[c], id0 + c);
                   if (key > thr) { __stcg(my_list + cnt, key); ++cnt; }
                 }

@@ -349,9 +349,11 @@ score_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant
         for (int c0 = 0; c0 < QP; c0 += 8) {
           const float4 ta = *reinterpret_cast<const float4*>(s_thrf + c0);
           const float4 tb = *reinterpret_cast<const float4*>(s_thrf + c0 + 4);
-          const float m = fmaxf(fmaxf(fmaxf(acc[c0] - ta.x, acc[c0 + 1] - ta.y), fmaxf(acc[c0 + 2] - ta.z, acc[c0 + 3] - ta.w)),
-                                fmaxf(fmaxf(acc[c0 + 4] - tb.x, acc[c0 + 5] - tb.y), fmaxf(acc[c0 + 6] - tb.z, acc[c0 + 7] - tb.w)));
-          if (m >= 0.f) {
+          // NaN-propagating max and !(m < 0): a NaN score, or inf - inf of a score and threshold in the same infinite
+          // class, reaches the key compare (fmaxf would drop it, and the answer would depend on the group's mates)
+          const float m = fmax_nan(fmax_nan(fmax_nan(acc[c0] - ta.x, acc[c0 + 1] - ta.y), fmax_nan(acc[c0 + 2] - ta.z, acc[c0 + 3] - ta.w)),
+                                   fmax_nan(fmax_nan(acc[c0 + 4] - tb.x, acc[c0 + 5] - tb.y), fmax_nan(acc[c0 + 6] - tb.z, acc[c0 + 7] - tb.w)));
+          if (!(m < 0.f)) {
 #pragma unroll
             for (int j = 0; j < 8; ++j) {
               const int c = c0 + j;

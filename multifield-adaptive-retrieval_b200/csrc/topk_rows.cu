@@ -110,14 +110,15 @@ topk_rows_kernel(const float* __restrict__ base, long long base_ld, long long n_
 #pragma unroll
     for (int j = 0; j < 4; ++j) {
       // one compare per lane (max of its 4 docs) and one ballot reject the 128 docs of this sub-step in the common case
-      const float m = fmaxf(fmaxf(cur[j].x, cur[j].y), fmaxf(cur[j].z, cur[j].w));
-      if (__ballot_sync(0xffffffffu, m >= thr_f) == 0u) continue;
+      // NaN-propagating max and !(x < thr_f): NaN scores (NaN > +inf in the key order) reach the key compare
+      const float m = fmax_nan(fmax_nan(cur[j].x, cur[j].y), fmax_nan(cur[j].z, cur[j].w));
+      if (__ballot_sync(0xffffffffu, !(m < thr_f)) == 0u) continue;
       const long long d = s0 + j * 128 + lane * 4;
       const float x[4] = {cur[j].x, cur[j].y, cur[j].z, cur[j].w};
 #pragma unroll
       for (int e = 0; e < 4; ++e) {
         const unsigned long long key = make_key(x[e], uint32_t(doc_id_base + d + e));
-        const bool pass = (d + e < d1) && x[e] >= thr_f && key > thr;
+        const bool pass = (d + e < d1) && !(x[e] < thr_f) && key > thr;
         const unsigned b = __ballot_sync(0xffffffffu, pass);
         if (b) {
           if (pass) __stcg(list + cnt + __popc(b & lt_mask), key);

@@ -75,10 +75,15 @@ def rebalanced_boundaries(cuts: Sequence[int], step_ms: Sequence[float], base_cu
 
 
 # ---- host-side mirror of the device key packing (csrc/common.cuh) - used by tests and debugging
+NAN_ORDERED = 0xFFC00000          # the one score word of every NaN (sign and payload ignored): above +inf's 0xFF800000
+
+
 def encode_keys(scores: np.ndarray, ids: np.ndarray) -> np.ndarray:
-    u = np.ascontiguousarray(scores, dtype=np.float32).view(np.uint32).astype(np.uint64)
+    f = np.ascontiguousarray(scores, dtype=np.float32)
+    u = f.view(np.uint32).astype(np.uint64)
     neg = (u & np.uint64(0x80000000)) != 0
     o = np.where(neg, (~u) & np.uint64(0xFFFFFFFF), u | np.uint64(0x80000000))
+    o = np.where(np.isnan(f), np.uint64(NAN_ORDERED), o)
     low = (~np.asarray(ids).astype(np.uint64)) & np.uint64(0xFFFFFFFF)
     return (o << np.uint64(32)) | low
 

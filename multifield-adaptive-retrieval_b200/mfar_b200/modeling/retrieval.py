@@ -329,7 +329,8 @@ class MultiFieldRetriever:
                         field j, or the prebuilt int32 [n,3] entry tensor of ``BM25FieldSet.entries`` - the sparse
                         fields are then scored on the device (bm25s ``get_scores``, index.py:72-76).
         batch          : number of queries, needed only for a sparse-only retriever fed with an entry tensor.
-        Returns (scores [Q,k] fp32, ids [Q,k] int64) sorted by (score desc, id asc); with
+        Returns (scores [Q,k] fp32, ids [Q,k] int64) sorted by (score desc, id asc), NaN scores first (as
+        ``torch.topk`` ranks them), then +inf, finite, -inf; with
         return_keys also the packed uint64 keys (as int64) used for cross-shard merging."""
         k = top_k or self.top_k
         q_bf16 = self.corpus.prepare_queries(q_vecs) if self.corpus is not None else None

@@ -143,24 +143,42 @@ def exhaustive_scores(q_vecs: torch.Tensor, dense_fields: Sequence[torch.Tensor]
     return out
 
 
+NAN_ORDERED = 0xFFC00000          # csrc/common.cuh kNanOrdered: the one score word of every NaN, above +inf's
+
+
+def ordered_words(scores: np.ndarray) -> np.ndarray:
+    """uint64 score words of the device key (csrc/common.cuh ``float_to_ordered``): unsigned order == the rank order
+    NaN (any sign or payload) > +inf > finite (desc) > -inf.  -0.0 is folded into +0.0 first (one zero, as in
+    ``torch.topk``; the kernels' sums never produce -0.0)."""
+    with np.errstate(invalid="ignore"):
+        f = np.asarray(scores, dtype=np.float32) + np.float32(0.0)
+    u = f.view(np.uint32).astype(np.uint64)
+    o = np.where((u & np.uint64(0x80000000)) != 0, (~u) & np.uint64(0xFFFFFFFF), u | np.uint64(0x80000000))
+    return np.where(np.isnan(f), np.uint64(NAN_ORDERED), o)
+
+
+def rank_rows(scores: np.ndarray, k: int) -> np.ndarray:
+    """Rows of the top k of one fp32 score row under the kernels' rule: NaN (every NaN one value) > +inf > finite
+    scores descending > -inf, the lower row first inside a class - ``torch.topk``'s order (NaN counts as the largest
+    value) with the tie order made explicit.  Ranks the composite uint64 (score word, ~row) key, the device's own."""
+    N = int(np.asarray(scores).shape[0])
+    k = min(k, N)
+    assert N < (1 << 32)
+    key = (ordered_words(scores) << np.uint64(32)) | (~np.arange(N, dtype=np.uint64) & np.uint64(0xFFFFFFFF))
+    part = np.argpartition(key, N - k)[N - k:] if k < N else np.arange(N)
+    return part[np.argsort(key[part])[::-1]]
+
+
 def topk_sorted(scores: torch.Tensor, k: int) -> Tuple[torch.Tensor, torch.Tensor]:
-    """``torch.topk(k)`` (contrastive.py:696) with the tie order made explicit: score
-    descending, then row ascending (torch leaves tie order unspecified)."""
+    """``torch.topk(k)`` (contrastive.py:696) with the tie order made explicit: NaN > +inf > finite scores
+    descending > -inf, then row ascending (``rank_rows``; torch leaves tie order unspecified)."""
     s = scores.float().numpy()
     Q, N = s.shape
     k = min(k, N)
     out_s = np.empty((Q, k), dtype=np.float32)
     out_i = np.empty((Q, k), dtype=np.int64)
-    rows = np.arange(N)
     for qi in range(Q):
-        if N > 4 * k:
-            part = np.argpartition(-s[qi], k - 1)[:k]
-            kth = s[qi][part].min()
-            cand = np.nonzero(s[qi] >= kth)[0]          # keep every tie at the boundary
-        else:
-            cand = rows
-        order = np.lexsort((cand, -s[qi][cand]))[:k]
-        sel = cand[order]
+        sel = rank_rows(s[qi], k)
         out_i[qi] = sel
         out_s[qi] = s[qi][sel]
     return torch.from_numpy(out_s), torch.from_numpy(out_i)
