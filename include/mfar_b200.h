@@ -49,7 +49,7 @@ typedef enum mfar_status {
   MFAR_ERR_K_RANGE = 6     /* k > number of docs (reference: torch.topk raises)      */
 } mfar_status;
 
-typedef enum mfar_dtype { MFAR_F32 = 0, MFAR_BF16 = 1, MFAR_F16 = 2 } mfar_dtype;
+typedef enum mfar_dtype { MFAR_F32 = 0, MFAR_BF16 = 1, MFAR_F16 = 2, MFAR_E4M3 = 3 } mfar_dtype;
 
 /* which scoring kernel mfar_score_topk runs */
 typedef enum mfar_impl {
@@ -87,6 +87,29 @@ MFAR_API int mfar_corpus_pack_rows(const void* src, int src_dtype, int64_t n_row
 /* Inverse view for tests / candidate export: copy rows of one field out as fp32 [n_rows, dim]. */
 MFAR_API int mfar_corpus_unpack_rows(const void* packed, int64_t n_docs, int n_fields, int field, int dim,
                             int64_t row_begin, int64_t n_rows, float* dst, void* stream);
+
+/* ------------------------------------------------------------------------------------------
+ * FP8 (E4M3) corpus: half the bytes of the bf16 store, scored at the tensor cores' FP8 rate.
+ *   payload  uint8 [n_tiles][n_fields][MFAR_TILE_DOCS][dim]   one E4M3 byte per element
+ *   scales   fp32  [n_tiles][n_fields][MFAR_TILE_DOCS]        one power of two per (doc, field) row
+ * The scoring kernels need dim % 128 == 0 (one 128-byte swizzle span per K-chunk).  Tail rows of the last tile hold
+ * payload 0 and scale 1: zero the payload and fill the scales with 1.0f before the first pack.
+ *
+ * A row x (fp32 or bf16; with normalize, first x / max(||x||_2, float32(1e-12)) in float64, as mfar_corpus_pack_rows)
+ * is stored as s = 2^e with e = clamp(ceil(log2(amax / 448)), -117, 119), amax = max|x_i|, and p_i = the E4M3 value
+ * nearest to x_i / s (ties to even, ONE rounding from float64, saturating to +-448).  p_i * s is then exactly a normal
+ * fp32 / bf16 number: scoring the E4M3 corpus equals scoring its dequantized bf16 copy up to fp32 summation order.
+ * A row of zeros stores s = 1 and payload 0; a row holding a NaN or an infinity stores s = NaN and payload 0 (its
+ * dequantized row, and every score of its doc, is NaN).  Queries are quantized by the same call as a one-field corpus
+ * of Q docs: [Q][dim] payload rows and [Q] scales.
+ * ------------------------------------------------------------------------------------------ */
+MFAR_API int mfar_corpus_pack_rows_e4m3(const void* src, int src_dtype, int64_t n_rows, int64_t row_begin,
+                                        uint8_t* payload, float* scales, int64_t n_docs, int n_fields, int field,
+                                        int dim, int normalize, void* stream);
+/* Exact dequantization of rows of one field: dst fp32 [n_rows, dim] = float(p) * s. */
+MFAR_API int mfar_corpus_unpack_rows_e4m3(const uint8_t* payload, const float* scales, int64_t n_docs, int n_fields,
+                                          int field, int dim, int64_t row_begin, int64_t n_rows, float* dst,
+                                          void* stream);
 
 /* ------------------------------------------------------------------------------------------
  * Field mixture.  Replaces LinearWeights.forward, mfar/modeling/weighting.py:17-29, and the
@@ -216,6 +239,34 @@ MFAR_API int mfar_score_topk_bm25(const void* corpus, int64_t n_docs, int corpus
  * per-CTA partial lists inside mfar_score_topk and (b) the per-shard lists after the NCCL
  * all-gather (replaces the {rank}.qres file merge of mfar/modeling/contrastive.py:616-631).
  * keys: uint64 [L, Q, k_in]; key 0 = empty slot. */
+/* The three entry points above on an E4M3 corpus (mfar_corpus_pack_rows_e4m3) and E4M3 queries: same arguments, plus
+ * corpus_scales fp32 [n_tiles][corpus_fields][128] and q_scales fp32 [Q]; q_vecs is uint8 [Q, dim].
+ *   score[q,n] = sum_f fmaf-accumulated  w[q,f] * ((D_f[q,n] * q_scales[q]) * corpus_scales[n,f])  (+ sparse terms)
+ * with D_f the fp32 dot product of the two payload rows (every E4M3 x E4M3 product is exact in fp32).  The two scale
+ * products are rounded one after the other: folded into one factor they could underflow (2^-117 * 2^-117).
+ * impl: AUTO runs the tcgen05 kernel (kind::f8f6f4) at every batch size, SIMT the CUDA-core cross-check;
+ * MFAR_IMPL_TCGEN05_QS returns MFAR_ERR_SHAPE.  Ordering, ties, NaN ranking, doc_id_base and k as mfar_score_topk. */
+MFAR_API int mfar_score_topk_e4m3(const void* corpus, const float* corpus_scales, int64_t n_docs, int corpus_fields,
+                                  int field_begin, int n_dense, int dim, const void* q_vecs, const float* q_scales,
+                                  int Q, const float* w, const void* sparse, int n_sparse, int sparse_dtype,
+                                  int64_t sparse_ld, int64_t doc_id_base, int k, uint64_t* out_keys, float* out_scores,
+                                  int64_t* out_ids, void* workspace, size_t workspace_bytes, int impl, void* stream);
+MFAR_API int mfar_score_topk_coo_e4m3(const void* corpus, const float* corpus_scales, int64_t n_docs,
+                                      int corpus_fields, int field_begin, int n_dense, int dim, const void* q_vecs,
+                                      const float* q_scales, int Q, const float* w, const int32_t* coo_keys,
+                                      const void* coo_vals, int coo_dtype, const int64_t* field_offsets_host,
+                                      int n_sparse, int64_t doc_id_base, int k, uint64_t* out_keys, float* out_scores,
+                                      int64_t* out_ids, void* workspace, size_t workspace_bytes, int impl,
+                                      void* stream);
+MFAR_API int mfar_score_topk_bm25_e4m3(const void* corpus, const float* corpus_scales, int64_t n_docs,
+                                       int corpus_fields, int field_begin, int n_dense, int dim, const void* q_vecs,
+                                       const float* q_scales, int Q, const float* w, const void* const* indptr_host,
+                                       const void* const* indices_host, const void* const* data_host,
+                                       const int32_t* vocab_host, int n_sparse, const int32_t* entries,
+                                       int64_t n_entries, int64_t doc_id_base, int k, uint64_t* out_keys,
+                                       float* out_scores, int64_t* out_ids, void* workspace, size_t workspace_bytes,
+                                       int impl, void* stream);
+
 MFAR_API int mfar_topk_merge(const uint64_t* keys, int L, int Q, int k_in, int k, uint64_t* out_keys,
                     float* out_scores, int64_t* out_ids, void* stream);
 
@@ -282,6 +333,11 @@ MFAR_API int mfar_topk_apply_zero_init(float* scores, int64_t* ids, int Q, int k
 MFAR_API int mfar_score_candidates(const void* corpus, int64_t n_docs, int corpus_fields, int field_begin,
                           int n_fields, int dim, const void* q_vecs, int Q, const int64_t* rows, int C,
                           float* out, void* stream);
+/* The same on an E4M3 corpus and E4M3 queries:  out[f, q, c] = (D * q_scales[q]) * corpus_scales[rows[c], f]. */
+MFAR_API int mfar_score_candidates_e4m3(const void* corpus, const float* corpus_scales, int64_t n_docs,
+                                        int corpus_fields, int field_begin, int n_fields, int dim, const void* q_vecs,
+                                        const float* q_scales, int Q, const int64_t* rows, int C, float* out,
+                                        void* stream);
 
 /* ------------------------------------------------------------------------------------------
  * Host-buffer convenience call (the end-to-end path a reference-side caller uses): copies the

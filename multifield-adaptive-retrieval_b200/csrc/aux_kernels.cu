@@ -54,6 +54,95 @@ __global__ void unpack_rows_kernel(const __nv_bfloat16* __restrict__ packed, int
 }
 
 // ---------------------------------------------------------------------------------------
+// E4M3 pack: one warp per source row -> payload bytes [tile][field][128][dim] + one fp32 scale per row
+// [tile][field][128].  The row (after the optional float64 normalisation above) gets s = 2^e,
+// e = clamp(ceil(log2(amax / 448)), -117, 119): the lower bound keeps the smallest E4M3 subnormal times s at 2^-126 (a
+// normal fp32 / bf16 number), the upper bound keeps 448 * s finite in bf16.  Each element is rounded ONCE, from
+// float64, to the nearest E4M3 value of x / s (ties to even, saturating to +-448 - reached only when the clamp at 119
+// binds).  Zero rows store s = 1, rows holding a NaN / infinity s = NaN; both store payload 0.
+// ---------------------------------------------------------------------------------------
+constexpr int kE4m3MinScaleExp = -117;
+constexpr int kE4m3MaxScaleExp = 119;
+
+// nearest E4M3 value of v (ties to even, saturating at 448), as its byte
+__device__ __forceinline__ uint8_t e4m3_rne_byte(double v) {
+  const double a = fabs(v);
+  int k;
+  frexp(a, &k);                                      // a = m 2^k, m in [0.5, 1): 4 significant bits -> spacing 2^(k-4)
+  const int q = max(k - 4, -9);                      // -9: the subnormal spacing
+  double r = ldexp(rint(ldexp(a, -q)), q);           // exact scalings; rint rounds half to even
+  if (r > 448.0) r = 448.0;
+  uint32_t b;
+  if (r < 0.015625) {                                // below 2^-6: subnormal (or zero), mantissa = r * 2^9
+    b = uint32_t(r * 512.0);
+  } else {
+    int k2;
+    const double m = frexp(r, &k2);                  // r = (2m) 2^(k2-1), 2m = 1 + mant/8
+    b = (uint32_t(k2 + 6) << 3) | uint32_t(m * 16.0 - 8.0);
+  }
+  return uint8_t(b | (signbit(v) ? 0x80u : 0u));
+}
+
+template <typename SrcT>
+__global__ void pack_rows_e4m3_kernel(const SrcT* __restrict__ src, int64_t n_rows, int64_t row_begin,
+                                      uint8_t* __restrict__ payload, float* __restrict__ scales, int n_fields,
+                                      int field, int dim, int normalize) {
+  const int lane = threadIdx.x & 31;
+  const int64_t r = (int64_t(blockIdx.x) * blockDim.x + threadIdx.x) >> 5;
+  if (r >= n_rows) return;
+  const SrcT* s = src + r * dim;
+  const int64_t doc = row_begin + r;
+  const int64_t row = ((doc / kTileDocs) * n_fields + field) * kTileDocs + doc % kTileDocs;
+  uint8_t* d = payload + row * int64_t(dim);
+  double ss = 0.0, amax = 0.0;
+  bool bad = false;
+  for (int i = lane; i < dim; i += 32) {
+    const double v = double(float(s[i]));
+    bad |= !isfinite(v);
+    ss = fma(v, v, ss);
+    amax = fmax(amax, fabs(v));
+  }
+  bad = __any_sync(0xffffffffu, bad);
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) {
+    ss += __shfl_xor_sync(0xffffffffu, ss, o);
+    amax = fmax(amax, __shfl_xor_sync(0xffffffffu, amax, o));
+  }
+  // F.normalize's eps on an fp32 tensor; division is exact-rounded, so amax / norm is the largest |quotient|
+  const double norm = normalize ? fmax(sqrt(ss), double(1e-12f)) : 1.0;
+  if (normalize) amax = amax / norm;
+  if (bad || amax == 0.0) {
+    for (int i = lane; i < dim; i += 32) d[i] = 0;
+    if (lane == 0) scales[row] = bad ? __int_as_float(0x7fc00000) : 1.f;
+    return;
+  }
+  int k;
+  const double m = frexp(amax, &k);                  // amax <= 448 2^e  <=>  e >= k - 9 + (m > 0.875)
+  const int e = min(max(k - 9 + (m > 0.875 ? 1 : 0), kE4m3MinScaleExp), kE4m3MaxScaleExp);
+  for (int i = lane; i < dim; i += 32) {
+    double v = double(float(s[i]));
+    if (normalize) v = v / norm;
+    d[i] = e4m3_rne_byte(ldexp(v, -e));
+  }
+  if (lane == 0) scales[row] = ldexpf(1.f, e);
+}
+
+__device__ __forceinline__ float e4m3_to_float(uint8_t b) { return e4m3x2_to_float2(b).x; }
+
+__global__ void unpack_rows_e4m3_kernel(const uint8_t* __restrict__ payload, const float* __restrict__ scales,
+                                        int n_fields, int field, int dim, int64_t row_begin, int64_t n_rows,
+                                        float* __restrict__ dst) {
+  const int lane = threadIdx.x & 31;
+  const int64_t r = (int64_t(blockIdx.x) * blockDim.x + threadIdx.x) >> 5;
+  if (r >= n_rows) return;
+  const int64_t doc = row_begin + r;
+  const int64_t row = ((doc / kTileDocs) * n_fields + field) * kTileDocs + doc % kTileDocs;
+  const float sc = scales[row];
+  const uint8_t* s = payload + row * int64_t(dim);
+  for (int i = lane; i < dim; i += 32) dst[r * dim + i] = e4m3_to_float(s[i]) * sc;
+}
+
+// ---------------------------------------------------------------------------------------
 // mixture weights: one CTA per query (or one CTA total when !query_cond).
 // logits[f] = sum_e q[e] * W[e*F + f];  w = softmax(logits) * mask.   weighting.py:25-28
 // ---------------------------------------------------------------------------------------
@@ -109,9 +198,11 @@ __global__ void mixture_apply_kernel(const float* __restrict__ x, const float* _
 // candidate re-scoring: one warp per (candidate, field); loops over queries.
 // out[f, q, c] = <q_vec[q], corpus[rows[c], field_begin + f]>;  rows[c] < 0 -> 0
 // ---------------------------------------------------------------------------------------
-__global__ void score_candidates_kernel(const __nv_bfloat16* __restrict__ corpus, int64_t n_docs, int corpus_fields,
-                                        int field_begin, int n_fields, int dim,
-                                        const __nv_bfloat16* __restrict__ q_vecs, int Q,
+// E4M3 (E8): D of the payload rows, then (D * s_q) * s_d as the scoring kernels apply it.
+template <bool E8>
+__global__ void score_candidates_kernel(const void* __restrict__ corpus_v, const float* __restrict__ corpus_scales,
+                                        int64_t n_docs, int corpus_fields, int field_begin, int n_fields, int dim,
+                                        const void* __restrict__ q_vecs_v, const float* __restrict__ q_scales, int Q,
                                         const int64_t* __restrict__ rows, int C, float* __restrict__ out) {
   const int lane = threadIdx.x & 31;
   const int64_t wid = (int64_t(blockIdx.x) * blockDim.x + threadIdx.x) >> 5;
@@ -122,10 +213,23 @@ __global__ void score_candidates_kernel(const __nv_bfloat16* __restrict__ corpus
     for (int q = lane; q < Q; q += 32) out[(int64_t(f) * Q + q) * C + c] = 0.f;
     return;
   }
-  const __nv_bfloat16* v =
-      corpus + (((row / kTileDocs) * corpus_fields + field_begin + f) * kTileDocs + (row % kTileDocs)) * int64_t(dim);
+  const int64_t crow = ((row / kTileDocs) * corpus_fields + field_begin + f) * kTileDocs + (row % kTileDocs);
+  if (E8) {
+    const uint8_t* v = static_cast<const uint8_t*>(corpus_v) + crow * int64_t(dim);
+    const float sd = corpus_scales[crow];
+    for (int q = 0; q < Q; ++q) {
+      const uint8_t* qv = static_cast<const uint8_t*>(q_vecs_v) + int64_t(q) * dim;
+      float acc = 0.f;
+      for (int i = lane; i < dim; i += 32) acc = fmaf(e4m3_to_float(qv[i]), e4m3_to_float(v[i]), acc);
+#pragma unroll
+      for (int o = 16; o > 0; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
+      if (lane == 0) out[(int64_t(f) * Q + q) * C + c] = (acc * q_scales[q]) * sd;
+    }
+    return;
+  }
+  const __nv_bfloat16* v = static_cast<const __nv_bfloat16*>(corpus_v) + crow * int64_t(dim);
   for (int q = 0; q < Q; ++q) {
-    const __nv_bfloat16* qv = q_vecs + int64_t(q) * dim;
+    const __nv_bfloat16* qv = static_cast<const __nv_bfloat16*>(q_vecs_v) + int64_t(q) * dim;
     float acc = 0.f;
     for (int i = lane; i < dim; i += 32) acc = fmaf(__bfloat162float(qv[i]), __bfloat162float(v[i]), acc);
 #pragma unroll
@@ -592,6 +696,34 @@ int launch_unpack_rows(const void* packed, int n_fields, int field, int dim, int
   return MFAR_OK;
 }
 
+int launch_pack_rows_e4m3(const void* src, int src_dtype, int64_t n_rows, int64_t row_begin, uint8_t* payload,
+                          float* scales, int n_fields, int field, int dim, int normalize, cudaStream_t st) {
+  if (n_rows == 0) return MFAR_OK;
+  const int threads = 256;
+  const unsigned blocks = unsigned((n_rows * 32 + threads - 1) / threads);
+  if (src_dtype == MFAR_F32)
+    pack_rows_e4m3_kernel<float><<<blocks, threads, 0, st>>>(static_cast<const float*>(src), n_rows, row_begin, payload,
+                                                             scales, n_fields, field, dim, normalize);
+  else if (src_dtype == MFAR_BF16)
+    pack_rows_e4m3_kernel<__nv_bfloat16><<<blocks, threads, 0, st>>>(static_cast<const __nv_bfloat16*>(src), n_rows,
+                                                                     row_begin, payload, scales, n_fields, field, dim,
+                                                                     normalize);
+  else
+    return MFAR_ERR_ARG;
+  MFAR_CUDA_OK(cudaGetLastError());
+  return MFAR_OK;
+}
+
+int launch_unpack_rows_e4m3(const uint8_t* payload, const float* scales, int n_fields, int field, int dim,
+                            int64_t row_begin, int64_t n_rows, float* dst, cudaStream_t st) {
+  if (n_rows == 0) return MFAR_OK;
+  const int threads = 256;
+  const unsigned blocks = unsigned((n_rows * 32 + threads - 1) / threads);
+  unpack_rows_e4m3_kernel<<<blocks, threads, 0, st>>>(payload, scales, n_fields, field, dim, row_begin, n_rows, dst);
+  MFAR_CUDA_OK(cudaGetLastError());
+  return MFAR_OK;
+}
+
 int launch_mixture_weights(const float* q_emb, const float* W, const float* mask, int Q, int E, int F,
                            int query_cond, float* out_w, cudaStream_t st) {
   mixture_weights_kernel<<<Q, 256, 0, st>>>(q_emb, W, mask, E, F, query_cond, out_w);
@@ -608,14 +740,18 @@ int launch_mixture_apply(const float* x, const float* w, int B, int S, int F, in
   return MFAR_OK;
 }
 
-int launch_score_candidates(const void* corpus, int64_t n_docs, int corpus_fields, int field_begin, int n_fields,
-                            int dim, const void* q_vecs, int Q, const int64_t* rows, int C, float* out,
-                            cudaStream_t st) {
+int launch_score_candidates(const void* corpus, const float* corpus_scales, int64_t n_docs, int corpus_fields,
+                            int field_begin, int n_fields, int dim, const void* q_vecs, const float* q_scales, int Q,
+                            const int64_t* rows, int C, float* out, cudaStream_t st) {
   if (C == 0 || n_fields == 0) return MFAR_OK;
   const int64_t warps = int64_t(C) * n_fields;
-  score_candidates_kernel<<<(unsigned)((warps * 32 + 255) / 256), 256, 0, st>>>(
-      static_cast<const __nv_bfloat16*>(corpus), n_docs, corpus_fields, field_begin, n_fields, dim,
-      static_cast<const __nv_bfloat16*>(q_vecs), Q, rows, C, out);
+  const unsigned blocks = unsigned((warps * 32 + 255) / 256);
+  if (corpus_scales)
+    score_candidates_kernel<true><<<blocks, 256, 0, st>>>(corpus, corpus_scales, n_docs, corpus_fields, field_begin,
+                                                          n_fields, dim, q_vecs, q_scales, Q, rows, C, out);
+  else
+    score_candidates_kernel<false><<<blocks, 256, 0, st>>>(corpus, nullptr, n_docs, corpus_fields, field_begin,
+                                                           n_fields, dim, q_vecs, nullptr, Q, rows, C, out);
   MFAR_CUDA_OK(cudaGetLastError());
   return MFAR_OK;
 }

@@ -140,6 +140,27 @@ int mfar_corpus_unpack_rows(const void* packed, int64_t n_docs, int n_fields, in
   return launch_unpack_rows(packed, n_fields, field, dim, row_begin, n_rows, dst, static_cast<cudaStream_t>(stream));
 }
 
+// Replaces, as mfar_corpus_pack_rows does, the per-field fp32 memmaps of mfar/modeling/contrastive.py:482-490 (read at
+// mfar/data/index.py:196,230), stored at one byte per element.
+int mfar_corpus_pack_rows_e4m3(const void* src, int src_dtype, int64_t n_rows, int64_t row_begin, uint8_t* payload,
+                               float* scales, int64_t n_docs, int n_fields, int field, int dim, int normalize,
+                               void* stream) {
+  if (!src || !payload || !scales || n_rows < 0 || row_begin < 0 || row_begin + n_rows > n_docs) return MFAR_ERR_ARG;
+  if (field < 0 || field >= n_fields || dim <= 0) return MFAR_ERR_SHAPE;
+  if (int rc = check_arch()) return rc;
+  return launch_pack_rows_e4m3(src, src_dtype, n_rows, row_begin, payload, scales, n_fields, field, dim, normalize,
+                               static_cast<cudaStream_t>(stream));
+}
+
+int mfar_corpus_unpack_rows_e4m3(const uint8_t* payload, const float* scales, int64_t n_docs, int n_fields, int field,
+                                 int dim, int64_t row_begin, int64_t n_rows, float* dst, void* stream) {
+  if (!payload || !scales || !dst || n_rows < 0 || row_begin < 0 || row_begin + n_rows > n_docs) return MFAR_ERR_ARG;
+  if (field < 0 || field >= n_fields || dim <= 0) return MFAR_ERR_SHAPE;
+  if (int rc = check_arch()) return rc;
+  return launch_unpack_rows_e4m3(payload, scales, n_fields, field, dim, row_begin, n_rows, dst,
+                                 static_cast<cudaStream_t>(stream));
+}
+
 int mfar_mixture_weights(const float* q_emb, const float* W, const float* mask, int Q, int E, int F, int query_cond,
                          float* out_w, void* stream) {
   if (!W || !out_w || Q <= 0 || (query_cond && (!q_emb || E <= 0))) return MFAR_ERR_ARG;
@@ -214,16 +235,24 @@ static int fill_bm25_fields(const void* const* indptr_host, const void* const* i
   return MFAR_OK;
 }
 
-static int score_topk_core(const void* corpus, int64_t n_docs, int corpus_fields, int field_begin, int n_dense, int dim,
-                           const void* q_vecs, int Q, const float* w, const SparseInput& sp, int n_sparse,
+// Dense operands of a scoring call: the corpus and the queries, bf16, or E4M3 with their row scales.
+struct DenseInput {
+  const void* corpus; const float* corpus_scales; const void* q_vecs; const float* q_scales; int dtype;
+};
+
+static int score_topk_core(const DenseInput& dn, int64_t n_docs, int corpus_fields, int field_begin, int n_dense,
+                           int dim, int Q, const float* w, const SparseInput& sp, int n_sparse,
                            int64_t doc_id_base, int k, uint64_t* out_keys, float* out_scores, int64_t* out_ids,
                            void* workspace, size_t workspace_bytes, int impl, void* stream) {
+  const void* corpus = dn.corpus;
+  const void* q_vecs = dn.q_vecs;
   t_last_launches = 0;
   if (n_docs <= 0 || Q <= 0 || !w || !workspace || (!out_scores && !out_ids && !out_keys)) return MFAR_ERR_ARG;
   if (n_dense < 0 || n_sparse < 0 || n_dense + n_sparse <= 0 || n_dense + n_sparse > MFAR_MAX_FIELDS)
     return MFAR_ERR_SHAPE;
   if (n_dense > 0 && (!corpus || !q_vecs || dim <= 0 || field_begin < 0 || field_begin + n_dense > corpus_fields))
     return MFAR_ERR_ARG;
+  if (n_dense > 0 && dn.dtype == MFAR_E4M3 && (!dn.corpus_scales || !dn.q_scales)) return MFAR_ERR_ARG;
   if (n_sparse > 0 && sp.kind == 1 && (!sp.dense || sp.dense_ld < n_docs)) return MFAR_ERR_ARG;
   if (n_sparse > 0 && sp.kind == 2 && (!sp.field_offsets_host || sp.field_offsets_host[0] != 0)) return MFAR_ERR_ARG;
   if (n_sparse > 0 && sp.kind == 0) return MFAR_ERR_ARG;
@@ -235,7 +264,8 @@ static int score_topk_core(const void* corpus, int64_t n_docs, int corpus_fields
   cudaStream_t st = static_cast<cudaStream_t>(stream);
 
   ScoreArgs a{};
-  a.corpus = corpus; a.n_docs = n_docs; a.n_tiles = int((n_docs + kTileDocs - 1) / kTileDocs);
+  a.corpus = corpus; a.corpus_dtype = dn.dtype; a.corpus_scales = dn.corpus_scales; a.q_scales = dn.q_scales;
+  a.n_docs = n_docs; a.n_tiles = int((n_docs + kTileDocs - 1) / kTileDocs);
   a.corpus_fields = corpus_fields; a.field_begin = field_begin; a.n_dense = n_dense; a.dim = dim;
   a.q_vecs = q_vecs; a.Q = Q; a.w = w; a.w_ld = n_dense + n_sparse; a.doc_id_base = doc_id_base; a.k = k;
   if (n_dense > 0 && impl == MFAR_IMPL_TCGEN05 && !score_tc_supported(a)) return MFAR_ERR_SHAPE;
@@ -345,7 +375,9 @@ static int score_topk_core(const void* corpus, int64_t n_docs, int corpus_fields
       // A prefix is not scored twice: the next pass starts behind it (every per-doc pointer advanced by the prefix's
       // whole tiles) and the next merge takes the prefix's ranked top k as one more list.
       const int64_t skip = ap.n_docs;
-      a.corpus = static_cast<const char*>(a.corpus) + size_t(ap.n_tiles) * a.corpus_fields * kTileDocs * a.dim * 2;
+      const size_t skip_rows = size_t(ap.n_tiles) * a.corpus_fields * kTileDocs;
+      a.corpus = static_cast<const char*>(a.corpus) + skip_rows * a.dim * (a.corpus_dtype == MFAR_E4M3 ? 1 : 2);
+      if (a.corpus_scales) a.corpus_scales += skip_rows;
       a.n_tiles -= ap.n_tiles;
       a.n_docs -= skip;
       a.doc_id_base += skip;
@@ -385,8 +417,22 @@ int mfar_score_topk(const void* corpus, int64_t n_docs, int corpus_fields, int f
                     int64_t* out_ids, void* workspace, size_t workspace_bytes, int impl, void* stream) {
   SparseInput sp;
   if (n_sparse > 0) { sp.kind = 1; sp.dense = sparse; sp.dense_dtype = sparse_dtype; sp.dense_ld = sparse_ld; }
-  return score_topk_core(corpus, n_docs, corpus_fields, field_begin, n_dense, dim, q_vecs, Q, w, sp, n_sparse,
-                         doc_id_base, k, out_keys, out_scores, out_ids, workspace, workspace_bytes, impl, stream);
+  return score_topk_core({corpus, nullptr, q_vecs, nullptr, MFAR_BF16}, n_docs, corpus_fields, field_begin, n_dense,
+                         dim, Q, w, sp, n_sparse, doc_id_base, k, out_keys, out_scores, out_ids, workspace,
+                         workspace_bytes, impl, stream);
+}
+
+// mfar_score_topk on an E4M3 corpus: the same reference lines (index.py:181-232, 111-118; contrastive.py:686,694,696)
+int mfar_score_topk_e4m3(const void* corpus, const float* corpus_scales, int64_t n_docs, int corpus_fields,
+                         int field_begin, int n_dense, int dim, const void* q_vecs, const float* q_scales, int Q,
+                         const float* w, const void* sparse, int n_sparse, int sparse_dtype, int64_t sparse_ld,
+                         int64_t doc_id_base, int k, uint64_t* out_keys, float* out_scores, int64_t* out_ids,
+                         void* workspace, size_t workspace_bytes, int impl, void* stream) {
+  SparseInput sp;
+  if (n_sparse > 0) { sp.kind = 1; sp.dense = sparse; sp.dense_dtype = sparse_dtype; sp.dense_ld = sparse_ld; }
+  return score_topk_core({corpus, corpus_scales, q_vecs, q_scales, MFAR_E4M3}, n_docs, corpus_fields, field_begin,
+                         n_dense, dim, Q, w, sp, n_sparse, doc_id_base, k, out_keys, out_scores, out_ids, workspace,
+                         workspace_bytes, impl, stream);
 }
 
 int mfar_score_topk_coo(const void* corpus, int64_t n_docs, int corpus_fields, int field_begin, int n_dense, int dim,
@@ -399,8 +445,26 @@ int mfar_score_topk_coo(const void* corpus, int64_t n_docs, int corpus_fields, i
   SparseInput sp;
   sp.kind = 2; sp.coo_keys = coo_keys; sp.coo_vals = coo_vals; sp.coo_dtype = coo_dtype;
   sp.field_offsets_host = field_offsets_host;
-  return score_topk_core(corpus, n_docs, corpus_fields, field_begin, n_dense, dim, q_vecs, Q, w, sp, n_sparse,
-                         doc_id_base, k, out_keys, out_scores, out_ids, workspace, workspace_bytes, impl, stream);
+  return score_topk_core({corpus, nullptr, q_vecs, nullptr, MFAR_BF16}, n_docs, corpus_fields, field_begin, n_dense,
+                         dim, Q, w, sp, n_sparse, doc_id_base, k, out_keys, out_scores, out_ids, workspace,
+                         workspace_bytes, impl, stream);
+}
+
+// mfar_score_topk_coo on an E4M3 corpus (precompute_bm25s_scores.py:21-30, util.py:151-173, index.py:120-125)
+int mfar_score_topk_coo_e4m3(const void* corpus, const float* corpus_scales, int64_t n_docs, int corpus_fields,
+                             int field_begin, int n_dense, int dim, const void* q_vecs, const float* q_scales, int Q,
+                             const float* w, const int32_t* coo_keys, const void* coo_vals, int coo_dtype,
+                             const int64_t* field_offsets_host, int n_sparse, int64_t doc_id_base, int k,
+                             uint64_t* out_keys, float* out_scores, int64_t* out_ids, void* workspace,
+                             size_t workspace_bytes, int impl, void* stream) {
+  if (n_sparse <= 0 || !field_offsets_host) return MFAR_ERR_ARG;
+  if (field_offsets_host[n_sparse] > 0 && (!coo_keys || !coo_vals)) return MFAR_ERR_ARG;
+  SparseInput sp;
+  sp.kind = 2; sp.coo_keys = coo_keys; sp.coo_vals = coo_vals; sp.coo_dtype = coo_dtype;
+  sp.field_offsets_host = field_offsets_host;
+  return score_topk_core({corpus, corpus_scales, q_vecs, q_scales, MFAR_E4M3}, n_docs, corpus_fields, field_begin,
+                         n_dense, dim, Q, w, sp, n_sparse, doc_id_base, k, out_keys, out_scores, out_ids, workspace,
+                         workspace_bytes, impl, stream);
 }
 
 int mfar_bm25_build_scores(const int32_t* post_token, const int32_t* post_doc, const int32_t* post_tf, int64_t nnz,
@@ -493,8 +557,25 @@ int mfar_score_topk_bm25(const void* corpus, int64_t n_docs, int corpus_fields, 
   SparseInput sp;
   sp.kind = 3; sp.entries = entries; sp.n_entries = n_entries;
   if (int rc = fill_bm25_fields(indptr_host, indices_host, data_host, vocab_host, n_sparse, &sp.bm25)) return rc;
-  return score_topk_core(corpus, n_docs, corpus_fields, field_begin, n_dense, dim, q_vecs, Q, w, sp, n_sparse,
-                         doc_id_base, k, out_keys, out_scores, out_ids, workspace, workspace_bytes, impl, stream);
+  return score_topk_core({corpus, nullptr, q_vecs, nullptr, MFAR_BF16}, n_docs, corpus_fields, field_begin, n_dense,
+                         dim, Q, w, sp, n_sparse, doc_id_base, k, out_keys, out_scores, out_ids, workspace,
+                         workspace_bytes, impl, stream);
+}
+
+// mfar_score_topk_bm25 on an E4M3 corpus (index.py:72-76, 95-118 for the sparse fields)
+int mfar_score_topk_bm25_e4m3(const void* corpus, const float* corpus_scales, int64_t n_docs, int corpus_fields,
+                              int field_begin, int n_dense, int dim, const void* q_vecs, const float* q_scales, int Q,
+                              const float* w, const void* const* indptr_host, const void* const* indices_host,
+                              const void* const* data_host, const int32_t* vocab_host, int n_sparse,
+                              const int32_t* entries, int64_t n_entries, int64_t doc_id_base, int k,
+                              uint64_t* out_keys, float* out_scores, int64_t* out_ids, void* workspace,
+                              size_t workspace_bytes, int impl, void* stream) {
+  SparseInput sp;
+  sp.kind = 3; sp.entries = entries; sp.n_entries = n_entries;
+  if (int rc = fill_bm25_fields(indptr_host, indices_host, data_host, vocab_host, n_sparse, &sp.bm25)) return rc;
+  return score_topk_core({corpus, corpus_scales, q_vecs, q_scales, MFAR_E4M3}, n_docs, corpus_fields, field_begin,
+                         n_dense, dim, Q, w, sp, n_sparse, doc_id_base, k, out_keys, out_scores, out_ids, workspace,
+                         workspace_bytes, impl, stream);
 }
 
 int mfar_topk_merge(const uint64_t* keys, int L, int Q, int k_in, int k, uint64_t* out_keys, float* out_scores,
@@ -571,8 +652,20 @@ int mfar_score_candidates(const void* corpus, int64_t n_docs, int corpus_fields,
   if (!corpus || !q_vecs || !rows || !out || Q <= 0 || C < 0 || n_docs <= 0) return MFAR_ERR_ARG;
   if (n_fields <= 0 || field_begin < 0 || field_begin + n_fields > corpus_fields || dim <= 0) return MFAR_ERR_SHAPE;
   if (int rc = check_arch()) return rc;
-  return launch_score_candidates(corpus, n_docs, corpus_fields, field_begin, n_fields, dim, q_vecs, Q, rows, C, out,
-                                 static_cast<cudaStream_t>(stream));
+  return launch_score_candidates(corpus, nullptr, n_docs, corpus_fields, field_begin, n_fields, dim, q_vecs, nullptr, Q,
+                                 rows, C, out, static_cast<cudaStream_t>(stream));
+}
+
+// mfar_score_candidates on an E4M3 corpus (index.py:227-232)
+int mfar_score_candidates_e4m3(const void* corpus, const float* corpus_scales, int64_t n_docs, int corpus_fields,
+                               int field_begin, int n_fields, int dim, const void* q_vecs, const float* q_scales, int Q,
+                               const int64_t* rows, int C, float* out, void* stream) {
+  if (!corpus || !corpus_scales || !q_vecs || !q_scales || !rows || !out || Q <= 0 || C < 0 || n_docs <= 0)
+    return MFAR_ERR_ARG;
+  if (n_fields <= 0 || field_begin < 0 || field_begin + n_fields > corpus_fields || dim <= 0) return MFAR_ERR_SHAPE;
+  if (int rc = check_arch()) return rc;
+  return launch_score_candidates(corpus, corpus_scales, n_docs, corpus_fields, field_begin, n_fields, dim, q_vecs,
+                                 q_scales, Q, rows, C, out, static_cast<cudaStream_t>(stream));
 }
 
 int mfar_union_rescore(const void* corpus, int64_t n_docs, int corpus_fields, int n_dense, int dim, const void* q_vecs,

@@ -375,4 +375,18 @@ __device__ __forceinline__ unsigned long long pool_publish_min(unsigned long lon
   return m;
 }
 
+// Two E4M3 bytes (the low byte is element 0) -> fp32.  Every E4M3 value is exact in f16, so the one conversion
+// instruction (cvt.rn.f16x2.e4m3x2) and the widening are exact.
+__device__ __forceinline__ float2 e4m3x2_to_float2(uint32_t two_bytes) {
+  uint32_t h;
+  asm("cvt.rn.f16x2.e4m3x2 %0, %1;" : "=r"(h) : "h"(uint16_t(two_bytes)));
+  return __half22float2(*reinterpret_cast<const __half2*>(&h));
+}
+// 8 E4M3 bytes -> 8 fp32
+__device__ __forceinline__ void e4m3x8_to_f32(const uint2& v, float (&f)[8]) {
+  float2 a = e4m3x2_to_float2(v.x), b = e4m3x2_to_float2(v.x >> 16), c = e4m3x2_to_float2(v.y),
+         d = e4m3x2_to_float2(v.y >> 16);
+  f[0] = a.x; f[1] = a.y; f[2] = b.x; f[3] = b.y; f[4] = c.x; f[5] = c.y; f[6] = d.x; f[7] = d.y;
+}
+
 }  // namespace mfar

@@ -35,13 +35,18 @@ int launch_pack_rows(const void* src, int src_dtype, int64_t n_rows, int64_t row
                      int n_fields, int field, int dim, int normalize, cudaStream_t st);
 int launch_unpack_rows(const void* packed, int n_fields, int field, int dim, int64_t row_begin, int64_t n_rows,
                        float* dst, cudaStream_t st);
+int launch_pack_rows_e4m3(const void* src, int src_dtype, int64_t n_rows, int64_t row_begin, uint8_t* payload,
+                          float* scales, int n_fields, int field, int dim, int normalize, cudaStream_t st);
+int launch_unpack_rows_e4m3(const uint8_t* payload, const float* scales, int n_fields, int field, int dim,
+                            int64_t row_begin, int64_t n_rows, float* dst, cudaStream_t st);
 int launch_mixture_weights(const float* q_emb, const float* W, const float* mask, int Q, int E, int F,
                            int query_cond, float* out_w, cudaStream_t st);
 int launch_mixture_apply(const float* x, const float* w, int B, int S, int F, int w_rows, float* out,
                          cudaStream_t st);
-int launch_score_candidates(const void* corpus, int64_t n_docs, int corpus_fields, int field_begin, int n_fields,
-                            int dim, const void* q_vecs, int Q, const int64_t* rows, int C, float* out,
-                            cudaStream_t st);
+// corpus_scales / q_scales: nullptr for a bf16 corpus, the row scales of an E4M3 corpus and its queries otherwise
+int launch_score_candidates(const void* corpus, const float* corpus_scales, int64_t n_docs, int corpus_fields,
+                            int field_begin, int n_fields, int dim, const void* q_vecs, const float* q_scales, int Q,
+                            const int64_t* rows, int C, float* out, cudaStream_t st);
 int launch_sparse_premix(const void* sparse, int sparse_dtype, int64_t sparse_ld, int n_sparse, const float* w,
                          int w_ld, int w_off, int Q, int64_t n_docs, float* base, int64_t base_ld,
                          cudaStream_t st);
@@ -76,14 +81,17 @@ int launch_mixture_bwd(const float* x, const float* q, const float* W, const flo
 
 // Arguments common to both scoring kernels (all device pointers).
 struct ScoreArgs {
-  const void* corpus;       // packed bf16 [tiles][corpus_fields][128][dim]
+  const void* corpus;       // packed bf16 [tiles][corpus_fields][128][dim], or E4M3 bytes (corpus_dtype == MFAR_E4M3)
+  int corpus_dtype;         // MFAR_BF16 or MFAR_E4M3 (queries have the corpus's type)
+  const float* corpus_scales;   // E4M3: fp32 [tiles][corpus_fields][128] row scales (powers of two), else nullptr
+  const float* q_scales;        // E4M3: fp32 [Q] query scales, else nullptr
   int64_t n_docs;
   int n_tiles;
   int corpus_fields;
   int field_begin;
   int n_dense;
   int dim;
-  const void* q_vecs;       // bf16 [Q, dim]
+  const void* q_vecs;       // bf16 / E4M3 [Q, dim]
   int Q;
   const float* w;           // fp32 [Q, w_ld]
   int w_ld;

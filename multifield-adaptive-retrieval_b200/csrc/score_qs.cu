@@ -592,7 +592,7 @@ score_qs_kernel(const __grid_constant__ CUtensorMap map_b, const __grid_constant
 
 // ------------------------------------------------------------------------------------ host side
 bool score_qs_supported(const ScoreArgs& a) {
-  return a.n_dense >= 1 && a.dim % kChunkK == 0 && a.dim >= kChunkK && a.dim / 2 <= kQsDCol &&
+  return a.n_dense >= 1 && a.corpus_dtype != MFAR_E4M3 && a.dim % kChunkK == 0 && a.dim >= kChunkK && a.dim / 2 <= kQsDCol &&
          (reinterpret_cast<uintptr_t>(a.corpus) % 16 == 0) && (reinterpret_cast<uintptr_t>(a.q_vecs) % 16 == 0) &&
          int64_t(a.n_tiles) * a.corpus_fields * kTileDocs < (int64_t(1) << 31);
 }

@@ -8,6 +8,9 @@
 // Scores never leave registers: lane j keeps doc j's final score, adds the pre-mixed sparse
 // term, and pushes (score,id) keys that beat the CTA's per-query threshold into its candidate
 // list (threshold + compaction logic in common.cuh).
+// E4M3 corpus (E8): the same mapping with 8-byte vectors of 8 elements, decoded by cvt.rn.f16x2.e4m3x2 (exact); the
+// payload dot product D is then scaled as the tensor-core path does it, w * ((D * s_q) * s_d) - the CUDA-core
+// cross-check of the kind::f8f6f4 kernel.
 #include "common.cuh"
 #include "kernels.h"
 
@@ -17,10 +20,12 @@ constexpr int kSimtThreads = 128;
 constexpr int kSimtMaxVec = 4;  // 16-byte vectors per lane per row: dim <= 4*32*8 = 1024
 
 struct SimtParams {
-  const uint4* corpus;
+  const void* corpus;
   int64_t n_docs;
   int n_tiles, corpus_fields, field_begin, n_dense, dim;
-  const __nv_bfloat16* q_vecs;
+  const void* q_vecs;
+  const float* corpus_scales;   // E8 only
+  const float* q_scales;        // E8 only
   int Q;
   const float* w;
   int w_ld;
@@ -46,7 +51,7 @@ __device__ __forceinline__ uint4 ld_stream(const uint4* p) {
 }
 
 // QB = queries handled per corpus pass (their slices live in registers)
-template <int QB>
+template <int QB, bool E8>
 __global__ void __launch_bounds__(kSimtThreads) score_simt_kernel(SimtParams p) {
   extern __shared__ float s_w[];                      // [QB][n_dense]
   __shared__ unsigned long long s_thr[QB];
@@ -56,7 +61,6 @@ __global__ void __launch_bounds__(kSimtThreads) score_simt_kernel(SimtParams p) 
   const int g = blockIdx.x;
   const int nvec = p.dim / 8;                         // 16-byte vectors per row
   const int vec_per_lane = (nvec + 31) / 32;
-  const int64_t row_vecs = nvec;
 
   for (int q0 = 0; q0 < p.Q; q0 += QB) {
     const int nq = min(QB, p.Q - q0);
@@ -68,14 +72,23 @@ __global__ void __launch_bounds__(kSimtThreads) score_simt_kernel(SimtParams p) 
     if (threadIdx.x < QB) { s_thr[threadIdx.x] = 0ull; s_cnt[threadIdx.x] = 0; }
     // query slices -> registers (fp32)
     float qreg[QB][kSimtMaxVec][8];
+    float sq[QB];
+#pragma unroll
+    for (int qi = 0; qi < QB; ++qi) sq[qi] = (E8 && qi < nq) ? p.q_scales[q0 + qi] : 1.f;
 #pragma unroll
     for (int qi = 0; qi < QB; ++qi)
 #pragma unroll
       for (int v = 0; v < kSimtMaxVec; ++v) {
         const int vi = lane + 32 * v;
         if (p.n_dense > 0 && v < vec_per_lane && vi < nvec && qi < nq) {
-          uint4 raw = *reinterpret_cast<const uint4*>(p.q_vecs + int64_t(q0 + qi) * p.dim + vi * 8);
-          bf16x8_to_f32(raw, qreg[qi][v]);
+          if constexpr (E8) {
+            e4m3x8_to_f32(*reinterpret_cast<const uint2*>(static_cast<const uint8_t*>(p.q_vecs) + int64_t(q0 + qi) * p.dim +
+                                                          vi * 8), qreg[qi][v]);
+          } else {
+            uint4 raw = *reinterpret_cast<const uint4*>(static_cast<const __nv_bfloat16*>(p.q_vecs) +
+                                                        int64_t(q0 + qi) * p.dim + vi * 8);
+            bf16x8_to_f32(raw, qreg[qi][v]);
+          }
         } else {
 #pragma unroll
           for (int e = 0; e < 8; ++e) qreg[qi][v][e] = 0.f;
@@ -93,31 +106,58 @@ __global__ void __launch_bounds__(kSimtThreads) score_simt_kernel(SimtParams p) 
 #pragma unroll
         for (int qi = 0; qi < QB; ++qi) acc[qi] = 0.f;
         for (int f = 0; f < p.n_dense; ++f) {
-          const uint4* row = p.corpus +
-              ((int64_t(t) * p.corpus_fields + p.field_begin + f) * kTileDocs + warp * 32 + j) * row_vecs;
-          uint4 raw[kSimtMaxVec];
-#pragma unroll
-          for (int v = 0; v < kSimtMaxVec; ++v) {
-            const int vi = lane + 32 * v;
-            raw[v] = (v < vec_per_lane && vi < nvec) ? ld_stream(row + vi) : make_uint4(0, 0, 0, 0);
-          }
+          const int64_t row_idx = (int64_t(t) * p.corpus_fields + p.field_begin + f) * kTileDocs + warp * 32 + j;
           float part[QB];
 #pragma unroll
           for (int qi = 0; qi < QB; ++qi) part[qi] = 0.f;
+          float sd = 1.f;
+          if constexpr (E8) {
+            const uint2* row = static_cast<const uint2*>(p.corpus) + row_idx * nvec;
+            uint2 raw[kSimtMaxVec];
 #pragma unroll
-          for (int v = 0; v < kSimtMaxVec; ++v) {
-            float x[8];
-            bf16x8_to_f32(raw[v], x);
+            for (int v = 0; v < kSimtMaxVec; ++v) {
+              const int vi = lane + 32 * v;
+              if (v < vec_per_lane && vi < nvec) {
+                asm volatile("ld.global.nc.L1::no_allocate.v2.u32 {%0,%1}, [%2];"
+                             : "=r"(raw[v].x), "=r"(raw[v].y) : "l"(row + vi));
+              } else {
+                raw[v] = make_uint2(0, 0);
+              }
+            }
+            sd = __ldg(p.corpus_scales + row_idx);
 #pragma unroll
-            for (int qi = 0; qi < QB; ++qi)
+            for (int v = 0; v < kSimtMaxVec; ++v) {
+              float x[8];
+              e4m3x8_to_f32(raw[v], x);
 #pragma unroll
-              for (int e = 0; e < 8; ++e) part[qi] = fmaf(x[e], qreg[qi][v][e], part[qi]);
+              for (int qi = 0; qi < QB; ++qi)
+#pragma unroll
+                for (int e = 0; e < 8; ++e) part[qi] = fmaf(x[e], qreg[qi][v][e], part[qi]);
+            }
+          } else {
+            const uint4* row = static_cast<const uint4*>(p.corpus) + row_idx * nvec;
+            uint4 raw[kSimtMaxVec];
+#pragma unroll
+            for (int v = 0; v < kSimtMaxVec; ++v) {
+              const int vi = lane + 32 * v;
+              raw[v] = (v < vec_per_lane && vi < nvec) ? ld_stream(row + vi) : make_uint4(0, 0, 0, 0);
+            }
+#pragma unroll
+            for (int v = 0; v < kSimtMaxVec; ++v) {
+              float x[8];
+              bf16x8_to_f32(raw[v], x);
+#pragma unroll
+              for (int qi = 0; qi < QB; ++qi)
+#pragma unroll
+                for (int e = 0; e < 8; ++e) part[qi] = fmaf(x[e], qreg[qi][v][e], part[qi]);
+            }
           }
 #pragma unroll
           for (int qi = 0; qi < QB; ++qi) {
             float s = part[qi];
 #pragma unroll
             for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
+            if (E8) s = (s * sq[qi]) * sd;
             acc[qi] = fmaf(s_w[qi * p.n_dense + f], s, acc[qi]);
           }
         }
@@ -168,21 +208,31 @@ void score_simt_geometry(int Q, int n_tiles, int* q_pad, int* workers) {
   *workers = w;
 }
 
+template <bool E8>
+static void launch_simt_qb(const SimtParams& p, int Q, int n_dense, int workers, cudaStream_t st) {
+  if (Q == 1) {
+    score_simt_kernel<1, E8><<<workers, kSimtThreads, 1 * n_dense * sizeof(float) + 16, st>>>(p);
+  } else if (Q == 2) {
+    score_simt_kernel<2, E8><<<workers, kSimtThreads, 2 * n_dense * sizeof(float) + 16, st>>>(p);
+  } else {
+    score_simt_kernel<4, E8><<<workers, kSimtThreads, 4 * n_dense * sizeof(float) + 16, st>>>(p);
+  }
+}
+
 int launch_score_simt(const ScoreArgs& a, void* ws_base, int workers, int q_pad, cudaStream_t st) {
   if (a.dim % 8 != 0 || a.dim > kSimtMaxVec * 32 * 8) return MFAR_ERR_SHAPE;
+  const bool e8 = a.corpus_dtype == MFAR_E4M3;
+  if (e8 && a.n_dense > 0 && (!a.corpus_scales || !a.q_scales || reinterpret_cast<uintptr_t>(a.corpus) % 8 ||
+                             reinterpret_cast<uintptr_t>(a.q_vecs) % 8))
+    return MFAR_ERR_ARG;
   SimtParams p;
-  p.corpus = static_cast<const uint4*>(a.corpus);
+  p.corpus = a.corpus; p.corpus_scales = a.corpus_scales; p.q_scales = a.q_scales;
   p.n_docs = a.n_docs; p.n_tiles = a.n_tiles; p.corpus_fields = a.corpus_fields; p.field_begin = a.field_begin;
-  p.n_dense = a.n_dense; p.dim = a.dim; p.q_vecs = static_cast<const __nv_bfloat16*>(a.q_vecs); p.Q = a.Q;
+  p.n_dense = a.n_dense; p.dim = a.dim; p.q_vecs = a.q_vecs; p.Q = a.Q;
   p.w = a.w; p.w_ld = a.w_ld; p.base = a.base; p.base_ld = a.base_ld; p.doc_id_base = a.doc_id_base; p.k = a.k;
   p.ws = carve_workspace(ws_base, workers, q_pad);
-  if (a.Q == 1) {
-    score_simt_kernel<1><<<workers, kSimtThreads, 1 * a.n_dense * sizeof(float) + 16, st>>>(p);
-  } else if (a.Q == 2) {
-    score_simt_kernel<2><<<workers, kSimtThreads, 2 * a.n_dense * sizeof(float) + 16, st>>>(p);
-  } else {
-    score_simt_kernel<4><<<workers, kSimtThreads, 4 * a.n_dense * sizeof(float) + 16, st>>>(p);
-  }
+  if (e8) launch_simt_qb<true>(p, a.Q, a.n_dense, workers, st);
+  else launch_simt_qb<false>(p, a.Q, a.n_dense, workers, st);
   MFAR_CUDA_OK(cudaGetLastError());
   return MFAR_OK;
 }

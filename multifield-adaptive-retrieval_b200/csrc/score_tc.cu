@@ -45,6 +45,8 @@ struct TcParams {
   int64_t sparse_cols;  // columns addressable from `sparse` (<= sparse_ld)
   int n_sparse;
   int sparse_f16;
+  const float* corpus_scales;   // E4M3 corpus: [tiles][corpus_fields][128] row scales
+  const float* q_scales;        // E4M3 queries: [Q]
   int64_t doc_id_base;
   int k;
   int stages;
@@ -137,22 +139,27 @@ __device__ __forceinline__ void tc_stage_sparse(float* base_s, const TcParams& p
 
 // ------------------------------------------------------------------------------------ the kernel
 // QP: query columns per CTA (UMMA N), one of 16 / 32 / 64.
-template <int QP, bool SP>   // SP: sparse fields gathered in-kernel (tc_stage_sparse, 2 more warps); separate instantiation
+// E8: E4M3 corpus and queries.  A K-chunk is still one 128-byte swizzled row span (128 elements instead of 64), so the
+// ring, the descriptors and the producer are those of bf16; the MMA is kind::f8f6f4 (K = 32), and the epilogue applies
+// the query scale (shared memory) and the doc's row scale (one coalesced 512-byte load per (tile, field)) to D_f.
+template <int QP, bool SP, bool E8>   // SP: sparse fields gathered in-kernel (tc_stage_sparse, 2 more warps)
 __global__ void __launch_bounds__(SP ? kTcThreads + kStagerThreads : kTcThreads, 1)
 score_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ CUtensorMap map_b, TcParams p) {
   extern __shared__ __align__(1024) uint8_t smem_raw[];
-  // carve: [A stages][B resident][w_s][thr as float][thr][cnt][flags][barriers][tmem ptr]
+  // carve: [A stages][B resident][w_s][s_q (E8)][thr as float][thr][cnt][flags][barriers][tmem ptr]
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
   uint8_t* smem_a = smem;
   uint8_t* smem_b = smem_a + size_t(p.stages) * kABytes;
-  const int b_chunk_bytes = QP * kChunkK * 2;
-  float* w_s = reinterpret_cast<float*>(smem_b + size_t(p.k_chunks) * b_chunk_bytes);     // [n_dense][QP]
-  float* s_thrf = w_s + size_t(p.n_dense + (SP ? p.n_sparse : 0)) * QP;    // [QP] score of s_thr (float pre-filter), +inf for padding queries
+  constexpr int kChunkElems = E8 ? kChunkK8 : kChunkK;
+  const int b_chunk_bytes = QP * 128;              // QP rows of one 128-byte K-chunk
+  const int n_w = p.n_dense + (SP ? p.n_sparse : 0);   // weight rows kept in shared memory
+  float* w_s = reinterpret_cast<float*>(smem_b + size_t(p.k_chunks) * b_chunk_bytes);     // [n_w][QP]
+  float* sq_s = w_s + size_t(n_w) * QP;            // [QP] query scales (E8)
+  float* s_thrf = sq_s + (E8 ? QP : 0);            // [QP] score of s_thr (float pre-filter), +inf for padding queries
   unsigned long long* s_thr = reinterpret_cast<unsigned long long*>(s_thrf + QP);
   int* s_cnt = reinterpret_cast<int*>(s_thr + QP);
   int* s_flags = s_cnt + QP;                       // reserved (keeps the shared-memory layout)
   float* base_s = reinterpret_cast<float*>((reinterpret_cast<uintptr_t>(s_flags + QP) + 15) & ~uintptr_t(15));   // [QP][128]
-  const int n_w = p.n_dense + (SP ? p.n_sparse : 0);   // weight rows kept in shared memory
   uint64_t* bars = reinterpret_cast<uint64_t*>(
       (reinterpret_cast<uintptr_t>(base_s + (SP ? QP * kTileDocs : 0)) + 7) & ~uintptr_t(7));
   uint64_t* full_bar = bars;                       // [stages]
@@ -177,6 +184,7 @@ score_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant
     const int f = i / QP, c = i % QP;
     w_s[i] = (c < nq) ? p.w[int64_t(q0 + c) * p.w_ld + f] : 0.f;
   }
+  if (E8 && threadIdx.x < QP) sq_s[threadIdx.x] = int(threadIdx.x) < nq ? p.q_scales[q0 + threadIdx.x] : 1.f;
   if (threadIdx.x < QP) {
     s_thr[threadIdx.x] = 0ull; s_cnt[threadIdx.x] = 0; s_flags[threadIdx.x] = 0;
     s_thrf[threadIdx.x] = int(threadIdx.x) < nq ? -INFINITY : INFINITY;
@@ -206,7 +214,7 @@ score_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant
       if (elect_one()) {
         mbar_expect_tx(bq_bar, uint32_t(p.k_chunks) * b_chunk_bytes);
         for (int kc = 0; kc < p.k_chunks; ++kc)
-          tma_load_2d(&map_b, bq_bar, smem_b + size_t(kc) * b_chunk_bytes, kc * kChunkK, q0);
+          tma_load_2d(&map_b, bq_bar, smem_b + size_t(kc) * b_chunk_bytes, kc * kChunkElems, q0);
       }
       __syncwarp();
       int stage = 0; uint32_t phase = 0;
@@ -218,7 +226,7 @@ score_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant
             mbar_wait(&empty_bar[stage], phase ^ 1, err, 1);
             if (elect_one()) {
               mbar_expect_tx(&full_bar[stage], kABytes);
-              tma_load_2d(&map_a, &full_bar[stage], smem_a + size_t(stage) * kABytes, kc * kChunkK, row0);
+              tma_load_2d(&map_a, &full_bar[stage], smem_a + size_t(stage) * kABytes, kc * kChunkElems, row0);
             }
             __syncwarp();
             if (++stage == p.stages) { stage = 0; phase ^= 1; }
@@ -229,7 +237,7 @@ score_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant
   } else if (warp == 1) {
     // ===================================================================== MMA issuer
     if (units > 0) {                                // whole warp walks the loop, one elected lane issues
-      constexpr uint32_t idesc = make_idesc(kTileDocs, QP);
+      constexpr uint32_t idesc = E8 ? make_idesc_e4m3(kTileDocs, QP) : make_idesc(kTileDocs, QP);
       const uint32_t issue = elect_one() ? 1u : 0u;
       mbar_wait(bq_bar, 0, err, 2);
       tc_fence_after();
@@ -246,8 +254,9 @@ score_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant
           const uint64_t b_desc = make_sw128_desc(smem_u32(smem_b + size_t(kc) * b_chunk_bytes));
 #pragma unroll
           for (int kk = 0; kk < kChunkK / kUmmaK; ++kk) {
-            // advance 16 elements = 32 B along K inside the 128 B swizzle span: +2 in the >>4 address field
-            umma_bf16_pred(d_tmem, a_desc + uint64_t(kk * 2), b_desc + uint64_t(kk * 2), idesc, (kc | kk) != 0, issue);
+            // advance 32 B (16 bf16 / 32 E4M3 elements) along K inside the 128 B swizzle span: +2 in the >>4 address field
+            if (E8) umma_e4m3_pred(d_tmem, a_desc + uint64_t(kk * 2), b_desc + uint64_t(kk * 2), idesc, (kc | kk) != 0, issue);
+            else umma_bf16_pred(d_tmem, a_desc + uint64_t(kk * 2), b_desc + uint64_t(kk * 2), idesc, (kc | kk) != 0, issue);
           }
           __syncwarp();
           if (elect_one()) tc_commit(&empty_bar[stage]);   // smem stage reusable once these MMAs retire
@@ -312,6 +321,10 @@ score_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant
       }
       for (int f = 0; f < p.n_dense; ++f, ++u) {
         const int buf = u & 1;
+        // the doc's row scale: 128 consecutive floats per (tile, field), loaded ahead of the wait for the accumulator
+        const float sd = E8 ? __ldg(p.corpus_scales + (int64_t(t) * p.corpus_fields + p.field_begin + f) * kTileDocs +
+                                    doc_in_tile)
+                            : 1.f;
         mbar_wait(&tfull_bar[buf], (u >> 1) & 1, err, 5);
         tc_fence_after();
         const uint32_t taddr = tmem_base + (uint32_t(lane_grp * 32) << 16) + uint32_t(buf * QP);
@@ -324,6 +337,10 @@ score_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant
 #pragma unroll
           for (int c = 0; c < 16; c += 4) {
             const float4 w4 = *reinterpret_cast<const float4*>(wf + c0 + c);
+            if (E8) {                                // w * ((D * s_q) * s_d): two roundings, never s_q * s_d first
+#pragma unroll
+              for (int j = 0; j < 4; ++j) v[c + j] = __float_as_uint((__uint_as_float(v[c + j]) * sq_s[c0 + c + j]) * sd);
+            }
             acc[c0 + c + 0] = fmaf(w4.x, __uint_as_float(v[c + 0]), acc[c0 + c + 0]);
             acc[c0 + c + 1] = fmaf(w4.y, __uint_as_float(v[c + 1]), acc[c0 + c + 1]);
             acc[c0 + c + 2] = fmaf(w4.z, __uint_as_float(v[c + 2]), acc[c0 + c + 2]);
@@ -410,7 +427,8 @@ score_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant
 
 // ------------------------------------------------------------------------------------ host side
 bool score_tc_supported(const ScoreArgs& a) {
-  return a.n_dense >= 1 && a.dim % kChunkK == 0 && a.dim >= kChunkK && a.dim <= 1024 &&
+  const int chunk = a.corpus_dtype == MFAR_E4M3 ? kChunkK8 : kChunkK;
+  return a.n_dense >= 1 && a.dim % chunk == 0 && a.dim >= chunk && a.dim <= 1024 &&
          (reinterpret_cast<uintptr_t>(a.corpus) % 16 == 0) && (reinterpret_cast<uintptr_t>(a.q_vecs) % 16 == 0) &&
          int64_t(a.n_tiles) * a.corpus_fields * kTileDocs < (int64_t(1) << 31);
 }
@@ -425,22 +443,24 @@ void score_tc_geometry(int Q, int n_tiles, int* q_pad, int* q_tiles, int* worker
   *q_pad = qp; *q_tiles = qt; *workers = w;
 }
 
+// n_weights: rows of [QP] floats next to the weights (E8: + the query scales)
 static size_t tc_smem_bytes(int qp, int n_weights, bool sparse, int k_chunks, int stages) {
-  return 1024 + size_t(stages) * kABytes + size_t(k_chunks) * qp * kChunkK * 2 + size_t(n_weights) * qp * 4 +
+  return 1024 + size_t(stages) * kABytes + size_t(k_chunks) * qp * 128 + size_t(n_weights) * qp * 4 +
          size_t(qp) * 20 + 16 + (sparse ? size_t(qp) * kTileDocs * 4 : 0) + 8 + (2 * stages + 7) * 8 + 16;
 }
 
-template <int QP, bool SP>
+template <int QP, bool SP, bool E8>
 static int launch_tc_impl(const ScoreArgs& a, void* ws_base, int workers, int q_tiles, cudaStream_t st) {
   TcParams p;
   p.n_docs = a.n_docs; p.n_tiles = a.n_tiles; p.corpus_fields = a.corpus_fields; p.field_begin = a.field_begin;
-  p.n_dense = a.n_dense; p.k_chunks = a.dim / kChunkK; p.Q = a.Q; p.w = a.w; p.w_ld = a.w_ld; p.base = a.base;
+  p.n_dense = a.n_dense; p.k_chunks = a.dim / (E8 ? kChunkK8 : kChunkK);
+  p.corpus_scales = a.corpus_scales; p.q_scales = a.q_scales; p.Q = a.Q; p.w = a.w; p.w_ld = a.w_ld; p.base = a.base;
   p.base_ld = a.base_ld; p.doc_id_base = a.doc_id_base; p.k = a.k;
   p.sparse = a.sparse; p.sparse_ld = a.sparse_ld; p.n_sparse = a.sparse ? a.n_sparse : 0;
   p.sparse_cols = a.sparse_cols ? a.sparse_cols : a.sparse_ld;
   p.sparse_f16 = a.sparse_dtype == MFAR_F16;
   if (a.sparse && (a.base || !sparse_rows_fusable(a.sparse, a.sparse_dtype, a.sparse_ld))) return MFAR_ERR_ARG;
-  const int n_w = a.n_dense + p.n_sparse;
+  const int n_w = a.n_dense + p.n_sparse + (E8 ? 1 : 0);
   p.ws = carve_workspace(ws_base, workers, q_tiles * QP);
   int stages = 8;
   const size_t smem_cap = 227 * 1024;
@@ -451,34 +471,43 @@ static int launch_tc_impl(const ScoreArgs& a, void* ws_base, int workers, int q_
 
   CUtensorMap map_a, map_b;
   int rc = make_tensor_map_2d(&map_a, a.corpus, uint64_t(a.n_tiles) * a.corpus_fields * kTileDocs, a.dim, kTileDocs,
-                       CU_TENSOR_MAP_L2_PROMOTION_L2_256B);
+                       CU_TENSOR_MAP_L2_PROMOTION_L2_256B, E8);
   if (rc) return rc;
-  rc = make_tensor_map_2d(&map_b, a.q_vecs, uint64_t(a.Q), a.dim, QP, CU_TENSOR_MAP_L2_PROMOTION_L2_128B);
+  rc = make_tensor_map_2d(&map_b, a.q_vecs, uint64_t(a.Q), a.dim, QP, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, E8);
   if (rc) return rc;
 
   static PerDeviceOnce attr_once;   // per template instantiation
   MFAR_CUDA_OK(attr_once.run([&] {
-    return cudaFuncSetAttribute(score_tc_kernel<QP, SP>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem_cap));
+    return cudaFuncSetAttribute(score_tc_kernel<QP, SP, E8>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem_cap));
   }));
   MFAR_CUDA_OK(cudaMemsetAsync(p.ws.progress, 0, workspace_zero_bytes(p.ws.workers, p.ws.q_pad), st));   // shared thresholds
   if (a.gthr_seed) { if (int rc2 = launch_seed_gthr(p.ws.gthr, a.gthr_seed, a.Q, st)) return rc2; }
   dim3 grid(workers, q_tiles);
-  score_tc_kernel<QP, SP><<<grid, SP ? kTcThreads + kStagerThreads : kTcThreads, smem, st>>>(map_a, map_b, p);
+  score_tc_kernel<QP, SP, E8><<<grid, SP ? kTcThreads + kStagerThreads : kTcThreads, smem, st>>>(map_a, map_b, p);
   MFAR_CUDA_OK(cudaGetLastError());
   return MFAR_OK;
 }
 
-int launch_score_tc(const ScoreArgs& a, void* ws_base, int workers, int q_tiles, int q_pad, cudaStream_t st) {
-  if (!score_tc_supported(a)) return MFAR_ERR_SHAPE;
+template <bool E8>
+static int launch_tc_qp(const ScoreArgs& a, void* ws_base, int workers, int q_tiles, int q_pad, cudaStream_t st) {
   switch (q_pad) {
-    case 16: return a.sparse ? launch_tc_impl<16, true>(a, ws_base, workers, q_tiles, st)
-                             : launch_tc_impl<16, false>(a, ws_base, workers, q_tiles, st);
-    case 32: return a.sparse ? launch_tc_impl<32, true>(a, ws_base, workers, q_tiles, st)
-                             : launch_tc_impl<32, false>(a, ws_base, workers, q_tiles, st);
-    case 64: return a.sparse ? launch_tc_impl<64, true>(a, ws_base, workers, q_tiles, st)
-                             : launch_tc_impl<64, false>(a, ws_base, workers, q_tiles, st);
+    case 16: return a.sparse ? launch_tc_impl<16, true, E8>(a, ws_base, workers, q_tiles, st)
+                             : launch_tc_impl<16, false, E8>(a, ws_base, workers, q_tiles, st);
+    case 32: return a.sparse ? launch_tc_impl<32, true, E8>(a, ws_base, workers, q_tiles, st)
+                             : launch_tc_impl<32, false, E8>(a, ws_base, workers, q_tiles, st);
+    case 64: return a.sparse ? launch_tc_impl<64, true, E8>(a, ws_base, workers, q_tiles, st)
+                             : launch_tc_impl<64, false, E8>(a, ws_base, workers, q_tiles, st);
     default: return MFAR_ERR_SHAPE;
   }
+}
+
+int launch_score_tc(const ScoreArgs& a, void* ws_base, int workers, int q_tiles, int q_pad, cudaStream_t st) {
+  if (!score_tc_supported(a)) return MFAR_ERR_SHAPE;
+  if (a.corpus_dtype == MFAR_E4M3) {
+    if (!a.corpus_scales || !a.q_scales) return MFAR_ERR_ARG;
+    return launch_tc_qp<true>(a, ws_base, workers, q_tiles, q_pad, st);
+  }
+  return launch_tc_qp<false>(a, ws_base, workers, q_tiles, q_pad, st);
 }
 
 }  // namespace mfar

@@ -8,6 +8,7 @@
 namespace mfar {
 
 constexpr int kChunkK = 64;   // bf16 elements per K-chunk = 128 B = swizzle span
+constexpr int kChunkK8 = 128; // E4M3 elements per K-chunk: the same 128 B span, consumed by 4 MMAs of K = 32
 constexpr int kUmmaK = 16;
 constexpr int kEpiThreads = 128;   // 4 epilogue warps: one per 32-lane TMEM sub-partition
 #ifdef MFAR_TIMEOUT_EXIT
@@ -147,6 +148,10 @@ __device__ __forceinline__ uint64_t make_sw128_desc(uint32_t smem_addr) {
 __host__ __device__ constexpr uint32_t make_idesc(int M, int N) {
   return (1u << 4) | (1u << 7) | (1u << 10) | (uint32_t(N >> 3) << 17) | (uint32_t(M >> 4) << 24);
 }
+// kind::f8f6f4 instruction descriptor: D=f32 (bit 4), A=B=E4M3 (format 0 in bits [7,10) and [10,13)), K-major both
+__host__ __device__ constexpr uint32_t make_idesc_e4m3(int M, int N) {
+  return (1u << 4) | (uint32_t(N >> 3) << 17) | (uint32_t(M >> 4) << 24);
+}
 
 
 // ------------------------------------------------------------------------------------ CTA pairs (cta_group::2)
@@ -222,6 +227,16 @@ __device__ __forceinline__ void umma_bf16_pred(uint32_t d_tmem, uint64_t a_desc,
       "@e tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}"
       ::"r"(d_tmem), "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(accumulate), "r"(issue) : "memory");
 }
+// E4M3 x E4M3 -> fp32 (kind::f8f6f4, K = 32 per instruction: the same 32 bytes of a K-chunk as one bf16 MMA)
+__device__ __forceinline__ void umma_e4m3_pred(uint32_t d_tmem, uint64_t a_desc, uint64_t b_desc, uint32_t idesc,
+                                               uint32_t accumulate, uint32_t issue) {
+  asm volatile(
+      "{\n\t.reg .pred p, e;\n\t"
+      "setp.ne.b32 p, %4, 0;\n\t"
+      "setp.ne.b32 e, %5, 0;\n\t"
+      "@e tcgen05.mma.cta_group::1.kind::f8f6f4 [%0], %1, %2, %3, p;\n\t}"
+      ::"r"(d_tmem), "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(accumulate), "r"(issue) : "memory");
+}
 __device__ __forceinline__ void umma_bf16_ts_pred(uint32_t d_tmem, uint32_t a_tmem, uint64_t b_desc, uint32_t idesc,
                                                   uint32_t accumulate, uint32_t issue) {
   asm volatile(
@@ -266,16 +281,17 @@ static inline PFN_encodeTiled get_encode_fn() {
   return fn;
 }
 
-// 2-D bf16 row-major [rows, cols] tensor, box = [box_rows, 64 cols], 128-byte swizzle.
+// 2-D row-major [rows, cols] tensor, box = [box_rows, 128 bytes of cols], 128-byte swizzle: bf16 (64 cols) or, with
+// e4m3, bytes (128 cols).
 static inline int make_tensor_map_2d(CUtensorMap* map, const void* base, uint64_t rows, uint64_t cols, uint32_t box_rows,
-                       CUtensorMapL2promotion promo) {
+                       CUtensorMapL2promotion promo, bool e4m3 = false) {
   PFN_encodeTiled enc = get_encode_fn();
   if (!enc) return MFAR_ERR_CUDA;
   cuuint64_t gdim[2] = {cols, rows};
-  cuuint64_t gstride[1] = {cols * 2};
-  cuuint32_t box[2] = {kChunkK, box_rows};
+  cuuint64_t gstride[1] = {cols * (e4m3 ? 1 : 2)};
+  cuuint32_t box[2] = {cuuint32_t(e4m3 ? kChunkK8 : kChunkK), box_rows};
   cuuint32_t estr[2] = {1, 1};
-  CUresult r = enc(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(base), gdim, gstride, box, estr,
+  CUresult r = enc(map, e4m3 ? CU_TENSOR_MAP_DATA_TYPE_UINT8 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(base), gdim, gstride, box, estr,
                    CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, promo, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   if (r != CUDA_SUCCESS) {
     fprintf(stderr, "[mfar_b200] cuTensorMapEncodeTiled failed: %d\n", int(r));

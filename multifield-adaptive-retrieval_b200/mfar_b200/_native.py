@@ -11,7 +11,7 @@ import os
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("MFAR_LIB") or os.path.join(_HERE, "libmfar_b200.so")   # MFAR_LIB: instrumented builds
 
-F32, BF16, F16 = 0, 1, 2
+F32, BF16, F16, E4M3 = 0, 1, 2, 3
 IMPL = {"auto": 0, "simt": 1, "tcgen05": 2, "tcgen05_qs": 3}
 TILE_DOCS = 128
 MAX_K = 128
@@ -29,6 +29,8 @@ PROTOTYPES = {
     "mfar_corpus_packed_elems": (_i64, [_i64, _i, _i]),
     "mfar_corpus_pack_rows": (_i, [_vp, _i, _i64, _i64, _vp, _i64, _i, _i, _i, _i, _vp]),
     "mfar_corpus_unpack_rows": (_i, [_vp, _i64, _i, _i, _i, _i64, _i64, _vp, _vp]),
+    "mfar_corpus_pack_rows_e4m3": (_i, [_vp, _i, _i64, _i64, _vp, _vp, _i64, _i, _i, _i, _i, _vp]),
+    "mfar_corpus_unpack_rows_e4m3": (_i, [_vp, _vp, _i64, _i, _i, _i, _i64, _i64, _vp, _vp]),
     "mfar_mixture_weights": (_i, [_vp, _vp, _vp, _i, _i, _i, _i, _vp, _vp]),
     "mfar_mixture_apply": (_i, [_vp, _vp, _i, _i, _i, _i, _vp, _vp]),
     "mfar_score_topk_workspace_bytes": (_sz, [_i, _i, _i64, _i]),
@@ -36,6 +38,13 @@ PROTOTYPES = {
                              _vp, _sz, _i, _vp]),
     "mfar_score_topk_coo": (_i, [_vp, _i64, _i, _i, _i, _i, _vp, _i, _vp, _vp, _vp, _i, _vp, _i, _i64, _i, _vp, _vp, _vp,
                                  _vp, _sz, _i, _vp]),
+    "mfar_score_topk_e4m3": (_i, [_vp, _vp, _i64, _i, _i, _i, _i, _vp, _vp, _i, _vp, _vp, _i, _i, _i64, _i64, _i, _vp,
+                                  _vp, _vp, _vp, _sz, _i, _vp]),
+    "mfar_score_topk_coo_e4m3": (_i, [_vp, _vp, _i64, _i, _i, _i, _i, _vp, _vp, _i, _vp, _vp, _vp, _i, _vp, _i, _i64, _i,
+                                      _vp, _vp, _vp, _vp, _sz, _i, _vp]),
+    "mfar_score_topk_bm25_e4m3": (_i, [_vp, _vp, _i64, _i, _i, _i, _i, _vp, _vp, _i, _vp, _vp, _vp, _vp, _vp, _i, _vp,
+                                       _i64, _i64, _i, _vp, _vp, _vp, _vp, _sz, _i, _vp]),
+    "mfar_score_candidates_e4m3": (_i, [_vp, _vp, _i64, _i, _i, _i, _i, _vp, _vp, _i, _vp, _i, _vp, _vp]),
     "mfar_topk_merge": (_i, [_vp, _i, _i, _i, _i, _vp, _vp, _vp, _vp]),
     "mfar_exchange_buffer_bytes": (_sz, [_i, _i, _i]),
     "mfar_topk_exchange_merge": (_i, [_vp, _i, _i, _i, _i, _i, _vp, _i, _i, _i, _vp, _vp, _vp, _vp]),

@@ -1,8 +1,8 @@
 """Multi-field retrieval over the packed corpus: the B200 replacement of
 ``RetrievalTrainingModule.trec_eval_step`` / ``mask_field`` (mfar/modeling/contrastive.py:669-714).
 
-``PackedCorpus``         - device-resident bf16 corpus [tiles][F][128][dim] built from the
-                           reference's per-field fp32 memmaps (or any [N,d] slabs)
+``PackedCorpus``         - device-resident bf16 (or E4M3 + per-row scale) corpus [tiles][F][128][dim] built from
+                           the reference's per-field fp32 memmaps (or any [N,d] slabs)
 ``MultiFieldRetriever``  - exhaustive fused scoring + mixture + top-k (``search``), the
                            reference-faithful union/rescore pipeline (``union_rescore``), field
                            masking, per-field top-k, QRes emission
@@ -20,6 +20,8 @@ from .weighting import LinearWeights
 
 TILE_DOCS = nv.TILE_DOCS
 KCHUNK = 64   # the tensor-core path consumes K in 64-element (128-byte) chunks
+KCHUNK_E4M3 = 128   # ... and an E4M3 corpus in 128-element (128-byte) chunks
+DTYPES = ("bf16", "e4m3")
 
 
 def _round_up(x: int, m: int) -> int:
@@ -30,19 +32,35 @@ class PackedCorpus:
     """bf16 corpus in the tile layout the scoring kernels stream (include/mfar_b200.h).
 
     ``dim`` is zero-padded to a multiple of 64 (dot products are unchanged); queries are padded
-    the same way by ``prepare_queries``."""
+    the same way by ``prepare_queries``.
 
-    def __init__(self, n_docs: int, n_fields: int, dim: int, device="cuda", normalize: bool = False):
+    ``dtype="e4m3"`` stores one E4M3 byte per element (``data`` is uint8, ``dim`` padded to a multiple of 128) and one
+    power-of-two fp32 scale per (doc, field) row (``scales``, [tiles][F][128]): half the bytes of bf16, scored at the
+    tensor cores' FP8 rate.  The dequantized values are bf16 numbers, so a search equals the bf16 search of the
+    dequantized corpus up to fp32 summation order (``mfar_corpus_pack_rows_e4m3`` states the rounding rule)."""
+
+    def __init__(self, n_docs: int, n_fields: int, dim: int, device="cuda", normalize: bool = False,
+                 dtype: str = "bf16"):
         if n_docs <= 0 or n_fields <= 0 or dim <= 0:
             raise ValueError("n_docs, n_fields, dim must be positive")
+        if dtype not in DTYPES:
+            raise ValueError(f"dtype must be one of {DTYPES}, got {dtype!r}")
         self.device = torch.device(device)
         if self.device.type != "cuda":
             raise RuntimeError("PackedCorpus lives in HBM: device must be CUDA (no CPU path)")
         self.n_docs, self.n_fields, self.dim = int(n_docs), int(n_fields), int(dim)
-        self.dim_pad = _round_up(self.dim, KCHUNK)
+        self.dtype = dtype
+        self.dim_pad = _round_up(self.dim, KCHUNK_E4M3 if self.e4m3 else KCHUNK)
         self.normalize = bool(normalize)
         n_el = nv.lib().mfar_corpus_packed_elems(self.n_docs, self.n_fields, self.dim_pad)
-        self.data = torch.zeros(n_el, dtype=torch.bfloat16, device=self.device)
+        self.data = torch.zeros(n_el, dtype=torch.uint8 if self.e4m3 else torch.bfloat16, device=self.device)
+        # tail rows of the last tile: payload 0, scale 1
+        self.scales = (torch.ones(n_el // self.dim_pad, dtype=torch.float32, device=self.device) if self.e4m3
+                       else None)
+
+    @property
+    def e4m3(self) -> bool:
+        return self.dtype == "e4m3"
 
     # ------------------------------------------------------------------ loading
     def load_rows(self, field: int, row_begin: int, rows: torch.Tensor) -> None:
@@ -56,6 +74,12 @@ class PackedCorpus:
             r = torch.nn.functional.pad(r, (0, self.dim_pad - self.dim))
         r = r.contiguous()
         code = nv.F32 if r.dtype == torch.float32 else nv.BF16
+        if self.e4m3:
+            nv.check(nv.lib().mfar_corpus_pack_rows_e4m3(nv.ptr(r), code, r.shape[0], int(row_begin), nv.ptr(self.data),
+                                                         nv.ptr(self.scales), self.n_docs, self.n_fields, int(field),
+                                                         self.dim_pad, int(self.normalize), nv.stream()),
+                     "corpus_pack_rows_e4m3")
+            return
         nv.check(nv.lib().mfar_corpus_pack_rows(nv.ptr(r), code, r.shape[0], int(row_begin), nv.ptr(self.data),
                                                 self.n_docs, self.n_fields, int(field), self.dim_pad,
                                                 int(self.normalize), nv.stream()), "corpus_pack_rows")
@@ -73,19 +97,19 @@ class PackedCorpus:
             self.load_rows(field, lb, chunk)
 
     @classmethod
-    def from_fields(cls, fields: Sequence, device="cuda", normalize: bool = False) -> "PackedCorpus":
+    def from_fields(cls, fields: Sequence, device="cuda", normalize: bool = False, dtype: str = "bf16") -> "PackedCorpus":
         """fields: F array-likes [N, dim], in scorer column order (``resolve_fields`` order)."""
         n, d = fields[0].shape
-        pc = cls(n, len(fields), d, device, normalize)
+        pc = cls(n, len(fields), d, device, normalize, dtype)
         for f, v in enumerate(fields):
             pc.load_field(f, v)
         return pc
 
     @classmethod
     def from_vectors_dict(cls, vectors_dict: Dict[str, "object"], dense_keys: Sequence[str], device="cuda",
-                          normalize: bool = False) -> "PackedCorpus":
+                          normalize: bool = False, dtype: str = "bf16") -> "PackedCorpus":
         """vectors_dict: field key -> MemoryMapDict, as returned by ``read_and_create_indices``."""
-        return cls.from_fields([vectors_dict[k].file for k in dense_keys], device, normalize)
+        return cls.from_fields([vectors_dict[k].file for k in dense_keys], device, normalize, dtype)
 
     def window(self, doc_begin: int, n_docs: int) -> "PackedCorpus":
         """Docs [doc_begin, doc_begin + n_docs) as a corpus of their own WITHOUT a copy (the layout is tile-major, so a
@@ -96,32 +120,58 @@ class PackedCorpus:
                              f"inside the corpus of {self.n_docs} docs")
         view = PackedCorpus.__new__(PackedCorpus)
         view.device, view.n_fields, view.dim, view.dim_pad = self.device, self.n_fields, self.dim, self.dim_pad
-        view.normalize, view.n_docs = self.normalize, int(n_docs)
+        view.normalize, view.n_docs, view.dtype = self.normalize, int(n_docs), self.dtype
         per_tile = self.n_fields * TILE_DOCS * self.dim_pad
         n_el = nv.lib().mfar_corpus_packed_elems(view.n_docs, self.n_fields, self.dim_pad)
         first = (doc_begin // TILE_DOCS) * per_tile
         view.data = self.data[first:first + n_el]
+        view.scales = None
+        if self.e4m3:
+            first_row = (doc_begin // TILE_DOCS) * self.n_fields * TILE_DOCS
+            view.scales = self.scales[first_row:first_row + n_el // self.dim_pad]
         return view
 
     def unpack_field(self, field: int, row_begin: int = 0, n_rows: Optional[int] = None) -> torch.Tensor:
         n_rows = self.n_docs - row_begin if n_rows is None else n_rows
         out = torch.empty((n_rows, self.dim_pad), dtype=torch.float32, device=self.device)
+        if self.e4m3:                                 # exact: every dequantized value is a normal fp32 number
+            nv.check(nv.lib().mfar_corpus_unpack_rows_e4m3(nv.ptr(self.data), nv.ptr(self.scales), self.n_docs,
+                                                           self.n_fields, int(field), self.dim_pad, int(row_begin),
+                                                           int(n_rows), nv.ptr(out), nv.stream()),
+                     "corpus_unpack_rows_e4m3")
+            return out[:, : self.dim]
         nv.check(nv.lib().mfar_corpus_unpack_rows(nv.ptr(self.data), self.n_docs, self.n_fields, int(field),
                                                   self.dim_pad, int(row_begin), int(n_rows), nv.ptr(out), nv.stream()),
                  "corpus_unpack_rows")
         return out[:, : self.dim]
 
-    def prepare_queries(self, q_vecs) -> torch.Tensor:
+    def prepare_queries(self, q_vecs):
         """[Q, dim] (any float dtype, host or device) -> contiguous bf16 [Q, dim_pad] on the device.
 
         On a cosine corpus the queries are normalised by the kernel that packs the docs, so both sides are rounded to
         bf16 once, by the same arithmetic: with one field the packed layout [tile][1][128][dim_pad] of Q rows is plain
-        row-major [Q, dim_pad].  Inputs other than fp32 / bf16 are taken to fp32 first, as in ``load_rows``."""
+        row-major [Q, dim_pad].  Inputs other than fp32 / bf16 are taken to fp32 first, as in ``load_rows``.
+
+        On an E4M3 corpus the queries are quantized by the kernel that packs the docs, by the same rule, and the call
+        returns (uint8 payload [Q, dim_pad], fp32 scales [Q])."""
         if not torch.is_tensor(q_vecs):
             q_vecs = torch.from_numpy(np.ascontiguousarray(q_vecs))
         if q_vecs.dim() != 2 or q_vecs.shape[1] != self.dim:
             raise ValueError(f"expected [Q,{self.dim}] query vectors, got {tuple(q_vecs.shape)}")
         q = q_vecs.to(self.device)
+        if self.e4m3:
+            if q.dtype not in (torch.float32, torch.bfloat16):
+                q = q.float()
+            if self.dim_pad != self.dim:
+                q = torch.nn.functional.pad(q, (0, self.dim_pad - self.dim))
+            q = q.contiguous()
+            out = torch.empty((q.shape[0], self.dim_pad), dtype=torch.uint8, device=self.device)
+            qs = torch.empty((q.shape[0],), dtype=torch.float32, device=self.device)
+            if q.shape[0]:
+                nv.check(nv.lib().mfar_corpus_pack_rows_e4m3(
+                    nv.ptr(q), nv.F32 if q.dtype == torch.float32 else nv.BF16, q.shape[0], 0, nv.ptr(out), nv.ptr(qs),
+                    q.shape[0], 1, 0, self.dim_pad, int(self.normalize), nv.stream()), "corpus_pack_rows_e4m3 (queries)")
+            return out, qs
         if self.normalize:
             if q.dtype not in (torch.float32, torch.bfloat16):
                 q = q.float()
@@ -226,10 +276,22 @@ class MultiFieldRetriever:
             sparse = sparse.float()
         return sparse.contiguous(), (nv.F16 if sparse.dtype == torch.float16 else nv.F32)
 
+    def _queries(self, q_vecs) -> Tuple[Optional[torch.Tensor], Optional[torch.Tensor]]:
+        """(query operand, query scales) of a call: bf16 rows and None, or E4M3 rows and their fp32 scales."""
+        if self.corpus is None:
+            return None, None
+        q = self.corpus.prepare_queries(q_vecs)
+        return q if self.corpus.e4m3 else (q, None)
+
+    def _require_bf16(self, what: str) -> None:
+        if self.corpus is not None and self.corpus.e4m3:
+            raise ValueError(f"{what} runs on a bf16 corpus only; this corpus is E4M3 (use search / score_candidates)")
+
     def _score_topk(self, q_bf16: Optional[torch.Tensor], w: torch.Tensor, sparse, sparse_code: int, k: int,
                     field_begin: int, n_dense: int, n_sparse: int, want_keys: bool = False, impl: Optional[str] = None,
                     n_docs: Optional[int] = None, doc_id_base: Optional[int] = None, sparse_coo=None,
-                    bm25_entries: Optional[torch.Tensor] = None):
+                    bm25_entries: Optional[torch.Tensor] = None, q_scales: Optional[torch.Tensor] = None):
+        """``q_bf16``: the query operand (bf16, or E4M3 bytes with ``q_scales`` on an E4M3 corpus)."""
         Q = w.shape[0]
         n_docs = self.n_docs if n_docs is None else n_docs
         doc_id_base = self.doc_id_base if doc_id_base is None else doc_id_base
@@ -240,9 +302,20 @@ class MultiFieldRetriever:
         keys = torch.empty((Q, k), dtype=torch.int64, device=self.device) if want_keys else None
         ws = self._workspace(Q, k, n_sparse, n_docs, 0 if bm25_entries is None else bm25_entries.shape[0])
         c = self.corpus
+        e8 = c is not None and c.e4m3
+        if e8:
+            # the *_e4m3 entry points: the bf16 arguments with the corpus / query scale pointers after their operands
+            lib = nv.lib()
+            sc, qs = nv.ptr(c.scales), nv.ptr(q_scales)
+            ep = {"bm25": lambda cp, *a: lib.mfar_score_topk_bm25_e4m3(cp, sc, *a[:6], qs, *a[6:]),
+                  "coo": lambda cp, *a: lib.mfar_score_topk_coo_e4m3(cp, sc, *a[:6], qs, *a[6:]),
+                  "dense": lambda cp, *a: lib.mfar_score_topk_e4m3(cp, sc, *a[:6], qs, *a[6:])}
+        else:
+            ep = {"bm25": nv.lib().mfar_score_topk_bm25, "coo": nv.lib().mfar_score_topk_coo,
+                  "dense": nv.lib().mfar_score_topk}
         if bm25_entries is not None:
             b = self.bm25
-            nv.check(nv.lib().mfar_score_topk_bm25(
+            nv.check(ep["bm25"](
                 nv.ptr(c.data) if c is not None else 0, n_docs, c.n_fields if c is not None else 0, field_begin,
                 n_dense, c.dim_pad if c is not None else 0, nv.ptr(q_bf16), Q, nv.ptr(w), b.indptr, b.indices, b.data,
                 b.vocab, n_sparse, nv.ptr(bm25_entries), bm25_entries.shape[0], doc_id_base, k, nv.ptr(keys),
@@ -254,7 +327,7 @@ class MultiFieldRetriever:
             import ctypes
             coo_keys, coo_vals, offsets = sparse_coo
             off = (ctypes.c_int64 * (n_sparse + 1))(*[int(x) for x in offsets])
-            nv.check(nv.lib().mfar_score_topk_coo(
+            nv.check(ep["coo"](
                 nv.ptr(c.data) if c is not None else 0, n_docs, c.n_fields if c is not None else 0, field_begin,
                 n_dense, c.dim_pad if c is not None else 0, nv.ptr(q_bf16), Q, nv.ptr(w), nv.ptr(coo_keys),
                 nv.ptr(coo_vals), nv.F16 if coo_vals.dtype == torch.float16 else nv.F32, ctypes.addressof(off), n_sparse,
@@ -262,7 +335,7 @@ class MultiFieldRetriever:
                 nv.IMPL[impl or self.impl], nv.stream()), "score_topk_coo")
             self.last_launches = nv.lib().mfar_last_launch_count()
             return scores, ids, keys
-        nv.check(nv.lib().mfar_score_topk(
+        nv.check(ep["dense"](
             nv.ptr(c.data) if c is not None else 0, n_docs, c.n_fields if c is not None else 0, field_begin,
             n_dense, c.dim_pad if c is not None else 0, nv.ptr(q_bf16), Q, nv.ptr(w), nv.ptr(sparse), n_sparse,
             sparse_code, (sparse.shape[2] if sparse is not None else n_docs), doc_id_base, k, nv.ptr(keys),
@@ -333,7 +406,7 @@ class MultiFieldRetriever:
         ``torch.topk`` ranks them), then +inf, finite, -inf; with
         return_keys also the packed uint64 keys (as int64) used for cross-shard merging."""
         k = top_k or self.top_k
-        q_bf16 = self.corpus.prepare_queries(q_vecs) if self.corpus is not None else None
+        q_bf16, q_sc = self._queries(q_vecs)
         if q_bf16 is None and sparse is None and batch is None and q_emb is not None and (
                 sparse_tokens is None or torch.is_tensor(sparse_tokens)):
             batch = int(q_emb.shape[0])
@@ -343,7 +416,7 @@ class MultiFieldRetriever:
         if sparse_tokens is not None:
             ent = self._bm25_entries(sparse_tokens)
             scores, ids, keys = self._score_topk(q_bf16, w, None, nv.F16, k, 0, self.n_dense, self.n_sparse,
-                                                 want_keys=return_keys, impl=impl, bm25_entries=ent)
+                                                 want_keys=return_keys, impl=impl, bm25_entries=ent, q_scales=q_sc)
             return (scores, ids, keys) if return_keys else (scores, ids)
         if sparse_coo is not None:
             if self.n_sparse == 0:
@@ -358,11 +431,11 @@ class MultiFieldRetriever:
                 cv = cv.float()
             scores, ids, keys = self._score_topk(q_bf16, w, None, nv.F16, k, 0, self.n_dense, self.n_sparse,
                                                  want_keys=return_keys, impl=impl,
-                                                 sparse_coo=(ck.contiguous(), cv.contiguous(), off))
+                                                 sparse_coo=(ck.contiguous(), cv.contiguous(), off), q_scales=q_sc)
             return (scores, ids, keys) if return_keys else (scores, ids)
         sp, code = self._check_sparse(sparse, Q)
         scores, ids, keys = self._score_topk(q_bf16, w, sp, code, k, 0, self.n_dense, self.n_sparse,
-                                             want_keys=return_keys, impl=impl)
+                                             want_keys=return_keys, impl=impl, q_scales=q_sc)
         return (scores, ids, keys) if return_keys else (scores, ids)
 
     # ------------------------------------------------------------------ field-masking sweep in one corpus pass
@@ -396,7 +469,7 @@ class MultiFieldRetriever:
         at most ``max_rows`` pseudo-queries; dense sparse-score tensors are repeated per chunk, BM25 token entries
         (``sparse_tokens``, for a retriever with ``sparse_indices``) are replicated with shifted query rows."""
         k = top_k or self.top_k
-        q_bf16 = self.corpus.prepare_queries(q_vecs) if self.corpus is not None else None
+        q_bf16, q_sc = self._queries(q_vecs)
         ent = self._bm25_entries(sparse_tokens) if sparse_tokens is not None else None
         Q = self._batch_size(q_bf16, sparse, sparse_tokens, batch)
         qe = self.mixture_input(q_vecs, q_emb)
@@ -414,6 +487,7 @@ class MultiFieldRetriever:
             reps = m1 - m0
             w_rows = (w.unsqueeze(0) * masks[m0:m1].unsqueeze(1)).reshape(reps * Q, -1).contiguous()
             q_rows = q_bf16.repeat(reps, 1) if q_bf16 is not None else None
+            qs_rows = q_sc.repeat(reps) if q_sc is not None else None
             sp_rows = sp.repeat(reps, 1, 1) if sp is not None else None
             ent_rows = None
             if ent is not None:                                            # query-major order is kept: rep-major
@@ -421,7 +495,7 @@ class MultiFieldRetriever:
                 ent_rows[:, :, 0] += (torch.arange(reps, device=self.device, dtype=torch.int32) * Q).view(reps, 1)
                 ent_rows = ent_rows.view(-1, 3).contiguous()
             s, i, _ = self._score_topk(q_rows, w_rows, sp_rows, code, k, 0, self.n_dense, self.n_sparse,
-                                       bm25_entries=ent_rows)
+                                       bm25_entries=ent_rows, q_scales=qs_rows)
             out_s[m0:m1] = s.view(reps, Q, k)
             out_i[m0:m1] = i.view(reps, Q, k)
         return out_s, out_i
@@ -433,7 +507,8 @@ class MultiFieldRetriever:
                     impl: Optional[str] = None):
         """One C-ABI call with HOST buffers (``mfar_search_host``): H2D of the batch, mixture weights,
         fused scoring + top-k, D2H of the [Q,k] result, stream sync.  q_vecs_host: bf16 [Q,dim_pad] host tensor
-        (pinned for full PCIe speed); q_emb_host fp32 [Q,E]; sparse_host f16/f32 [Q,Fs,N]."""
+        (pinned for full PCIe speed); q_emb_host fp32 [Q,E]; sparse_host f16/f32 [Q,Fs,N].  bf16 corpus only."""
+        self._require_bf16("search_host")
         k = top_k or self.top_k
         c = self.corpus
         Q = q_vecs_host.shape[0] if q_vecs_host is not None else sparse_host.shape[0]
@@ -476,6 +551,7 @@ class MultiFieldRetriever:
         (``BM25FieldSet.entries_host``, ideally pinned) cross PCIe."""
         if self.bm25 is None:
             raise ValueError("search_host_bm25 needs a retriever built with sparse_indices=[DeviceBM25, ...]")
+        self._require_bf16("search_host_bm25")
         k = top_k or self.top_k
         c = self.corpus
         if q_vecs_host is not None:
@@ -523,14 +599,14 @@ class MultiFieldRetriever:
         (scores [F,Q,k], rows [F,Q,k]).  Dense fields reproduce the reference's (0.0, row 0) running-top-k
         initialisation (index.py:192-193) when zero_init is set."""
         k = top_k or self.top_k
-        q_bf16 = self.corpus.prepare_queries(q_vecs) if self.corpus is not None else None
+        q_bf16, q_sc = self._queries(q_vecs)
         sparse = self._sparse_from_tokens(sparse, sparse_tokens, q_bf16, batch)
         Q = self._batch_size(q_bf16, sparse, None, batch)
         sp, code = self._check_sparse(sparse, Q)
         ones = torch.ones((Q, 1), dtype=torch.float32, device=self.device)
         all_s, all_i, launches = [], [], 0
         for f in range(self.n_dense):
-            s, i, _ = self._score_topk(q_bf16, ones, None, nv.F16, k, f, 1, 0)
+            s, i, _ = self._score_topk(q_bf16, ones, None, nv.F16, k, f, 1, 0, q_scales=q_sc)
             launches += self.last_launches
             i = i - self.doc_id_base
             if zero_init:
@@ -552,7 +628,7 @@ class MultiFieldRetriever:
     def score_candidates(self, q_vecs, rows: torch.Tensor, sparse: Optional[torch.Tensor] = None,
                          sparse_tokens=None, batch: Optional[int] = None) -> torch.Tensor:
         """Per-field scores of the given local rows: [F, Q, C] (rows < 0 -> 0, index.py:112-117)."""
-        q_bf16 = self.corpus.prepare_queries(q_vecs) if self.corpus is not None else None
+        q_bf16, q_sc = self._queries(q_vecs)
         sparse = self._sparse_from_tokens(sparse, sparse_tokens, q_bf16, batch)
         Q = self._batch_size(q_bf16, sparse, None, batch)
         rows = rows.to(self.device, dtype=torch.int64).contiguous()
@@ -560,9 +636,15 @@ class MultiFieldRetriever:
         out = torch.zeros((self.num_fields, Q, C), dtype=torch.float32, device=self.device)
         if self.n_dense and C:
             c = self.corpus
-            nv.check(nv.lib().mfar_score_candidates(nv.ptr(c.data), self.n_docs, c.n_fields, 0, self.n_dense,
-                                                    c.dim_pad, nv.ptr(q_bf16), Q, nv.ptr(rows), C, nv.ptr(out),
-                                                    nv.stream()), "score_candidates")
+            if c.e4m3:
+                nv.check(nv.lib().mfar_score_candidates_e4m3(nv.ptr(c.data), nv.ptr(c.scales), self.n_docs, c.n_fields,
+                                                             0, self.n_dense, c.dim_pad, nv.ptr(q_bf16), nv.ptr(q_sc),
+                                                             Q, nv.ptr(rows), C, nv.ptr(out), nv.stream()),
+                         "score_candidates_e4m3")
+            else:
+                nv.check(nv.lib().mfar_score_candidates(nv.ptr(c.data), self.n_docs, c.n_fields, 0, self.n_dense,
+                                                        c.dim_pad, nv.ptr(q_bf16), Q, nv.ptr(rows), C, nv.ptr(out),
+                                                        nv.stream()), "score_candidates")
         if self.n_sparse and C:
             sp, _ = self._check_sparse(sparse, Q)
             g = sp[:, :, rows.clamp(min=0)].float()                       # [Q,Fs,C] gather (index.py:116)
@@ -579,7 +661,9 @@ class MultiFieldRetriever:
         ``retrieve_batch``, contrastive.py:672-674) then ONE kernel (``mfar_union_rescore``) for per-query union ->
         rescore under every field -> * mask -> mixture -> top-k (676-696).
         Returns (values [Q,k], local rows [Q,k], union sizes [Q]); rows of a query whose union is smaller than k are
-        padded with (-inf, -1) - ``union_rescore`` raises for those, like the reference's ``torch.topk``."""
+        padded with (-inf, -1) - ``union_rescore`` raises for those, like the reference's ``torch.topk``.
+        bf16 corpus only."""
+        self._require_bf16("union_rescore")
         k = top_k or self.top_k
         q_bf16 = self.corpus.prepare_queries(q_vecs) if self.corpus is not None else None
         if sparse_tokens is not None:                                      # BM25 get_scores once per (query, field)
@@ -660,7 +744,8 @@ class GraphedSearch:
         # a cosine corpus normalises the query it is given: the static buffer keeps fp32 queries unrounded, so the graph
         # rounds them to bf16 once, after the normalisation, as the eager search does (without normalisation the one
         # rounding is the copy into a bf16 buffer)
-        q_dtype = torch.float32 if r.corpus is not None and r.corpus.normalize else torch.bfloat16
+        # (an E4M3 corpus likewise quantizes fp32 queries inside the graph)
+        q_dtype = torch.float32 if r.corpus is not None and (r.corpus.normalize or r.corpus.e4m3) else torch.bfloat16
         self.q_vecs = torch.zeros((self.Q, dim), dtype=q_dtype, device=dev) if r.corpus is not None else None
         E = r.mixture.weight.shape[0] if r.mixture.query_cond else 0
         self.q_emb = torch.zeros((self.Q, E), dtype=torch.float32, device=dev) if E else None
