@@ -235,10 +235,6 @@ MFAR_API int mfar_score_topk_bm25(const void* corpus, int64_t n_docs, int corpus
                                   uint64_t* out_keys, float* out_scores, int64_t* out_ids, void* workspace,
                                   size_t workspace_bytes, int impl, void* stream);
 
-/* Merge L sorted-or-unsorted key lists per query into the global top-k.  Used for (a) the
- * per-CTA partial lists inside mfar_score_topk and (b) the per-shard lists after the NCCL
- * all-gather (replaces the {rank}.qres file merge of mfar/modeling/contrastive.py:616-631).
- * keys: uint64 [L, Q, k_in]; key 0 = empty slot. */
 /* The three entry points above on an E4M3 corpus (mfar_corpus_pack_rows_e4m3) and E4M3 queries: same arguments, plus
  * corpus_scales fp32 [n_tiles][corpus_fields][128] and q_scales fp32 [Q]; q_vecs is uint8 [Q, dim].
  *   score[q,n] = sum_f fmaf-accumulated  w[q,f] * ((D_f[q,n] * q_scales[q]) * corpus_scales[n,f])  (+ sparse terms)
@@ -267,6 +263,10 @@ MFAR_API int mfar_score_topk_bm25_e4m3(const void* corpus, const float* corpus_s
                                        float* out_scores, int64_t* out_ids, void* workspace, size_t workspace_bytes,
                                        int impl, void* stream);
 
+/* Merge L sorted-or-unsorted key lists per query into the global top-k.  Used for (a) the
+ * per-CTA partial lists inside mfar_score_topk and (b) the per-shard lists after the NCCL
+ * all-gather (replaces the {rank}.qres file merge of mfar/modeling/contrastive.py:616-631).
+ * keys: uint64 [L, Q, k_in]; key 0 = empty slot. */
 MFAR_API int mfar_topk_merge(const uint64_t* keys, int L, int Q, int k_in, int k, uint64_t* out_keys,
                     float* out_scores, int64_t* out_ids, void* stream);
 

@@ -207,13 +207,15 @@ size_t mfar_score_topk_workspace_bytes(int Q, int k, int64_t n_docs, int n_spars
   return total;
 }
 
-// precomputed per-field sparse scores: dense [Q,Fs,ld] or COO (query row, global doc row, value) grouped by field
+// The n_sparse fields' scores: dense [Q,Fs,ld] rows, COO (query row, global doc row, value) grouped by field, or BM25
+// postings + query tokens.  `status`: the layout's own argument checks, which run before every other check of a call.
+enum SparseKind { kSparseNone, kSparseRows, kSparseCoo, kSparseBm25 };
 struct SparseInput {
-  int kind = 0;                       // 0 none, 1 dense, 2 COO, 3 BM25 postings + query tokens
+  int status = MFAR_OK; SparseKind kind = kSparseNone; int n_sparse = 0;
   const void* dense = nullptr; int dense_dtype = MFAR_F16; int64_t dense_ld = 0;
   const int32_t* coo_keys = nullptr; const void* coo_vals = nullptr; int coo_dtype = MFAR_F16;
   const int64_t* field_offsets_host = nullptr;
-  Bm25Fields bm25{}; const int32_t* entries = nullptr; int64_t n_entries = 0;   // kind 3
+  Bm25Fields bm25{}; const int32_t* entries = nullptr; int64_t n_entries = 0;
 };
 
 static size_t bm25_plan_bytes(int64_t n_entries) {
@@ -235,39 +237,84 @@ static int fill_bm25_fields(const void* const* indptr_host, const void* const* i
   return MFAR_OK;
 }
 
-// Dense operands of a scoring call: the corpus and the queries, bf16, or E4M3 with their row scales.
-struct DenseInput {
-  const void* corpus; const float* corpus_scales; const void* q_vecs; const float* q_scales; int dtype;
-};
+static SparseInput rows_input(const void* rows, int n_sparse, int dtype, int64_t ld) {
+  SparseInput sp;
+  sp.n_sparse = n_sparse;
+  if (n_sparse > 0) { sp.kind = kSparseRows; sp.dense = rows; sp.dense_dtype = dtype; sp.dense_ld = ld; }
+  return sp;
+}
 
-static int score_topk_core(const DenseInput& dn, int64_t n_docs, int corpus_fields, int field_begin, int n_dense,
-                           int dim, int Q, const float* w, const SparseInput& sp, int n_sparse,
-                           int64_t doc_id_base, int k, uint64_t* out_keys, float* out_scores, int64_t* out_ids,
-                           void* workspace, size_t workspace_bytes, int impl, void* stream) {
-  const void* corpus = dn.corpus;
-  const void* q_vecs = dn.q_vecs;
+static SparseInput coo_input(const int32_t* coo_keys, const void* coo_vals, int coo_dtype,
+                             const int64_t* field_offsets_host, int n_sparse) {
+  SparseInput sp;
+  sp.kind = kSparseCoo; sp.n_sparse = n_sparse; sp.field_offsets_host = field_offsets_host;
+  sp.coo_keys = coo_keys; sp.coo_vals = coo_vals; sp.coo_dtype = coo_dtype;
+  if (n_sparse <= 0 || !field_offsets_host) sp.status = MFAR_ERR_ARG;
+  else if (field_offsets_host[n_sparse] > 0 && (!coo_keys || !coo_vals)) sp.status = MFAR_ERR_ARG;
+  return sp;
+}
+
+static SparseInput bm25_input(const void* const* indptr_host, const void* const* indices_host,
+                              const void* const* data_host, const int32_t* vocab_host, int n_sparse,
+                              const int32_t* entries, int64_t n_entries) {
+  SparseInput sp;
+  sp.kind = kSparseBm25; sp.n_sparse = n_sparse; sp.entries = entries; sp.n_entries = n_entries;
+  sp.status = fill_bm25_fields(indptr_host, indices_host, data_host, vocab_host, n_sparse, &sp.bm25);
+  return sp;
+}
+
+// score_topk_core's dense operands, in the ScoreArgs fields the kernels read: bf16, or E4M3 with the row scales.
+static ScoreArgs dense_operands(int dtype, const void* corpus, const float* corpus_scales, const void* q_vecs,
+                                const float* q_scales) {
+  ScoreArgs a{};
+  a.corpus_dtype = dtype; a.corpus = corpus; a.corpus_scales = corpus_scales; a.q_vecs = q_vecs; a.q_scales = q_scales;
+  return a;
+}
+
+// Moves every per-doc pointer and count of `a` past its first `tiles` tiles (the pass behind a seeding prefix).  A new
+// per-doc field of ScoreArgs must be moved here too, or that pass scores the prefix twice and reads past the shard.
+static void skip_tiles(ScoreArgs& a, int tiles) {
+  const int64_t docs = int64_t(tiles) * kTileDocs;
+  const size_t rows = size_t(tiles) * a.corpus_fields * kTileDocs;
+  a.corpus = static_cast<const char*>(a.corpus) + rows * a.dim * (a.corpus_dtype == MFAR_E4M3 ? 1 : 2);
+  if (a.corpus_scales) a.corpus_scales += rows;
+  a.n_tiles -= tiles;
+  a.n_docs -= docs;
+  a.doc_id_base += docs;
+  if (a.base) a.base += docs;
+  if (a.sparse) {
+    a.sparse = static_cast<const char*>(a.sparse) + size_t(docs) * (a.sparse_dtype == MFAR_F16 ? 2 : 4);
+    a.sparse_cols = (a.sparse_cols ? a.sparse_cols : a.sparse_ld) - docs;
+  }
+}
+
+static int score_topk_core(ScoreArgs a, int64_t n_docs, int corpus_fields, int field_begin, int n_dense, int dim,
+                           int Q, const float* w, const SparseInput& sp, int64_t doc_id_base, int k, uint64_t* out_keys,
+                           float* out_scores, int64_t* out_ids, void* workspace, size_t workspace_bytes, int impl,
+                           void* stream) {
+  if (sp.status) return sp.status;
+  const int n_sparse = sp.n_sparse;
   t_last_launches = 0;
   if (n_docs <= 0 || Q <= 0 || !w || !workspace || (!out_scores && !out_ids && !out_keys)) return MFAR_ERR_ARG;
   if (n_dense < 0 || n_sparse < 0 || n_dense + n_sparse <= 0 || n_dense + n_sparse > MFAR_MAX_FIELDS)
     return MFAR_ERR_SHAPE;
-  if (n_dense > 0 && (!corpus || !q_vecs || dim <= 0 || field_begin < 0 || field_begin + n_dense > corpus_fields))
+  if (n_dense > 0 && (!a.corpus || !a.q_vecs || dim <= 0 || field_begin < 0 || field_begin + n_dense > corpus_fields))
     return MFAR_ERR_ARG;
-  if (n_dense > 0 && dn.dtype == MFAR_E4M3 && (!dn.corpus_scales || !dn.q_scales)) return MFAR_ERR_ARG;
-  if (n_sparse > 0 && sp.kind == 1 && (!sp.dense || sp.dense_ld < n_docs)) return MFAR_ERR_ARG;
-  if (n_sparse > 0 && sp.kind == 2 && (!sp.field_offsets_host || sp.field_offsets_host[0] != 0)) return MFAR_ERR_ARG;
-  if (n_sparse > 0 && sp.kind == 0) return MFAR_ERR_ARG;
-  if (n_sparse > 0 && sp.kind == 3 && (sp.n_entries < 0 || (sp.n_entries > 0 && !sp.entries))) return MFAR_ERR_ARG;
+  if (n_dense > 0 && a.corpus_dtype == MFAR_E4M3 && (!a.corpus_scales || !a.q_scales)) return MFAR_ERR_ARG;
+  if (n_sparse > 0 && sp.kind == kSparseRows && (!sp.dense || sp.dense_ld < n_docs)) return MFAR_ERR_ARG;
+  if (n_sparse > 0 && sp.kind == kSparseCoo && (!sp.field_offsets_host || sp.field_offsets_host[0] != 0))
+    return MFAR_ERR_ARG;
+  if (n_sparse > 0 && sp.kind == kSparseBm25 && (sp.n_entries < 0 || (sp.n_entries > 0 && !sp.entries)))
+    return MFAR_ERR_ARG;
   if (k <= 0 || k > MFAR_MAX_K) return MFAR_ERR_SHAPE;
   if (doc_id_base < 0 || doc_id_base + n_docs > (int64_t(1) << 32)) return MFAR_ERR_SHAPE;
   if (impl < MFAR_IMPL_AUTO || impl > MFAR_IMPL_TCGEN05_QS) return MFAR_ERR_ARG;
   if (int rc = check_arch()) return rc;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
 
-  ScoreArgs a{};
-  a.corpus = corpus; a.corpus_dtype = dn.dtype; a.corpus_scales = dn.corpus_scales; a.q_scales = dn.q_scales;
   a.n_docs = n_docs; a.n_tiles = int((n_docs + kTileDocs - 1) / kTileDocs);
   a.corpus_fields = corpus_fields; a.field_begin = field_begin; a.n_dense = n_dense; a.dim = dim;
-  a.q_vecs = q_vecs; a.Q = Q; a.w = w; a.w_ld = n_dense + n_sparse; a.doc_id_base = doc_id_base; a.k = k;
+  a.Q = Q; a.w = w; a.w_ld = n_dense + n_sparse; a.doc_id_base = doc_id_base; a.k = k;
   if (n_dense > 0 && impl == MFAR_IMPL_TCGEN05 && !score_tc_supported(a)) return MFAR_ERR_SHAPE;
   if (n_dense > 0 && impl == MFAR_IMPL_TCGEN05_QS && !score_qs_supported(a)) return MFAR_ERR_SHAPE;
   const Geometry g = resolve_geometry(a, impl);
@@ -277,11 +324,11 @@ static int score_topk_core(const DenseInput& dn, int64_t n_docs, int corpus_fiel
   // Dense [Q,Fs,ld] score rows are gathered and mixed INSIDE the tensor-core scoring epilogues (no [Q,N] intermediate
   // in HBM) when their rows are 32-byte aligned; COO pairs / BM25 postings scatter into the fp32 base block, and the
   // SIMT cross-check kernel and the sparse-only row scan read that block too.
-  const bool fuse_sparse = n_sparse > 0 && sp.kind == 1 && n_dense > 0 &&
+  const bool fuse_sparse = n_sparse > 0 && sp.kind == kSparseRows && n_dense > 0 &&
                            (g.impl == MFAR_IMPL_TCGEN05 || g.impl == MFAR_IMPL_TCGEN05_QS) &&
                            sparse_rows_fusable(sp.dense, sp.dense_dtype, sp.dense_ld);
   const size_t ws_base = (n_sparse > 0 && !fuse_sparse) ? align_up(size_t(Q) * base_ld * 4, 256) : 0;
-  const size_t ws_plan = (n_sparse > 0 && sp.kind == 3) ? bm25_plan_bytes(sp.n_entries) : 0;
+  const size_t ws_plan = (n_sparse > 0 && sp.kind == kSparseBm25) ? bm25_plan_bytes(sp.n_entries) : 0;
   // prefix keys 2 x [Q,k] + seed thresholds [Q] of the threshold-seeding passes (used when the caller's workspace has room)
   size_t ws_seed = seed_scratch_bytes(Q, k);
   if (workspace_bytes < ws_topk + ws_base + ws_plan) return MFAR_ERR_WORKSPACE;
@@ -292,12 +339,12 @@ static int score_topk_core(const DenseInput& dn, int64_t n_docs, int corpus_fiel
     a.sparse = sp.dense; a.sparse_dtype = sp.dense_dtype; a.sparse_ld = sp.dense_ld; a.n_sparse = n_sparse;
   } else if (n_sparse > 0) {
     float* base = reinterpret_cast<float*>(static_cast<char*>(workspace) + ws_topk);
-    if (sp.kind == 1) {
+    if (sp.kind == kSparseRows) {
       if (int rc = launch_sparse_premix(sp.dense, sp.dense_dtype, sp.dense_ld, n_sparse, w, a.w_ld, n_dense, Q, n_docs,
                                         base, base_ld, st))
         return rc;
       ++t_last_launches;
-    } else if (sp.kind == 3) {
+    } else if (sp.kind == kSparseBm25) {
       MFAR_CUDA_OK(cudaMemsetAsync(base, 0, size_t(Q) * base_ld * 4, st));
       ++t_last_launches;
       if (sp.n_entries > 0) {
@@ -372,20 +419,9 @@ static int score_topk_core(const DenseInput& dn, int64_t n_docs, int corpus_fiel
       if (g_debug_seed) MFAR_CUDA_OK(cudaMemcpyAsync(seed_thr, g_debug_seed, size_t(Q) * 8, cudaMemcpyDeviceToDevice, st));
 #endif
       t_last_launches += 4;                             // prefix scoring + merge + seed, and the copy into the next pass
-      // A prefix is not scored twice: the next pass starts behind it (every per-doc pointer advanced by the prefix's
-      // whole tiles) and the next merge takes the prefix's ranked top k as one more list.
-      const int64_t skip = ap.n_docs;
-      const size_t skip_rows = size_t(ap.n_tiles) * a.corpus_fields * kTileDocs;
-      a.corpus = static_cast<const char*>(a.corpus) + skip_rows * a.dim * (a.corpus_dtype == MFAR_E4M3 ? 1 : 2);
-      if (a.corpus_scales) a.corpus_scales += skip_rows;
-      a.n_tiles -= ap.n_tiles;
-      a.n_docs -= skip;
-      a.doc_id_base += skip;
-      if (a.base) a.base += skip;
-      if (a.sparse) {
-        a.sparse = static_cast<const char*>(a.sparse) + size_t(skip) * (a.sparse_dtype == MFAR_F16 ? 2 : 4);
-        a.sparse_cols = (a.sparse_cols ? a.sparse_cols : a.sparse_ld) - skip;
-      }
+      // A prefix is not scored twice: the next pass starts behind it and the next merge takes the prefix's ranked top
+      // k as one more list.
+      skip_tiles(a, ap.n_tiles);
       a.gthr_seed = seed_thr;
       prefix_keys = pref_keys;
     }
@@ -415,11 +451,9 @@ int mfar_score_topk(const void* corpus, int64_t n_docs, int corpus_fields, int f
                     const void* q_vecs, int Q, const float* w, const void* sparse, int n_sparse, int sparse_dtype,
                     int64_t sparse_ld, int64_t doc_id_base, int k, uint64_t* out_keys, float* out_scores,
                     int64_t* out_ids, void* workspace, size_t workspace_bytes, int impl, void* stream) {
-  SparseInput sp;
-  if (n_sparse > 0) { sp.kind = 1; sp.dense = sparse; sp.dense_dtype = sparse_dtype; sp.dense_ld = sparse_ld; }
-  return score_topk_core({corpus, nullptr, q_vecs, nullptr, MFAR_BF16}, n_docs, corpus_fields, field_begin, n_dense,
-                         dim, Q, w, sp, n_sparse, doc_id_base, k, out_keys, out_scores, out_ids, workspace,
-                         workspace_bytes, impl, stream);
+  return score_topk_core(dense_operands(MFAR_BF16, corpus, nullptr, q_vecs, nullptr), n_docs, corpus_fields,
+                         field_begin, n_dense, dim, Q, w, rows_input(sparse, n_sparse, sparse_dtype, sparse_ld),
+                         doc_id_base, k, out_keys, out_scores, out_ids, workspace, workspace_bytes, impl, stream);
 }
 
 // mfar_score_topk on an E4M3 corpus: the same reference lines (index.py:181-232, 111-118; contrastive.py:686,694,696)
@@ -428,11 +462,9 @@ int mfar_score_topk_e4m3(const void* corpus, const float* corpus_scales, int64_t
                          const float* w, const void* sparse, int n_sparse, int sparse_dtype, int64_t sparse_ld,
                          int64_t doc_id_base, int k, uint64_t* out_keys, float* out_scores, int64_t* out_ids,
                          void* workspace, size_t workspace_bytes, int impl, void* stream) {
-  SparseInput sp;
-  if (n_sparse > 0) { sp.kind = 1; sp.dense = sparse; sp.dense_dtype = sparse_dtype; sp.dense_ld = sparse_ld; }
-  return score_topk_core({corpus, corpus_scales, q_vecs, q_scales, MFAR_E4M3}, n_docs, corpus_fields, field_begin,
-                         n_dense, dim, Q, w, sp, n_sparse, doc_id_base, k, out_keys, out_scores, out_ids, workspace,
-                         workspace_bytes, impl, stream);
+  return score_topk_core(dense_operands(MFAR_E4M3, corpus, corpus_scales, q_vecs, q_scales), n_docs, corpus_fields,
+                         field_begin, n_dense, dim, Q, w, rows_input(sparse, n_sparse, sparse_dtype, sparse_ld),
+                         doc_id_base, k, out_keys, out_scores, out_ids, workspace, workspace_bytes, impl, stream);
 }
 
 int mfar_score_topk_coo(const void* corpus, int64_t n_docs, int corpus_fields, int field_begin, int n_dense, int dim,
@@ -440,14 +472,10 @@ int mfar_score_topk_coo(const void* corpus, int64_t n_docs, int corpus_fields, i
                         int coo_dtype, const int64_t* field_offsets_host, int n_sparse, int64_t doc_id_base, int k,
                         uint64_t* out_keys, float* out_scores, int64_t* out_ids, void* workspace,
                         size_t workspace_bytes, int impl, void* stream) {
-  if (n_sparse <= 0 || !field_offsets_host) return MFAR_ERR_ARG;
-  if (field_offsets_host[n_sparse] > 0 && (!coo_keys || !coo_vals)) return MFAR_ERR_ARG;
-  SparseInput sp;
-  sp.kind = 2; sp.coo_keys = coo_keys; sp.coo_vals = coo_vals; sp.coo_dtype = coo_dtype;
-  sp.field_offsets_host = field_offsets_host;
-  return score_topk_core({corpus, nullptr, q_vecs, nullptr, MFAR_BF16}, n_docs, corpus_fields, field_begin, n_dense,
-                         dim, Q, w, sp, n_sparse, doc_id_base, k, out_keys, out_scores, out_ids, workspace,
-                         workspace_bytes, impl, stream);
+  return score_topk_core(dense_operands(MFAR_BF16, corpus, nullptr, q_vecs, nullptr), n_docs, corpus_fields,
+                         field_begin, n_dense, dim, Q, w,
+                         coo_input(coo_keys, coo_vals, coo_dtype, field_offsets_host, n_sparse), doc_id_base, k,
+                         out_keys, out_scores, out_ids, workspace, workspace_bytes, impl, stream);
 }
 
 // mfar_score_topk_coo on an E4M3 corpus (precompute_bm25s_scores.py:21-30, util.py:151-173, index.py:120-125)
@@ -457,14 +485,10 @@ int mfar_score_topk_coo_e4m3(const void* corpus, const float* corpus_scales, int
                              const int64_t* field_offsets_host, int n_sparse, int64_t doc_id_base, int k,
                              uint64_t* out_keys, float* out_scores, int64_t* out_ids, void* workspace,
                              size_t workspace_bytes, int impl, void* stream) {
-  if (n_sparse <= 0 || !field_offsets_host) return MFAR_ERR_ARG;
-  if (field_offsets_host[n_sparse] > 0 && (!coo_keys || !coo_vals)) return MFAR_ERR_ARG;
-  SparseInput sp;
-  sp.kind = 2; sp.coo_keys = coo_keys; sp.coo_vals = coo_vals; sp.coo_dtype = coo_dtype;
-  sp.field_offsets_host = field_offsets_host;
-  return score_topk_core({corpus, corpus_scales, q_vecs, q_scales, MFAR_E4M3}, n_docs, corpus_fields, field_begin,
-                         n_dense, dim, Q, w, sp, n_sparse, doc_id_base, k, out_keys, out_scores, out_ids, workspace,
-                         workspace_bytes, impl, stream);
+  return score_topk_core(dense_operands(MFAR_E4M3, corpus, corpus_scales, q_vecs, q_scales), n_docs, corpus_fields,
+                         field_begin, n_dense, dim, Q, w,
+                         coo_input(coo_keys, coo_vals, coo_dtype, field_offsets_host, n_sparse), doc_id_base, k,
+                         out_keys, out_scores, out_ids, workspace, workspace_bytes, impl, stream);
 }
 
 int mfar_bm25_build_scores(const int32_t* post_token, const int32_t* post_doc, const int32_t* post_tf, int64_t nnz,
@@ -554,12 +578,10 @@ int mfar_score_topk_bm25(const void* corpus, int64_t n_docs, int corpus_fields, 
                          int n_sparse, const int32_t* entries, int64_t n_entries, int64_t doc_id_base, int k,
                          uint64_t* out_keys, float* out_scores, int64_t* out_ids, void* workspace,
                          size_t workspace_bytes, int impl, void* stream) {
-  SparseInput sp;
-  sp.kind = 3; sp.entries = entries; sp.n_entries = n_entries;
-  if (int rc = fill_bm25_fields(indptr_host, indices_host, data_host, vocab_host, n_sparse, &sp.bm25)) return rc;
-  return score_topk_core({corpus, nullptr, q_vecs, nullptr, MFAR_BF16}, n_docs, corpus_fields, field_begin, n_dense,
-                         dim, Q, w, sp, n_sparse, doc_id_base, k, out_keys, out_scores, out_ids, workspace,
-                         workspace_bytes, impl, stream);
+  return score_topk_core(dense_operands(MFAR_BF16, corpus, nullptr, q_vecs, nullptr), n_docs, corpus_fields,
+                         field_begin, n_dense, dim, Q, w,
+                         bm25_input(indptr_host, indices_host, data_host, vocab_host, n_sparse, entries, n_entries),
+                         doc_id_base, k, out_keys, out_scores, out_ids, workspace, workspace_bytes, impl, stream);
 }
 
 // mfar_score_topk_bm25 on an E4M3 corpus (index.py:72-76, 95-118 for the sparse fields)
@@ -570,12 +592,10 @@ int mfar_score_topk_bm25_e4m3(const void* corpus, const float* corpus_scales, in
                               const int32_t* entries, int64_t n_entries, int64_t doc_id_base, int k,
                               uint64_t* out_keys, float* out_scores, int64_t* out_ids, void* workspace,
                               size_t workspace_bytes, int impl, void* stream) {
-  SparseInput sp;
-  sp.kind = 3; sp.entries = entries; sp.n_entries = n_entries;
-  if (int rc = fill_bm25_fields(indptr_host, indices_host, data_host, vocab_host, n_sparse, &sp.bm25)) return rc;
-  return score_topk_core({corpus, corpus_scales, q_vecs, q_scales, MFAR_E4M3}, n_docs, corpus_fields, field_begin,
-                         n_dense, dim, Q, w, sp, n_sparse, doc_id_base, k, out_keys, out_scores, out_ids, workspace,
-                         workspace_bytes, impl, stream);
+  return score_topk_core(dense_operands(MFAR_E4M3, corpus, corpus_scales, q_vecs, q_scales), n_docs, corpus_fields,
+                         field_begin, n_dense, dim, Q, w,
+                         bm25_input(indptr_host, indices_host, data_host, vocab_host, n_sparse, entries, n_entries),
+                         doc_id_base, k, out_keys, out_scores, out_ids, workspace, workspace_bytes, impl, stream);
 }
 
 int mfar_topk_merge(const uint64_t* keys, int L, int Q, int k_in, int k, uint64_t* out_keys, float* out_scores,
@@ -690,24 +710,29 @@ int mfar_union_rescore(const void* corpus, int64_t n_docs, int corpus_fields, in
   return MFAR_OK;
 }
 
-// scratch layout for the host-buffer call
+// Scratch layout of the host-buffer calls: queries, query embedding, mixture weights, the sparse input (score rows
+// re-pitched to sparse_ld, or BM25 token entries), result, workspace.  The BM25 layout keeps a query block without a
+// dense field (its sizes are ABI).
 struct HostScratch {
   size_t off_q, off_qe, off_w, off_sparse, off_scores, off_ids, off_ws, total, ws_bytes;
   int64_t sparse_ld;
 };
-static HostScratch host_scratch_layout(int Q, int dim, int E, int n_dense, int n_sparse, int64_t n_docs,
-                                       int sparse_dtype, int k) {
+static HostScratch host_scratch_layout(int Q, int dim, int E, int n_dense, int n_sparse, int64_t n_docs, int k,
+                                       bool bm25, int sparse_dtype, int64_t n_entries) {
   HostScratch h{};
   size_t o = 0;
-  h.off_q = o;      o += align_up(size_t(Q) * dim * 2, 256);
+  h.off_q = o;      o += align_up(size_t(Q) * (bm25 ? std::max(dim, 1) : dim) * 2, 256);
   h.off_qe = o;     o += align_up(size_t(Q) * std::max(E, 1) * 4, 256);
   h.off_w = o;      o += align_up(size_t(Q) * (n_dense + n_sparse) * 4, 256);
   h.sparse_ld = int64_t(align_up(size_t(n_docs), 64));   // 128-/256-byte row pitch: the epilogue gather's vector loads
-  h.off_sparse = o; o += align_up(size_t(Q) * n_sparse * size_t(h.sparse_ld) * (sparse_dtype == MFAR_F32 ? 4 : 2), 256);
+  h.off_sparse = o;
+  if (bm25) o += align_up(size_t(std::max<int64_t>(n_entries, 1)) * 12, 256);
+  else      o += align_up(size_t(Q) * n_sparse * size_t(h.sparse_ld) * (sparse_dtype == MFAR_F32 ? 4 : 2), 256);
   h.off_scores = o; o += align_up(size_t(Q) * k * 4, 256);
   h.off_ids = o;    o += align_up(size_t(Q) * k * 8, 256);
   h.off_ws = o;
-  h.ws_bytes = mfar_score_topk_workspace_bytes(Q, k, n_docs, n_sparse);
+  h.ws_bytes = bm25 ? mfar_score_topk_bm25_workspace_bytes(Q, k, n_docs, n_sparse, n_entries)
+                    : mfar_score_topk_workspace_bytes(Q, k, n_docs, n_sparse);
   h.total = o + h.ws_bytes;
   return h;
 }
@@ -715,47 +740,62 @@ static HostScratch host_scratch_layout(int Q, int dim, int E, int n_dense, int n
 size_t mfar_search_host_scratch_bytes(int Q, int dim, int E, int n_dense, int n_sparse, int64_t n_docs,
                                       int sparse_dtype, int k) {
   if (Q <= 0 || n_docs <= 0) return 0;
-  return host_scratch_layout(Q, dim, E, n_dense, n_sparse, n_docs, sparse_dtype, k).total;
+  return host_scratch_layout(Q, dim, E, n_dense, n_sparse, n_docs, k, false, sparse_dtype, 0).total;
 }
 
-int mfar_search_host(const void* corpus, int64_t n_docs, int corpus_fields, int field_begin, int n_dense, int dim,
-                     const void* q_vecs_host, const float* q_emb_host, int Q, int E, const float* W, const float* mask,
-                     int query_cond, const void* sparse_host, int n_sparse, int sparse_dtype, int64_t doc_id_base,
-                     int k, float* out_scores_host, int64_t* out_ids_host, void* scratch, size_t scratch_bytes,
-                     int impl, void* stream) {
+size_t mfar_search_host_bm25_scratch_bytes(int Q, int dim, int E, int n_dense, int n_sparse, int64_t n_docs,
+                                           int64_t n_entries, int k) {
+  if (Q <= 0 || n_docs <= 0 || n_entries < 0) return 0;
+  return host_scratch_layout(Q, dim, E, n_dense, n_sparse, n_docs, k, true, MFAR_F16, n_entries).total;
+}
+
+// The host-buffer calls: `sp` (HOST score rows of pitch n_docs, or token entries) is copied into the scratch buffer.
+static int search_host_core(const void* corpus, int64_t n_docs, int corpus_fields, int field_begin, int n_dense,
+                            int dim, const void* q_vecs_host, const float* q_emb_host, int Q, int E, const float* W,
+                            const float* mask, int query_cond, SparseInput sp, int64_t doc_id_base, int k,
+                            float* out_scores_host, int64_t* out_ids_host, void* scratch, size_t scratch_bytes,
+                            int impl, void* stream) {
+  const int n_sparse = sp.n_sparse;
+  const bool bm25 = sp.kind == kSparseBm25;
   if (!scratch || !W || !out_scores_host || !out_ids_host || Q <= 0 || n_docs <= 0) return MFAR_ERR_ARG;
   if (n_dense > 0 && !q_vecs_host) return MFAR_ERR_ARG;
   if (query_cond && !q_emb_host) return MFAR_ERR_ARG;
-  if (n_sparse > 0 && !sparse_host) return MFAR_ERR_ARG;
+  if (sp.kind == kSparseRows && !sp.dense) return MFAR_ERR_ARG;
+  if (bm25 && (sp.n_entries < 0 || (sp.n_entries > 0 && !sp.entries))) return MFAR_ERR_ARG;
   if (reinterpret_cast<uintptr_t>(scratch) % 256 != 0) return MFAR_ERR_ARG;
   if (int rc = check_arch()) return rc;
-  const HostScratch h = host_scratch_layout(Q, dim, E, n_dense, n_sparse, n_docs, sparse_dtype, k);
+  const auto h = host_scratch_layout(Q, dim, E, n_dense, n_sparse, n_docs, k, bm25, sp.dense_dtype, sp.n_entries);
   if (scratch_bytes < h.total) return MFAR_ERR_WORKSPACE;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   char* s = static_cast<char*>(scratch);
-  const int F = n_dense + n_sparse;
   if (n_dense > 0)
     MFAR_CUDA_OK(cudaMemcpyAsync(s + h.off_q, q_vecs_host, size_t(Q) * dim * 2, cudaMemcpyHostToDevice, st));
   if (query_cond)
     MFAR_CUDA_OK(cudaMemcpyAsync(s + h.off_qe, q_emb_host, size_t(Q) * E * 4, cudaMemcpyHostToDevice, st));
-  if (n_sparse > 0) {                                  // [Q,Fs,N] host rows -> [Q,Fs,sparse_ld] device rows (aligned pitch)
-    const size_t es = sparse_dtype == MFAR_F32 ? 4 : 2;
+  if (sp.kind == kSparseRows) {   // [Q,Fs,N] host rows -> [Q,Fs,sparse_ld] device rows (aligned pitch)
+    const size_t es = sp.dense_dtype == MFAR_F32 ? 4 : 2;
     const size_t width = size_t(n_docs) * es, dpitch = size_t(h.sparse_ld) * es;
-    MFAR_CUDA_OK(cudaMemcpy2DAsync(s + h.off_sparse, dpitch, sparse_host, width, width, size_t(Q) * n_sparse,
+    MFAR_CUDA_OK(cudaMemcpy2DAsync(s + h.off_sparse, dpitch, sp.dense, width, width, size_t(Q) * n_sparse,
                                    cudaMemcpyHostToDevice, st));
     if (dpitch > width)
       MFAR_CUDA_OK(cudaMemset2DAsync(s + h.off_sparse + width, dpitch, 0, dpitch - width, size_t(Q) * n_sparse, st));
+    sp.dense = s + h.off_sparse;
+    sp.dense_ld = h.sparse_ld;
+  } else if (bm25) {
+    if (sp.n_entries > 0)
+      MFAR_CUDA_OK(cudaMemcpyAsync(s + h.off_sparse, sp.entries, sp.n_entries * 12, cudaMemcpyHostToDevice, st));
+    sp.entries = reinterpret_cast<const int32_t*>(s + h.off_sparse);
   }
   float* w_dev = reinterpret_cast<float*>(s + h.off_w);
   // query_cond == 0: the shared weight row is replicated per query so the scoring kernels index w[q, f] uniformly
   if (int rc = launch_mixture_weights(query_cond ? reinterpret_cast<const float*>(s + h.off_qe) : nullptr, W, mask, Q,
-                                      E, F, query_cond, w_dev, st))
+                                      E, n_dense + n_sparse, query_cond, w_dev, st))
     return rc;
   float* sc = reinterpret_cast<float*>(s + h.off_scores);
   int64_t* ids = reinterpret_cast<int64_t*>(s + h.off_ids);
-  int rc = mfar_score_topk(corpus, n_docs, corpus_fields, field_begin, n_dense, dim, s + h.off_q, Q, w_dev,
-                           n_sparse ? s + h.off_sparse : nullptr, n_sparse, sparse_dtype, h.sparse_ld, doc_id_base, k,
-                           nullptr, sc, ids, s + h.off_ws, h.ws_bytes, impl, st);
+  int rc = score_topk_core(dense_operands(MFAR_BF16, corpus, nullptr, s + h.off_q, nullptr), n_docs, corpus_fields,
+                           field_begin, n_dense, dim, Q, w_dev, sp, doc_id_base, k, nullptr, sc, ids,
+                           s + h.off_ws, h.ws_bytes, impl, st);
   if (rc) return rc;
   t_last_launches += 1;
   MFAR_CUDA_OK(cudaMemcpyAsync(out_scores_host, sc, size_t(Q) * k * 4, cudaMemcpyDeviceToHost, st));
@@ -764,27 +804,14 @@ int mfar_search_host(const void* corpus, int64_t n_docs, int corpus_fields, int 
   return MFAR_OK;
 }
 
-struct HostScratchBm25 { size_t off_q, off_qe, off_w, off_ent, off_scores, off_ids, off_ws, total, ws_bytes; };
-static HostScratchBm25 host_scratch_bm25_layout(int Q, int dim, int E, int n_dense, int n_sparse, int64_t n_docs,
-                                                int64_t n_entries, int k) {
-  HostScratchBm25 h{};
-  size_t o = 0;
-  h.off_q = o;      o += align_up(size_t(Q) * std::max(dim, 1) * 2, 256);
-  h.off_qe = o;     o += align_up(size_t(Q) * std::max(E, 1) * 4, 256);
-  h.off_w = o;      o += align_up(size_t(Q) * (n_dense + n_sparse) * 4, 256);
-  h.off_ent = o;    o += align_up(size_t(std::max<int64_t>(n_entries, 1)) * 12, 256);
-  h.off_scores = o; o += align_up(size_t(Q) * k * 4, 256);
-  h.off_ids = o;    o += align_up(size_t(Q) * k * 8, 256);
-  h.off_ws = o;
-  h.ws_bytes = mfar_score_topk_bm25_workspace_bytes(Q, k, n_docs, n_sparse, n_entries);
-  h.total = o + h.ws_bytes;
-  return h;
-}
-
-size_t mfar_search_host_bm25_scratch_bytes(int Q, int dim, int E, int n_dense, int n_sparse, int64_t n_docs,
-                                           int64_t n_entries, int k) {
-  if (Q <= 0 || n_docs <= 0 || n_entries < 0) return 0;
-  return host_scratch_bm25_layout(Q, dim, E, n_dense, n_sparse, n_docs, n_entries, k).total;
+int mfar_search_host(const void* corpus, int64_t n_docs, int corpus_fields, int field_begin, int n_dense, int dim,
+                     const void* q_vecs_host, const float* q_emb_host, int Q, int E, const float* W, const float* mask,
+                     int query_cond, const void* sparse_host, int n_sparse, int sparse_dtype, int64_t doc_id_base,
+                     int k, float* out_scores_host, int64_t* out_ids_host, void* scratch, size_t scratch_bytes,
+                     int impl, void* stream) {
+  return search_host_core(corpus, n_docs, corpus_fields, field_begin, n_dense, dim, q_vecs_host, q_emb_host, Q, E, W,
+                          mask, query_cond, rows_input(sparse_host, n_sparse, sparse_dtype, n_docs), doc_id_base, k,
+                          out_scores_host, out_ids_host, scratch, scratch_bytes, impl, stream);
 }
 
 int mfar_search_host_bm25(const void* corpus, int64_t n_docs, int corpus_fields, int field_begin, int n_dense, int dim,
@@ -794,40 +821,10 @@ int mfar_search_host_bm25(const void* corpus, int64_t n_docs, int corpus_fields,
                           int n_sparse, const int32_t* entries_host, int64_t n_entries, int64_t doc_id_base, int k,
                           float* out_scores_host, int64_t* out_ids_host, void* scratch, size_t scratch_bytes, int impl,
                           void* stream) {
-  if (!scratch || !W || !out_scores_host || !out_ids_host || Q <= 0 || n_docs <= 0 || n_entries < 0)
-    return MFAR_ERR_ARG;
-  if (n_dense > 0 && !q_vecs_host) return MFAR_ERR_ARG;
-  if (query_cond && !q_emb_host) return MFAR_ERR_ARG;
-  if (n_entries > 0 && !entries_host) return MFAR_ERR_ARG;
-  if (reinterpret_cast<uintptr_t>(scratch) % 256 != 0) return MFAR_ERR_ARG;
-  if (int rc = check_arch()) return rc;
-  const HostScratchBm25 h = host_scratch_bm25_layout(Q, dim, E, n_dense, n_sparse, n_docs, n_entries, k);
-  if (scratch_bytes < h.total) return MFAR_ERR_WORKSPACE;
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  char* s = static_cast<char*>(scratch);
-  const int F = n_dense + n_sparse;
-  if (n_dense > 0)
-    MFAR_CUDA_OK(cudaMemcpyAsync(s + h.off_q, q_vecs_host, size_t(Q) * dim * 2, cudaMemcpyHostToDevice, st));
-  if (query_cond)
-    MFAR_CUDA_OK(cudaMemcpyAsync(s + h.off_qe, q_emb_host, size_t(Q) * E * 4, cudaMemcpyHostToDevice, st));
-  if (n_entries > 0)
-    MFAR_CUDA_OK(cudaMemcpyAsync(s + h.off_ent, entries_host, size_t(n_entries) * 12, cudaMemcpyHostToDevice, st));
-  float* w_dev = reinterpret_cast<float*>(s + h.off_w);
-  if (int rc = launch_mixture_weights(query_cond ? reinterpret_cast<const float*>(s + h.off_qe) : nullptr, W, mask, Q,
-                                      E, F, query_cond, w_dev, st))
-    return rc;
-  float* sc = reinterpret_cast<float*>(s + h.off_scores);
-  int64_t* ids = reinterpret_cast<int64_t*>(s + h.off_ids);
-  int rc = mfar_score_topk_bm25(corpus, n_docs, corpus_fields, field_begin, n_dense, dim, s + h.off_q, Q, w_dev,
-                                indptr_host, indices_host, data_host, vocab_host, n_sparse,
-                                reinterpret_cast<const int32_t*>(s + h.off_ent), n_entries, doc_id_base, k, nullptr, sc,
-                                ids, s + h.off_ws, h.ws_bytes, impl, st);
-  if (rc) return rc;
-  t_last_launches += 1;
-  MFAR_CUDA_OK(cudaMemcpyAsync(out_scores_host, sc, size_t(Q) * k * 4, cudaMemcpyDeviceToHost, st));
-  MFAR_CUDA_OK(cudaMemcpyAsync(out_ids_host, ids, size_t(Q) * k * 8, cudaMemcpyDeviceToHost, st));
-  MFAR_CUDA_OK(cudaStreamSynchronize(st));
-  return MFAR_OK;
+  return search_host_core(corpus, n_docs, corpus_fields, field_begin, n_dense, dim, q_vecs_host, q_emb_host, Q, E, W,
+                          mask, query_cond, bm25_input(indptr_host, indices_host, data_host, vocab_host, n_sparse,
+                                                       entries_host, n_entries),
+                          doc_id_base, k, out_scores_host, out_ids_host, scratch, scratch_bytes, impl, stream);
 }
 
 static int check_doc_layout(const float* q, int B, int E, const float* docs, int64_t N, int F, int64_t inner,

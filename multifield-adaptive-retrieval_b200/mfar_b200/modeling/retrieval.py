@@ -9,6 +9,7 @@
 """
 from __future__ import annotations
 
+import ctypes
 from typing import Dict, List, Optional, Sequence, TextIO, Tuple
 
 import numpy as np
@@ -26,6 +27,11 @@ DTYPES = ("bf16", "e4m3")
 
 def _round_up(x: int, m: int) -> int:
     return (x + m - 1) // m * m
+
+
+def _operand(t: Optional[torch.Tensor], scales: Optional[torch.Tensor], e4m3: bool) -> tuple:
+    """Pointer arguments of one operand of an entry point: the tensor, then its row scales on the *_e4m3 twin."""
+    return (nv.ptr(t), nv.ptr(scales)) if e4m3 else (nv.ptr(t),)
 
 
 class PackedCorpus:
@@ -67,22 +73,24 @@ class PackedCorpus:
         """rows: [n, dim] fp32/bf16 tensor (host or device) -> docs [row_begin, row_begin+n) of `field`."""
         if rows.dim() != 2 or rows.shape[1] != self.dim:
             raise ValueError(f"expected [n,{self.dim}] rows, got {tuple(rows.shape)}")
-        r = rows.to(self.device, non_blocking=True)
-        if r.dtype not in (torch.float32, torch.bfloat16):
-            r = r.float()
+        self._pack(rows.to(self.device, non_blocking=True), self.data, self.scales, row_begin, self.n_docs,
+                   self.n_fields, field)
+
+    def _pack(self, rows: torch.Tensor, out: torch.Tensor, scales: Optional[torch.Tensor], row_begin: int, n_docs: int,
+              n_fields: int, field: int, what: str = "") -> None:
+        """Device rows [n, dim] -> rows [row_begin, row_begin + n) of `field` of the packed layout of an n_docs x
+        n_fields corpus in `out` (with their `scales` on an E4M3 corpus), padded to dim_pad.  Inputs other than
+        fp32 / bf16 are taken to fp32 first."""
+        if rows.dtype not in (torch.float32, torch.bfloat16):
+            rows = rows.float()
         if self.dim_pad != self.dim:
-            r = torch.nn.functional.pad(r, (0, self.dim_pad - self.dim))
-        r = r.contiguous()
-        code = nv.F32 if r.dtype == torch.float32 else nv.BF16
-        if self.e4m3:
-            nv.check(nv.lib().mfar_corpus_pack_rows_e4m3(nv.ptr(r), code, r.shape[0], int(row_begin), nv.ptr(self.data),
-                                                         nv.ptr(self.scales), self.n_docs, self.n_fields, int(field),
-                                                         self.dim_pad, int(self.normalize), nv.stream()),
-                     "corpus_pack_rows_e4m3")
-            return
-        nv.check(nv.lib().mfar_corpus_pack_rows(nv.ptr(r), code, r.shape[0], int(row_begin), nv.ptr(self.data),
-                                                self.n_docs, self.n_fields, int(field), self.dim_pad,
-                                                int(self.normalize), nv.stream()), "corpus_pack_rows")
+            rows = torch.nn.functional.pad(rows, (0, self.dim_pad - self.dim))
+        rows = rows.contiguous()
+        name = "corpus_pack_rows_e4m3" if self.e4m3 else "corpus_pack_rows"
+        nv.check(getattr(nv.lib(), "mfar_" + name)(
+            nv.ptr(rows), nv.F32 if rows.dtype == torch.float32 else nv.BF16, rows.shape[0], int(row_begin),
+            *_operand(out, scales, self.e4m3), n_docs, n_fields, int(field), self.dim_pad, int(self.normalize),
+            nv.stream()), name + what)
 
     def load_field(self, field: int, vectors, chunk_rows: int = 131072) -> None:
         """vectors: np.memmap / ndarray / tensor [N, dim] (the reference's ``MemoryMapDict.file``)."""
@@ -134,15 +142,11 @@ class PackedCorpus:
     def unpack_field(self, field: int, row_begin: int = 0, n_rows: Optional[int] = None) -> torch.Tensor:
         n_rows = self.n_docs - row_begin if n_rows is None else n_rows
         out = torch.empty((n_rows, self.dim_pad), dtype=torch.float32, device=self.device)
-        if self.e4m3:                                 # exact: every dequantized value is a normal fp32 number
-            nv.check(nv.lib().mfar_corpus_unpack_rows_e4m3(nv.ptr(self.data), nv.ptr(self.scales), self.n_docs,
-                                                           self.n_fields, int(field), self.dim_pad, int(row_begin),
-                                                           int(n_rows), nv.ptr(out), nv.stream()),
-                     "corpus_unpack_rows_e4m3")
-            return out[:, : self.dim]
-        nv.check(nv.lib().mfar_corpus_unpack_rows(nv.ptr(self.data), self.n_docs, self.n_fields, int(field),
-                                                  self.dim_pad, int(row_begin), int(n_rows), nv.ptr(out), nv.stream()),
-                 "corpus_unpack_rows")
+        # exact on an E4M3 corpus too: every dequantized value is a normal fp32 number
+        name = "corpus_unpack_rows_e4m3" if self.e4m3 else "corpus_unpack_rows"
+        nv.check(getattr(nv.lib(), "mfar_" + name)(*_operand(self.data, self.scales, self.e4m3), self.n_docs,
+                                                   self.n_fields, int(field), self.dim_pad, int(row_begin),
+                                                   int(n_rows), nv.ptr(out), nv.stream()), name)
         return out[:, : self.dim]
 
     def prepare_queries(self, q_vecs):
@@ -159,31 +163,12 @@ class PackedCorpus:
         if q_vecs.dim() != 2 or q_vecs.shape[1] != self.dim:
             raise ValueError(f"expected [Q,{self.dim}] query vectors, got {tuple(q_vecs.shape)}")
         q = q_vecs.to(self.device)
-        if self.e4m3:
-            if q.dtype not in (torch.float32, torch.bfloat16):
-                q = q.float()
-            if self.dim_pad != self.dim:
-                q = torch.nn.functional.pad(q, (0, self.dim_pad - self.dim))
-            q = q.contiguous()
-            out = torch.empty((q.shape[0], self.dim_pad), dtype=torch.uint8, device=self.device)
-            qs = torch.empty((q.shape[0],), dtype=torch.float32, device=self.device)
+        if self.e4m3 or self.normalize:
+            out = torch.empty((q.shape[0], self.dim_pad), dtype=self.data.dtype, device=self.device)
+            qs = torch.empty((q.shape[0],), dtype=torch.float32, device=self.device) if self.e4m3 else None
             if q.shape[0]:
-                nv.check(nv.lib().mfar_corpus_pack_rows_e4m3(
-                    nv.ptr(q), nv.F32 if q.dtype == torch.float32 else nv.BF16, q.shape[0], 0, nv.ptr(out), nv.ptr(qs),
-                    q.shape[0], 1, 0, self.dim_pad, int(self.normalize), nv.stream()), "corpus_pack_rows_e4m3 (queries)")
-            return out, qs
-        if self.normalize:
-            if q.dtype not in (torch.float32, torch.bfloat16):
-                q = q.float()
-            if self.dim_pad != self.dim:
-                q = torch.nn.functional.pad(q, (0, self.dim_pad - self.dim))
-            q = q.contiguous()
-            out = torch.empty((q.shape[0], self.dim_pad), dtype=torch.bfloat16, device=self.device)
-            if q.shape[0]:
-                nv.check(nv.lib().mfar_corpus_pack_rows(nv.ptr(q), nv.F32 if q.dtype == torch.float32 else nv.BF16,
-                                                        q.shape[0], 0, nv.ptr(out), q.shape[0], 1, 0, self.dim_pad, 1,
-                                                        nv.stream()), "corpus_pack_rows (queries)")
-            return out
+                self._pack(q, out, qs, 0, q.shape[0], 1, 0, " (queries)")
+            return (out, qs) if self.e4m3 else out
         q = q.to(torch.bfloat16)
         if self.dim_pad != self.dim:
             q = torch.nn.functional.pad(q, (0, self.dim_pad - self.dim))
@@ -287,11 +272,25 @@ class MultiFieldRetriever:
         if self.corpus is not None and self.corpus.e4m3:
             raise ValueError(f"{what} runs on a bf16 corpus only; this corpus is E4M3 (use search / score_candidates)")
 
-    def _score_topk(self, q_bf16: Optional[torch.Tensor], w: torch.Tensor, sparse, sparse_code: int, k: int,
-                    field_begin: int, n_dense: int, n_sparse: int, want_keys: bool = False, impl: Optional[str] = None,
-                    n_docs: Optional[int] = None, doc_id_base: Optional[int] = None, sparse_coo=None,
-                    bm25_entries: Optional[torch.Tensor] = None, q_scales: Optional[torch.Tensor] = None):
-        """``q_bf16``: the query operand (bf16, or E4M3 bytes with ``q_scales`` on an E4M3 corpus)."""
+    def _check_sparse_coo(self, sparse_coo) -> Tuple[torch.Tensor, torch.Tensor, Sequence[int]]:
+        if self.n_sparse == 0:
+            raise ValueError("retriever has no sparse fields")
+        ck, cv, off = sparse_coo
+        nv.require_device(ck, "sparse_coo keys"); nv.require_device(cv, "sparse_coo vals")
+        if ck.dtype != torch.int32 or ck.dim() != 2 or ck.shape[1] != 2 or cv.shape[0] != ck.shape[0]:
+            raise ValueError("sparse_coo keys must be int32 [nnz,2] with one value per row")
+        if len(off) != self.n_sparse + 1 or int(off[-1]) != ck.shape[0]:
+            raise ValueError("field_offsets must have n_sparse+1 entries ending at nnz")
+        if cv.dtype not in (torch.float16, torch.float32):
+            cv = cv.float()
+        return ck.contiguous(), cv.contiguous(), off
+
+    def _score_topk(self, q: Tuple[Optional[torch.Tensor], Optional[torch.Tensor]], w: torch.Tensor, sparse: tuple,
+                    k: int, field_begin: int, n_dense: int, n_sparse: int, want_keys: bool = False,
+                    impl: Optional[str] = None, n_docs: Optional[int] = None, doc_id_base: Optional[int] = None):
+        """``q``: the query operand of ``_queries`` (rows, scales).  ``sparse``: the sparse fields' input in one of
+        the layouts of the scoring entry points - ("rows", [Q,Fs,ld] tensor or None, dtype code),
+        ("coo", keys, vals, field_offsets) or ("bm25", int32 [n,3] token entries)."""
         Q = w.shape[0]
         n_docs = self.n_docs if n_docs is None else n_docs
         doc_id_base = self.doc_id_base if doc_id_base is None else doc_id_base
@@ -300,47 +299,30 @@ class MultiFieldRetriever:
         scores = torch.empty((Q, k), dtype=torch.float32, device=self.device)
         ids = torch.empty((Q, k), dtype=torch.int64, device=self.device)
         keys = torch.empty((Q, k), dtype=torch.int64, device=self.device) if want_keys else None
-        ws = self._workspace(Q, k, n_sparse, n_docs, 0 if bm25_entries is None else bm25_entries.shape[0])
+        layout, *sp = sparse
+        n_entries = 0
+        if layout == "bm25":
+            (ent,) = sp
+            n_entries = ent.shape[0]
+            b = self.bm25
+            sparse_args = (b.indptr, b.indices, b.data, b.vocab, n_sparse, nv.ptr(ent), n_entries)
+        elif layout == "coo":
+            ck, cv, off = sp
+            off = (ctypes.c_int64 * (n_sparse + 1))(*[int(x) for x in off])      # host array, alive through the call
+            sparse_args = (nv.ptr(ck), nv.ptr(cv), nv.F16 if cv.dtype == torch.float16 else nv.F32,
+                           ctypes.addressof(off), n_sparse)
+        else:
+            t, code = sp
+            sparse_args = (nv.ptr(t), n_sparse, code, t.shape[2] if t is not None else n_docs)
+        ws = self._workspace(Q, k, n_sparse, n_docs, n_entries)
         c = self.corpus
         e8 = c is not None and c.e4m3
-        if e8:
-            # the *_e4m3 entry points: the bf16 arguments with the corpus / query scale pointers after their operands
-            lib = nv.lib()
-            sc, qs = nv.ptr(c.scales), nv.ptr(q_scales)
-            ep = {"bm25": lambda cp, *a: lib.mfar_score_topk_bm25_e4m3(cp, sc, *a[:6], qs, *a[6:]),
-                  "coo": lambda cp, *a: lib.mfar_score_topk_coo_e4m3(cp, sc, *a[:6], qs, *a[6:]),
-                  "dense": lambda cp, *a: lib.mfar_score_topk_e4m3(cp, sc, *a[:6], qs, *a[6:])}
-        else:
-            ep = {"bm25": nv.lib().mfar_score_topk_bm25, "coo": nv.lib().mfar_score_topk_coo,
-                  "dense": nv.lib().mfar_score_topk}
-        if bm25_entries is not None:
-            b = self.bm25
-            nv.check(ep["bm25"](
-                nv.ptr(c.data) if c is not None else 0, n_docs, c.n_fields if c is not None else 0, field_begin,
-                n_dense, c.dim_pad if c is not None else 0, nv.ptr(q_bf16), Q, nv.ptr(w), b.indptr, b.indices, b.data,
-                b.vocab, n_sparse, nv.ptr(bm25_entries), bm25_entries.shape[0], doc_id_base, k, nv.ptr(keys),
-                nv.ptr(scores), nv.ptr(ids), nv.ptr(ws), ws.numel(), nv.IMPL[impl or self.impl], nv.stream()),
-                "score_topk_bm25")
-            self.last_launches = nv.lib().mfar_last_launch_count()
-            return scores, ids, keys
-        if sparse_coo is not None:
-            import ctypes
-            coo_keys, coo_vals, offsets = sparse_coo
-            off = (ctypes.c_int64 * (n_sparse + 1))(*[int(x) for x in offsets])
-            nv.check(ep["coo"](
-                nv.ptr(c.data) if c is not None else 0, n_docs, c.n_fields if c is not None else 0, field_begin,
-                n_dense, c.dim_pad if c is not None else 0, nv.ptr(q_bf16), Q, nv.ptr(w), nv.ptr(coo_keys),
-                nv.ptr(coo_vals), nv.F16 if coo_vals.dtype == torch.float16 else nv.F32, ctypes.addressof(off), n_sparse,
-                doc_id_base, k, nv.ptr(keys), nv.ptr(scores), nv.ptr(ids), nv.ptr(ws), ws.numel(),
-                nv.IMPL[impl or self.impl], nv.stream()), "score_topk_coo")
-            self.last_launches = nv.lib().mfar_last_launch_count()
-            return scores, ids, keys
-        nv.check(ep["dense"](
-            nv.ptr(c.data) if c is not None else 0, n_docs, c.n_fields if c is not None else 0, field_begin,
-            n_dense, c.dim_pad if c is not None else 0, nv.ptr(q_bf16), Q, nv.ptr(w), nv.ptr(sparse), n_sparse,
-            sparse_code, (sparse.shape[2] if sparse is not None else n_docs), doc_id_base, k, nv.ptr(keys),
-            nv.ptr(scores), nv.ptr(ids), nv.ptr(ws),
-            ws.numel(), nv.IMPL[impl or self.impl], nv.stream()), "score_topk")
+        name = "score_topk" if layout == "rows" else "score_topk_" + layout
+        fn = getattr(nv.lib(), f"mfar_{name}_e4m3" if e8 else f"mfar_{name}")
+        nv.check(fn(*_operand(c.data if c else None, c.scales if c else None, e8), n_docs, c.n_fields if c else 0,
+                    field_begin, n_dense, c.dim_pad if c else 0, *_operand(*q, e8), Q, nv.ptr(w), *sparse_args,
+                    doc_id_base, k, nv.ptr(keys), nv.ptr(scores), nv.ptr(ids), nv.ptr(ws), ws.numel(),
+                    nv.IMPL[impl or self.impl], nv.stream()), name)
         self.last_launches = nv.lib().mfar_last_launch_count()
         return scores, ids, keys
 
@@ -414,28 +396,13 @@ class MultiFieldRetriever:
         qe = self.mixture_input(q_vecs, q_emb)
         w = self.mixture.field_weights(qe, self.mask, batch=Q)
         if sparse_tokens is not None:
-            ent = self._bm25_entries(sparse_tokens)
-            scores, ids, keys = self._score_topk(q_bf16, w, None, nv.F16, k, 0, self.n_dense, self.n_sparse,
-                                                 want_keys=return_keys, impl=impl, bm25_entries=ent, q_scales=q_sc)
-            return (scores, ids, keys) if return_keys else (scores, ids)
-        if sparse_coo is not None:
-            if self.n_sparse == 0:
-                raise ValueError("retriever has no sparse fields")
-            ck, cv, off = sparse_coo
-            nv.require_device(ck, "sparse_coo keys"); nv.require_device(cv, "sparse_coo vals")
-            if ck.dtype != torch.int32 or ck.dim() != 2 or ck.shape[1] != 2 or cv.shape[0] != ck.shape[0]:
-                raise ValueError("sparse_coo keys must be int32 [nnz,2] with one value per row")
-            if len(off) != self.n_sparse + 1 or int(off[-1]) != ck.shape[0]:
-                raise ValueError("field_offsets must have n_sparse+1 entries ending at nnz")
-            if cv.dtype not in (torch.float16, torch.float32):
-                cv = cv.float()
-            scores, ids, keys = self._score_topk(q_bf16, w, None, nv.F16, k, 0, self.n_dense, self.n_sparse,
-                                                 want_keys=return_keys, impl=impl,
-                                                 sparse_coo=(ck.contiguous(), cv.contiguous(), off), q_scales=q_sc)
-            return (scores, ids, keys) if return_keys else (scores, ids)
-        sp, code = self._check_sparse(sparse, Q)
-        scores, ids, keys = self._score_topk(q_bf16, w, sp, code, k, 0, self.n_dense, self.n_sparse,
-                                             want_keys=return_keys, impl=impl, q_scales=q_sc)
+            sp = ("bm25", self._bm25_entries(sparse_tokens))
+        elif sparse_coo is not None:
+            sp = ("coo", *self._check_sparse_coo(sparse_coo))
+        else:
+            sp = ("rows", *self._check_sparse(sparse, Q))
+        scores, ids, keys = self._score_topk((q_bf16, q_sc), w, sp, k, 0, self.n_dense, self.n_sparse,
+                                             want_keys=return_keys, impl=impl)
         return (scores, ids, keys) if return_keys else (scores, ids)
 
     # ------------------------------------------------------------------ field-masking sweep in one corpus pass
@@ -488,14 +455,13 @@ class MultiFieldRetriever:
             w_rows = (w.unsqueeze(0) * masks[m0:m1].unsqueeze(1)).reshape(reps * Q, -1).contiguous()
             q_rows = q_bf16.repeat(reps, 1) if q_bf16 is not None else None
             qs_rows = q_sc.repeat(reps) if q_sc is not None else None
-            sp_rows = sp.repeat(reps, 1, 1) if sp is not None else None
-            ent_rows = None
             if ent is not None:                                            # query-major order is kept: rep-major
                 ent_rows = ent.unsqueeze(0).repeat(reps, 1, 1)
                 ent_rows[:, :, 0] += (torch.arange(reps, device=self.device, dtype=torch.int32) * Q).view(reps, 1)
-                ent_rows = ent_rows.view(-1, 3).contiguous()
-            s, i, _ = self._score_topk(q_rows, w_rows, sp_rows, code, k, 0, self.n_dense, self.n_sparse,
-                                       bm25_entries=ent_rows, q_scales=qs_rows)
+                sp_rows = ("bm25", ent_rows.view(-1, 3).contiguous())
+            else:
+                sp_rows = ("rows", sp.repeat(reps, 1, 1) if sp is not None else None, code)
+            s, i, _ = self._score_topk((q_rows, qs_rows), w_rows, sp_rows, k, 0, self.n_dense, self.n_sparse)
             out_s[m0:m1] = s.view(reps, Q, k)
             out_i[m0:m1] = i.view(reps, Q, k)
         return out_s, out_i
@@ -509,13 +475,11 @@ class MultiFieldRetriever:
         fused scoring + top-k, D2H of the [Q,k] result, stream sync.  q_vecs_host: bf16 [Q,dim_pad] host tensor
         (pinned for full PCIe speed); q_emb_host fp32 [Q,E]; sparse_host f16/f32 [Q,Fs,N].  bf16 corpus only."""
         self._require_bf16("search_host")
-        k = top_k or self.top_k
         c = self.corpus
         Q = q_vecs_host.shape[0] if q_vecs_host is not None else sparse_host.shape[0]
         if c is not None and (q_vecs_host.dtype != torch.bfloat16 or q_vecs_host.shape[1] != c.dim_pad
                               or q_vecs_host.is_cuda):
             raise ValueError("q_vecs_host must be a host bf16 [Q, dim_pad] tensor")
-        E = self.mixture.weight.shape[0] if self.mixture.query_cond else 0
         if self.mixture.query_cond and (q_emb_host is None or q_emb_host.dtype != torch.float32):
             raise ValueError("q_emb_host must be a host fp32 [Q,E] tensor")
         code = nv.F16
@@ -523,24 +487,8 @@ class MultiFieldRetriever:
             if tuple(sparse_host.shape) != (Q, self.n_sparse, self.n_docs) or not sparse_host.is_contiguous():
                 raise ValueError(f"sparse_host must be a contiguous [{Q},{self.n_sparse},{self.n_docs}] host tensor")
             code = nv.F16 if sparse_host.dtype == torch.float16 else nv.F32
-        need = nv.lib().mfar_search_host_scratch_bytes(Q, c.dim_pad if c else 0, E, self.n_dense, self.n_sparse,
-                                                       self.n_docs, code, k)
-        if self._host_scratch is None or self._host_scratch.numel() < need:
-            self._host_scratch = torch.empty(need, dtype=torch.uint8, device=self.device)
-        if out_scores is None:
-            out_scores = torch.empty((Q, k), dtype=torch.float32).pin_memory()
-        if out_ids is None:
-            out_ids = torch.empty((Q, k), dtype=torch.int64).pin_memory()
-        W = self.mixture.weight.detach().contiguous().float()
-        m = self.mask.reshape(-1).contiguous().float()
-        nv.check(nv.lib().mfar_search_host(
-            nv.ptr(c.data) if c else 0, self.n_docs, c.n_fields if c else 0, 0, self.n_dense, c.dim_pad if c else 0,
-            nv.ptr(q_vecs_host), nv.ptr(q_emb_host), Q, E, nv.ptr(W), nv.ptr(m), int(self.mixture.query_cond),
-            nv.ptr(sparse_host), self.n_sparse, code, self.doc_id_base, k, nv.ptr(out_scores), nv.ptr(out_ids),
-            nv.ptr(self._host_scratch), self._host_scratch.numel(), nv.IMPL[impl or self.impl], nv.stream()),
-            "search_host")
-        self.last_launches = nv.lib().mfar_last_launch_count()
-        return out_scores, out_ids
+        return self._search_host("search_host", Q, q_vecs_host, q_emb_host, (nv.ptr(sparse_host), self.n_sparse, code),
+                                 code, top_k, out_scores, out_ids, impl)
 
     def search_host_bm25(self, q_vecs_host: Optional[torch.Tensor], q_emb_host: Optional[torch.Tensor],
                          entries_host: torch.Tensor, top_k: Optional[int] = None,
@@ -552,7 +500,6 @@ class MultiFieldRetriever:
         if self.bm25 is None:
             raise ValueError("search_host_bm25 needs a retriever built with sparse_indices=[DeviceBM25, ...]")
         self._require_bf16("search_host_bm25")
-        k = top_k or self.top_k
         c = self.corpus
         if q_vecs_host is not None:
             Q = q_vecs_host.shape[0]
@@ -563,15 +510,28 @@ class MultiFieldRetriever:
         if c is not None and (q_vecs_host.dtype != torch.bfloat16 or q_vecs_host.shape[1] != c.dim_pad
                               or q_vecs_host.is_cuda):
             raise ValueError("q_vecs_host must be a host bf16 [Q, dim_pad] tensor")
-        E = self.mixture.weight.shape[0] if self.mixture.query_cond else 0
         if self.mixture.query_cond and (q_emb_host is None or q_emb_host.dtype != torch.float32):
             raise ValueError("q_emb_host must be a host fp32 [Q,E] tensor")
         if entries_host.is_cuda or entries_host.dtype != torch.int32 or entries_host.dim() != 2 \
                 or entries_host.shape[1] != 3 or not entries_host.is_contiguous():
             raise ValueError("entries_host must be a contiguous host int32 [n,3] tensor")
         n_ent = entries_host.shape[0]
-        need = nv.lib().mfar_search_host_bm25_scratch_bytes(Q, c.dim_pad if c else 0, E, self.n_dense, self.n_sparse,
-                                                            self.n_docs, n_ent, k)
+        b = self.bm25
+        return self._search_host("search_host_bm25", Q, q_vecs_host, q_emb_host,
+                                 (b.indptr, b.indices, b.data, b.vocab, self.n_sparse,
+                                  nv.ptr(entries_host) if n_ent else 0, n_ent),
+                                 n_ent, top_k, out_scores, out_ids, impl)
+
+    def _search_host(self, entry: str, Q: int, q_vecs_host, q_emb_host, sparse_args: tuple, sizing: int,
+                     top_k: Optional[int], out_scores: Optional[torch.Tensor], out_ids: Optional[torch.Tensor],
+                     impl: Optional[str]):
+        """The call of ``mfar_<entry>`` with the batch's sparse-field arguments ``sparse_args``.  ``sizing`` is the
+        sparse argument of ``mfar_<entry>_scratch_bytes``: the score dtype, or the number of token entries."""
+        k = top_k or self.top_k
+        c = self.corpus
+        E = self.mixture.weight.shape[0] if self.mixture.query_cond else 0
+        need = getattr(nv.lib(), f"mfar_{entry}_scratch_bytes")(Q, c.dim_pad if c else 0, E, self.n_dense,
+                                                                self.n_sparse, self.n_docs, sizing, k)
         if self._host_scratch is None or self._host_scratch.numel() < need:
             self._host_scratch = torch.empty(need, dtype=torch.uint8, device=self.device)
         if out_scores is None:
@@ -580,13 +540,11 @@ class MultiFieldRetriever:
             out_ids = torch.empty((Q, k), dtype=torch.int64).pin_memory()
         W = self.mixture.weight.detach().contiguous().float()
         m = self.mask.reshape(-1).contiguous().float()
-        b = self.bm25
-        nv.check(nv.lib().mfar_search_host_bm25(
+        nv.check(getattr(nv.lib(), "mfar_" + entry)(
             nv.ptr(c.data) if c else 0, self.n_docs, c.n_fields if c else 0, 0, self.n_dense, c.dim_pad if c else 0,
             nv.ptr(q_vecs_host), nv.ptr(q_emb_host), Q, E, nv.ptr(W), nv.ptr(m), int(self.mixture.query_cond),
-            b.indptr, b.indices, b.data, b.vocab, self.n_sparse, nv.ptr(entries_host) if n_ent else 0, n_ent,
-            self.doc_id_base, k, nv.ptr(out_scores), nv.ptr(out_ids), nv.ptr(self._host_scratch),
-            self._host_scratch.numel(), nv.IMPL[impl or self.impl], nv.stream()), "search_host_bm25")
+            *sparse_args, self.doc_id_base, k, nv.ptr(out_scores), nv.ptr(out_ids), nv.ptr(self._host_scratch),
+            self._host_scratch.numel(), nv.IMPL[impl or self.impl], nv.stream()), entry)
         self.last_launches = nv.lib().mfar_last_launch_count()
         return out_scores, out_ids
 
@@ -606,7 +564,7 @@ class MultiFieldRetriever:
         ones = torch.ones((Q, 1), dtype=torch.float32, device=self.device)
         all_s, all_i, launches = [], [], 0
         for f in range(self.n_dense):
-            s, i, _ = self._score_topk(q_bf16, ones, None, nv.F16, k, f, 1, 0, q_scales=q_sc)
+            s, i, _ = self._score_topk((q_bf16, q_sc), ones, ("rows", None, nv.F16), k, f, 1, 0)
             launches += self.last_launches
             i = i - self.doc_id_base
             if zero_init:
@@ -616,7 +574,7 @@ class MultiFieldRetriever:
             all_i.append(i)
         for j in range(self.n_sparse):
             sj = sp[:, j:j + 1, :].contiguous()
-            s, i, _ = self._score_topk(None, ones, sj, code, k, 0, 0, 1)
+            s, i, _ = self._score_topk((None, None), ones, ("rows", sj, code), k, 0, 0, 1)
             launches += self.last_launches
             all_s.append(s)
             all_i.append(i - self.doc_id_base)
@@ -636,15 +594,10 @@ class MultiFieldRetriever:
         out = torch.zeros((self.num_fields, Q, C), dtype=torch.float32, device=self.device)
         if self.n_dense and C:
             c = self.corpus
-            if c.e4m3:
-                nv.check(nv.lib().mfar_score_candidates_e4m3(nv.ptr(c.data), nv.ptr(c.scales), self.n_docs, c.n_fields,
-                                                             0, self.n_dense, c.dim_pad, nv.ptr(q_bf16), nv.ptr(q_sc),
-                                                             Q, nv.ptr(rows), C, nv.ptr(out), nv.stream()),
-                         "score_candidates_e4m3")
-            else:
-                nv.check(nv.lib().mfar_score_candidates(nv.ptr(c.data), self.n_docs, c.n_fields, 0, self.n_dense,
-                                                        c.dim_pad, nv.ptr(q_bf16), Q, nv.ptr(rows), C, nv.ptr(out),
-                                                        nv.stream()), "score_candidates")
+            name = "score_candidates_e4m3" if c.e4m3 else "score_candidates"
+            nv.check(getattr(nv.lib(), "mfar_" + name)(*_operand(c.data, c.scales, c.e4m3), self.n_docs, c.n_fields, 0,
+                                                       self.n_dense, c.dim_pad, *_operand(q_bf16, q_sc, c.e4m3), Q,
+                                                       nv.ptr(rows), C, nv.ptr(out), nv.stream()), name)
         if self.n_sparse and C:
             sp, _ = self._check_sparse(sparse, Q)
             g = sp[:, :, rows.clamp(min=0)].float()                       # [Q,Fs,C] gather (index.py:116)
