@@ -13,7 +13,7 @@
  *     point synchronises (except the *_host convenience calls, which say so);
  *   - return value: 0 = MFAR_OK, otherwise an mfar_status (mfar_status_string() names it);
  *   - re-entrant, no global mutable state apart from a per-process cache of TMA descriptors'
- *     driver entry point; one process per GPU;
+ *     driver entry point and the per-device diagnostic counter of mfar_profile_cluster4_ctas(); one process per GPU;
  *   - sm_100 only.  There is no CPU fallback: on any other device every compute entry point
  *     returns MFAR_ERR_ARCH.
  */
@@ -414,6 +414,10 @@ MFAR_API int mfar_last_launch_count(void);
  * by default and the compute entry points never depend on it. */
 MFAR_API int mfar_profile_enable(int on);
 MFAR_API int mfar_profile_collect(float* out_ms_host, int max_n);
+/* CTAs of the large-batch scoring kernel that ran in 4-CTA clusters (two CTA pairs sharing every doc tile by TMA
+ * multicast) on the current device since the previous call, which resets the count; -1 on a CUDA error.  Synchronous.
+ * Diagnostics only: the count is kept whether profiling is armed or not. */
+MFAR_API long long mfar_profile_cluster4_ctas(void);
 
 #ifdef __cplusplus
 }

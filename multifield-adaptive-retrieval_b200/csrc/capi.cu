@@ -905,4 +905,6 @@ int mfar_profile_collect(float* out_ms_host, int max_n) {
   return n;
 }
 
+long long mfar_profile_cluster4_ctas(void) { return qs_cluster4_ctas_collect(); }
+
 }  // extern "C"

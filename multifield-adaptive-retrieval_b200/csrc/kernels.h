@@ -123,6 +123,7 @@ int launch_score_simt(const ScoreArgs& a, void* ws_base, int workers, int q_pad,
 int launch_score_tc(const ScoreArgs& a, void* ws_base, int workers, int q_tiles, int q_pad, cudaStream_t st);
 // Query-stationary tcgen05 pass for large batches (queries resident in TMEM, CTA pairs when cg == 2).
 int launch_score_qs(const ScoreArgs& a, void* ws_base, int workers, int q_tiles, int cg, cudaStream_t st);
+long long qs_cluster4_ctas_collect();   // CTAs that ran in 4-CTA clusters since the last call (resets); -1: CUDA error
 bool score_qs_supported(const ScoreArgs& a);
 void score_qs_geometry(int Q, int n_tiles, int* q_tiles, int* workers, int* cg);
 // candidate lists per (worker CTA, query): 2 for a single-field scorer in CTA-pair mode (two epilogue sets), else 1

@@ -183,11 +183,16 @@ __device__ __noinline__ QsCompacted qs_compact_lists(unsigned need, uint64_t* my
   return QsCompacted{thr, cnt};
 }
 
+// CTAs that ran in 4-CTA clusters, since the last mfar_profile_cluster4_ctas() (one atomic per CTA)
+__device__ unsigned long long g_qs_cluster4_ctas;
+
 // SP: the epilogue gathers the sparse fields itself (qs_seed_sparse) - a separate instantiation, so the dense-only
-// kernels keep their register allocation
+// kernels keep their register allocation.  map_bh: the corpus view of map_b with half its K chunks per box (the
+// multicast loads of a 4-CTA cluster).
 template <int CG, int ES, bool SP>
 __global__ void __launch_bounds__(qs_threads(ES, SP), 1)
-score_qs_kernel(const __grid_constant__ CUtensorMap map_b, const __grid_constant__ CUtensorMap map_sp, QsParams p) {
+score_qs_kernel(const __grid_constant__ CUtensorMap map_b, const __grid_constant__ CUtensorMap map_bh,
+                const __grid_constant__ CUtensorMap map_sp, QsParams p) {
   constexpr int kRowsPerCta = kQsDocs / CG;               // doc rows this CTA loads per stage
   constexpr int kChunkBytes = kRowsPerCta * kChunkK * 2;  // one [rows x 64] K-major block: 8 KB (CG=1) / 4 KB (CG=2)
   const int kStageBytes = p.kc_per_stage * kChunkBytes;
@@ -218,7 +223,13 @@ score_qs_kernel(const __grid_constant__ CUtensorMap map_b, const __grid_constant
   const int G = gridDim.y;
   const int q0 = blockIdx.x * kQsQ;                // first query of this CTA
   const uint32_t cta_rank = (CG == 2) ? cluster_ctarank() : 0u;
-  const bool leader = cta_rank == 0;
+  // A 4-CTA cluster (launched as the preferred cluster shape) is the two pairs of one worker column: ranks {0,1} and
+  // {2,3}, each a cta_group::2 pair with its even rank as leader.  Where the GPC had no room, the hardware formed
+  // 2-CTA clusters instead; a column can come up either way.
+  const uint32_t cl_size = (CG == 2) ? cluster_nctarank() : 1u;
+  const bool mc = CG == 2 && cl_size == 4;         // doc tiles shared between the pairs by TMA multicast
+  const bool leader = (cta_rank & 1u) == 0;
+  const uint32_t pair_mask = 0x3u << (cta_rank & 2u);
   int* err = p.ws.err;
 
   // ---- one-time setup
@@ -228,10 +239,12 @@ score_qs_kernel(const __grid_constant__ CUtensorMap map_b, const __grid_constant
   }
   if (warp == 0 && lane == 0) {
     tma_prefetch_desc(&map_b);
-    for (int s = 0; s < p.stages; ++s) { mbar_init(&full_bar[s], 1); mbar_init(&empty_bar[s], 1); }
+    // multicast: a stage slot is written by both pairs' producers, so both pairs' MMAs must have consumed it
+    for (int s = 0; s < p.stages; ++s) { mbar_init(&full_bar[s], 1); mbar_init(&empty_bar[s], mc ? 2 : 1); }
     for (int b = 0; b < 2; ++b) { mbar_init(&tfull_bar[b], 1); mbar_init(&tempty_bar[b], 4 * CG); }
     for (int b = 0; b < kSpMaxSlots; ++b) { mbar_init(&sfull_bar[b], 1); mbar_init(&sempty_bar[b], 4); }
     if (SP) tma_prefetch_desc(&map_sp);
+    if (mc) { tma_prefetch_desc(&map_bh); atomicAdd(&g_qs_cluster4_ctas, 1ull); }
     fence_barrier_init();
   }
   if (warp == 1) {
@@ -301,7 +314,9 @@ score_qs_kernel(const __grid_constant__ CUtensorMap map_b, const __grid_constant
       const int n_groups = gridDim.x / CG;
       const int my_group = blockIdx.x / CG;
       int* prog = p.ws.progress + g * n_groups;
-      bool lockstep = n_groups > 1 && leader && (G * n_groups <= kProgressInts);
+      // (the pairs of one cluster are already held together by the shared stage slots: a column that is one cluster
+      // needs no counters)
+      bool lockstep = n_groups > 1 && leader && gridDim.x > cl_size && (G * n_groups <= kProgressInts);
       // a sync point every ~8 MMA units (= every half-tile when n_dense >= 8): the global round trip must not sit
       // in front of every TMA issue of a few-field scorer
       const int sync_every = p.n_dense >= 8 ? 1 : (8 + p.n_dense - 1) / p.n_dense;
@@ -324,7 +339,7 @@ score_qs_kernel(const __grid_constant__ CUtensorMap map_b, const __grid_constant
           }
           for (int f = 0; f < p.n_dense; ++f) {
             const int row0 = (t * p.corpus_fields + p.field_begin + f) * kTileDocs + h * kQsDocs +
-                             int(cta_rank) * kRowsPerCta;
+                             int(cta_rank & 1u) * kRowsPerCta;
             const int ib = unit & 1;                // issuer (= accumulator buffer) of this unit
             ++unit;
             for (int s = 0; s < stages_per_unit; ++s) {
@@ -332,7 +347,14 @@ score_qs_kernel(const __grid_constant__ CUtensorMap map_b, const __grid_constant
               const uint32_t phase = ib ? ph1 : ph0;
               mbar_wait(&empty_bar[stage], phase ^ 1, err, 11);
               if (elect_one()) {
-                if (CG == 2) {
+                if (mc) {
+                  // CTA r and r ^ 2 need the same rows: each loads one K half of the stage into both of them
+                  const int half = p.kc_per_stage >> 1;
+                  const int kh = int(cta_rank >> 1) * half;
+                  if (leader) mbar_expect_tx(&full_bar[stage], kStageBytes * 2);
+                  tma_load_3d_cg2_mc(&map_bh, &full_bar[stage], smem_b + size_t(stage) * kStageBytes + size_t(kh) * kChunkBytes,
+                                     0, row0, s * p.kc_per_stage + kh, uint16_t((1u << cta_rank) | (1u << (cta_rank ^ 2u))));
+                } else if (CG == 2) {
                   if (leader) mbar_expect_tx(&full_bar[stage], kStageBytes * 2);
                   tma_load_3d_cg2(&map_b, &full_bar[stage], smem_b + size_t(stage) * kStageBytes, 0, row0,
                                   s * p.kc_per_stage);
@@ -347,6 +369,16 @@ score_qs_kernel(const __grid_constant__ CUtensorMap map_b, const __grid_constant
               else { if (++st0 == S_half) { st0 = 0; ph0 ^= 1u; } }
             }
           }
+        }
+      }
+      // The MMAs of another pair release this CTA's stages through remote commits: wait until every stage has been
+      // released after its last fill, so that no commit lands in this CTA's shared memory after it has exited.
+      if (CG == 2) {
+        for (int i = 0; i < S_half; ++i) {
+          mbar_wait(&empty_bar[st0], ph0 ^ 1, err, 11);
+          mbar_wait(&empty_bar[S_half + st1], ph1 ^ 1, err, 11);
+          if (++st0 == S_half) { st0 = 0; ph0 ^= 1u; }
+          if (++st1 == S_half) { st1 = 0; ph1 ^= 1u; }
         }
       }
     }
@@ -419,9 +451,11 @@ score_qs_kernel(const __grid_constant__ CUtensorMap map_b, const __grid_constant
                                                                             desc0 + uint64_t(c * (kChunkBytes >> 4)),
                                                                             idesc, first_stage && c == 0, issue);
           __syncwarp();
-          if (elect_one()) { if (CG == 2) tc_commit_cg2(&empty_bar[stage], 0x3); else tc_commit(&empty_bar[stage]); }
+          if (elect_one()) {
+            if (CG == 2) tc_commit_cg2(&empty_bar[stage], mc ? 0xF : pair_mask); else tc_commit(&empty_bar[stage]);
+          }
         }
-        if (elect_one()) { if (CG == 2) tc_commit_cg2(&tfull_bar[buf], 0x3); else tc_commit(&tfull_bar[buf]); }
+        if (elect_one()) { if (CG == 2) tc_commit_cg2(&tfull_bar[buf], pair_mask); else tc_commit(&tfull_bar[buf]); }
         __syncwarp();
         QS_TICK(t_issue)
       }
@@ -515,7 +549,7 @@ score_qs_kernel(const __grid_constant__ CUtensorMap map_b, const __grid_constant
             tc_fence_before();
             __syncwarp();
             if (lane == 0) {                         // one arrival per epilogue warp frees the accumulator buffer
-              if (CG == 2) mbar_arrive_cluster_rank0(&tempty_bar[buf]); else mbar_arrive(&tempty_bar[buf]);
+              if (CG == 2) mbar_arrive_cluster(&tempty_bar[buf], cta_rank & ~1u); else mbar_arrive(&tempty_bar[buf]);
             }
 #pragma unroll
             for (int c = 0; c < kQsDocs; ++c) acc[c] = fmaf(wf, __uint_as_float(v[c]), acc[c]);
@@ -657,10 +691,22 @@ static int launch_qs_impl(const ScoreArgs& a, void* ws_base, int workers, int q_
   const size_t smem = qs_smem_bytes(n_w, stages, kStageBytes, sp_slots);
   if (smem > smem_cap) return MFAR_ERR_SHAPE;
 
+  // Two CTA pairs per cluster where they read the same doc tiles (grid x = query tiles: one cluster of 4 is two pairs
+  // of one worker column) and a stage splits into two K halves: each doc tile then crosses from L2 to the SMs once per
+  // column instead of once per pair.  A preferred cluster, not a required one: GPCs with no room for 4 CTAs get
+  // 2-CTA clusters, so every SM stays busy.
+  const bool cluster4 = CG == 2 && q_tiles % 4 == 0 && kc % 2 == 0;
+  const uint64_t corpus_rows = uint64_t(a.n_tiles) * a.corpus_fields * kTileDocs;
   CUtensorMap map_b;
-  int rc = make_tensor_map_kchunked(&map_b, a.corpus, uint64_t(a.n_tiles) * a.corpus_fields * kTileDocs, a.dim,
-                                    kQsDocs / CG, kc, CU_TENSOR_MAP_L2_PROMOTION_L2_256B);
+  int rc = make_tensor_map_kchunked(&map_b, a.corpus, corpus_rows, a.dim, kQsDocs / CG, kc,
+                                    CU_TENSOR_MAP_L2_PROMOTION_L2_256B);
   if (rc) return rc;
+  CUtensorMap map_bh = map_b;                       // unused unless cluster4
+  if (cluster4) {
+    rc = make_tensor_map_kchunked(&map_bh, a.corpus, corpus_rows, a.dim, kQsDocs / CG, kc / 2,
+                                  CU_TENSOR_MAP_L2_PROMOTION_L2_256B);
+    if (rc) return rc;
+  }
   CUtensorMap map_sp = map_b;                       // unused by the dense-only kernels
   if (SP) {
     rc = make_tensor_map_sparse_rows(&map_sp, a.sparse, a.sparse_dtype == MFAR_F16, uint64_t(a.sparse_ld),
@@ -680,13 +726,24 @@ static int launch_qs_impl(const ScoreArgs& a, void* ws_base, int workers, int q_
   cfg.blockDim = dim3(qs_threads(ES, SP));
   cfg.dynamicSmemBytes = smem;
   cfg.stream = st;
-  cudaLaunchAttribute attr[1];
+  cudaLaunchAttribute attr[2];
   attr[0].id = cudaLaunchAttributeClusterDimension;
   attr[0].val.clusterDim.x = CG; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
+  attr[1].id = cudaLaunchAttributePreferredClusterDimension;
+  attr[1].val.preferredClusterDim.x = 4; attr[1].val.preferredClusterDim.y = 1; attr[1].val.preferredClusterDim.z = 1;
   cfg.attrs = attr;
-  cfg.numAttrs = 1;
-  MFAR_CUDA_OK(cudaLaunchKernelEx(&cfg, score_qs_kernel<CG, ES, SP>, map_b, map_sp, p));
+  cfg.numAttrs = cluster4 ? 2 : 1;
+  MFAR_CUDA_OK(cudaLaunchKernelEx(&cfg, score_qs_kernel<CG, ES, SP>, map_b, map_bh, map_sp, p));
   return MFAR_OK;
+}
+
+long long qs_cluster4_ctas_collect() {
+  unsigned long long n = 0;
+  const unsigned long long zero = 0;
+  if (cudaMemcpyFromSymbol(&n, g_qs_cluster4_ctas, sizeof(n)) != cudaSuccess ||
+      cudaMemcpyToSymbol(g_qs_cluster4_ctas, &zero, sizeof(zero)) != cudaSuccess)
+    return -1;
+  return static_cast<long long>(n);
 }
 
 int launch_score_qs(const ScoreArgs& a, void* ws_base, int workers, int q_tiles, int cg, cudaStream_t st) {

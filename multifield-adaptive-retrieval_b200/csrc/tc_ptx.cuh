@@ -162,6 +162,11 @@ __device__ __forceinline__ uint32_t cluster_ctarank() {
   asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
   return r;
 }
+__device__ __forceinline__ uint32_t cluster_nctarank() {
+  uint32_t r;
+  asm volatile("mov.u32 %0, %%cluster_nctarank;" : "=r"(r));
+  return r;
+}
 __device__ __forceinline__ void cluster_sync_all() {
   asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory");
   asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory");
@@ -186,6 +191,16 @@ __device__ __forceinline__ void tma_load_3d_cg2(const CUtensorMap* map, uint64_t
       "cp.async.bulk.tensor.3d.cta_group::2.shared::cluster.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5}], [%2];"
       ::"r"(smem_u32(dst)), "l"(map), "r"(smem_u32(bar) & kPeerBitMask), "r"(c0), "r"(c1), "r"(c2) : "memory");
 }
+// the same, multicast: the box lands at the same offset in every CTA of cta_mask, and each destination's transaction
+// bytes land on the mbarrier of that destination's pair leader (even rank)
+__device__ __forceinline__ void tma_load_3d_cg2_mc(const CUtensorMap* map, uint64_t* bar, void* dst, int c0, int c1, int c2,
+                                                   uint16_t cta_mask) {
+  asm volatile(
+      "cp.async.bulk.tensor.3d.cta_group::2.shared::cluster.global.tile.mbarrier::complete_tx::bytes.multicast::cluster"
+      " [%0], [%1, {%3, %4, %5}], [%2], %6;"
+      ::"r"(smem_u32(dst)), "l"(map), "r"(smem_u32(bar) & kPeerBitMask), "r"(c0), "r"(c1), "r"(c2), "h"(cta_mask)
+      : "memory");
+}
 __device__ __forceinline__ void tma_load_3d(const CUtensorMap* map, uint64_t* bar, void* dst, int c0, int c1, int c2) {
   asm volatile(
       "cp.async.bulk.tensor.3d.shared::cluster.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5}], [%2];"
@@ -195,8 +210,13 @@ __device__ __forceinline__ void tc_commit_cg2(uint64_t* bar, uint16_t cta_mask) 
   asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
                ::"r"(smem_u32(bar)), "h"(cta_mask) : "memory");
 }
-__device__ __forceinline__ void mbar_arrive_cluster_rank0(uint64_t* bar) {
-  asm volatile("mbarrier.arrive.shared::cluster.b64 _, [%0];" ::"r"(smem_u32(bar) & kPeerBitMask) : "memory");
+// arrive on the mbarrier at the same offset in the shared memory of cluster CTA `rank`
+__device__ __forceinline__ void mbar_arrive_cluster(uint64_t* bar, uint32_t rank) {
+  asm volatile(
+      "{\n\t.reg .b32 a;\n\t"
+      "mapa.shared::cluster.u32 a, %0, %1;\n\t"
+      "mbarrier.arrive.shared::cluster.b64 _, [a];\n\t}"
+      ::"r"(smem_u32(bar)), "r"(rank) : "memory");
 }
 
 // ------------------------------------------------------------------------------------ A operand in tensor memory

@@ -76,6 +76,7 @@ PROTOTYPES = {
     "mfar_last_launch_count": (_i, []),
     "mfar_profile_enable": (_i, [_i]),
     "mfar_profile_collect": (_i, [_vp, _i]),
+    "mfar_profile_cluster4_ctas": (C.c_longlong, []),
 }
 
 
