@@ -263,6 +263,73 @@ MFAR_API int mfar_score_topk_bm25_e4m3(const void* corpus, const float* corpus_s
                                        float* out_scores, int64_t* out_ids, void* workspace, size_t workspace_bytes,
                                        int impl, void* stream);
 
+/* ------------------------------------------------------------------------------------------
+ * Filtered search: the six scoring entry points above with a doc filter.  No reference counterpart - a widening
+ * (DESIGN §0, §4.5): deleted docs, a metadata subset or docs a query has already seen are left out of the top-k
+ * inside the scoring pass, so a query still gets k eligible docs however many of its best docs are ineligible.
+ *   filter_bits  DEVICE uint32 bitmap over GLOBAL doc ids: bit d of word d >> 5 set <=> doc d is eligible (the
+ *                layout of mfar_sparse_coo_count's safe_bits); 4-byte aligned
+ *   filter_rows  1: one row [filter_ld] shared by every query;  Q: one row per query, [Q, filter_ld]
+ *   filter_ld    words per row, 32 * filter_ld >= doc_id_base + n_docs
+ * Each takes its unfiltered twin's arguments with these three after doc_id_base.  Result: the (score desc, id asc)
+ * top-k of the eligible docs (NaN > +inf > finite > -inf); a query with fewer than k eligible docs gets (-inf, -1) in
+ * the remaining slots.  Workspace sizes are the twin's.  MFAR_ERR_ARG: filter_bits NULL or misaligned, filter_rows
+ * not 1 or Q;  MFAR_ERR_SHAPE: a row shorter than doc_id_base + n_docs bits.
+ * ------------------------------------------------------------------------------------------ */
+MFAR_API int mfar_score_topk_filtered(const void* corpus, int64_t n_docs, int corpus_fields, int field_begin,
+                                      int n_dense, int dim, const void* q_vecs, int Q, const float* w,
+                                      const void* sparse, int n_sparse, int sparse_dtype, int64_t sparse_ld,
+                                      int64_t doc_id_base, const uint32_t* filter_bits, int filter_rows,
+                                      int64_t filter_ld, int k, uint64_t* out_keys, float* out_scores,
+                                      int64_t* out_ids, void* workspace, size_t workspace_bytes, int impl,
+                                      void* stream);
+/* mfar_score_topk_coo with a doc filter (no reference counterpart, DESIGN §4.5) */
+MFAR_API int mfar_score_topk_coo_filtered(const void* corpus, int64_t n_docs, int corpus_fields, int field_begin,
+                                          int n_dense, int dim, const void* q_vecs, int Q, const float* w,
+                                          const int32_t* coo_keys, const void* coo_vals, int coo_dtype,
+                                          const int64_t* field_offsets_host, int n_sparse, int64_t doc_id_base,
+                                          const uint32_t* filter_bits, int filter_rows, int64_t filter_ld, int k,
+                                          uint64_t* out_keys, float* out_scores, int64_t* out_ids, void* workspace,
+                                          size_t workspace_bytes, int impl, void* stream);
+/* mfar_score_topk_bm25 with a doc filter (no reference counterpart, DESIGN §4.5) */
+MFAR_API int mfar_score_topk_bm25_filtered(const void* corpus, int64_t n_docs, int corpus_fields, int field_begin,
+                                           int n_dense, int dim, const void* q_vecs, int Q, const float* w,
+                                           const void* const* indptr_host, const void* const* indices_host,
+                                           const void* const* data_host, const int32_t* vocab_host, int n_sparse,
+                                           const int32_t* entries, int64_t n_entries, int64_t doc_id_base,
+                                           const uint32_t* filter_bits, int filter_rows, int64_t filter_ld, int k,
+                                           uint64_t* out_keys, float* out_scores, int64_t* out_ids, void* workspace,
+                                           size_t workspace_bytes, int impl, void* stream);
+/* mfar_score_topk_e4m3 with a doc filter (no reference counterpart, DESIGN §4.5) */
+MFAR_API int mfar_score_topk_e4m3_filtered(const void* corpus, const float* corpus_scales, int64_t n_docs,
+                                           int corpus_fields, int field_begin, int n_dense, int dim,
+                                           const void* q_vecs, const float* q_scales, int Q, const float* w,
+                                           const void* sparse, int n_sparse, int sparse_dtype, int64_t sparse_ld,
+                                           int64_t doc_id_base, const uint32_t* filter_bits, int filter_rows,
+                                           int64_t filter_ld, int k, uint64_t* out_keys, float* out_scores,
+                                           int64_t* out_ids, void* workspace, size_t workspace_bytes, int impl,
+                                           void* stream);
+/* mfar_score_topk_coo_e4m3 with a doc filter (no reference counterpart, DESIGN §4.5) */
+MFAR_API int mfar_score_topk_coo_e4m3_filtered(const void* corpus, const float* corpus_scales, int64_t n_docs,
+                                               int corpus_fields, int field_begin, int n_dense, int dim,
+                                               const void* q_vecs, const float* q_scales, int Q, const float* w,
+                                               const int32_t* coo_keys, const void* coo_vals, int coo_dtype,
+                                               const int64_t* field_offsets_host, int n_sparse, int64_t doc_id_base,
+                                               const uint32_t* filter_bits, int filter_rows, int64_t filter_ld, int k,
+                                               uint64_t* out_keys, float* out_scores, int64_t* out_ids,
+                                               void* workspace, size_t workspace_bytes, int impl, void* stream);
+/* mfar_score_topk_bm25_e4m3 with a doc filter (no reference counterpart, DESIGN §4.5) */
+MFAR_API int mfar_score_topk_bm25_e4m3_filtered(const void* corpus, const float* corpus_scales, int64_t n_docs,
+                                                int corpus_fields, int field_begin, int n_dense, int dim,
+                                                const void* q_vecs, const float* q_scales, int Q, const float* w,
+                                                const void* const* indptr_host, const void* const* indices_host,
+                                                const void* const* data_host, const int32_t* vocab_host,
+                                                int n_sparse, const int32_t* entries, int64_t n_entries,
+                                                int64_t doc_id_base, const uint32_t* filter_bits, int filter_rows,
+                                                int64_t filter_ld, int k, uint64_t* out_keys, float* out_scores,
+                                                int64_t* out_ids, void* workspace, size_t workspace_bytes, int impl,
+                                                void* stream);
+
 /* Merge L sorted-or-unsorted key lists per query into the global top-k.  Used for (a) the
  * per-CTA partial lists inside mfar_score_topk and (b) the per-shard lists after the NCCL
  * all-gather (replaces the {rank}.qres file merge of mfar/modeling/contrastive.py:616-631).

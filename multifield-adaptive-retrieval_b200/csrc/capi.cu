@@ -273,6 +273,7 @@ static ScoreArgs dense_operands(int dtype, const void* corpus, const float* corp
 
 // Moves every per-doc pointer and count of `a` past its first `tiles` tiles (the pass behind a seeding prefix).  A new
 // per-doc field of ScoreArgs must be moved here too, or that pass scores the prefix twice and reads past the shard.
+// (The doc filter is indexed by global doc id, doc_id_base + local doc: moving doc_id_base moves it.)
 static void skip_tiles(ScoreArgs& a, int tiles) {
   const int64_t docs = int64_t(tiles) * kTileDocs;
   const size_t rows = size_t(tiles) * a.corpus_fields * kTileDocs;
@@ -288,10 +289,21 @@ static void skip_tiles(ScoreArgs& a, int tiles) {
   }
 }
 
+// The doc filter of a *_filtered call: bitmap rows over global doc ids, `rows` = 1 (shared) or Q, `ld` words each.
+struct FilterInput {
+  bool on = false; const uint32_t* bits = nullptr; int rows = 0; int64_t ld = 0;
+};
+
+static FilterInput filter_input(const uint32_t* bits, int rows, int64_t ld) {
+  FilterInput f;
+  f.on = true; f.bits = bits; f.rows = rows; f.ld = ld;
+  return f;
+}
+
 static int score_topk_core(ScoreArgs a, int64_t n_docs, int corpus_fields, int field_begin, int n_dense, int dim,
                            int Q, const float* w, const SparseInput& sp, int64_t doc_id_base, int k, uint64_t* out_keys,
                            float* out_scores, int64_t* out_ids, void* workspace, size_t workspace_bytes, int impl,
-                           void* stream) {
+                           void* stream, const FilterInput& filt = FilterInput{}) {
   if (sp.status) return sp.status;
   const int n_sparse = sp.n_sparse;
   t_last_launches = 0;
@@ -308,6 +320,11 @@ static int score_topk_core(ScoreArgs a, int64_t n_docs, int corpus_fields, int f
     return MFAR_ERR_ARG;
   if (k <= 0 || k > MFAR_MAX_K) return MFAR_ERR_SHAPE;
   if (doc_id_base < 0 || doc_id_base + n_docs > (int64_t(1) << 32)) return MFAR_ERR_SHAPE;
+  if (filt.on) {
+    if (!filt.bits || reinterpret_cast<uintptr_t>(filt.bits) % 4 != 0 || (filt.rows != 1 && filt.rows != Q))
+      return MFAR_ERR_ARG;
+    if (filt.ld < (doc_id_base + n_docs + 31) / 32) return MFAR_ERR_SHAPE;   // a row covers every doc of the shard
+  }
   if (impl < MFAR_IMPL_AUTO || impl > MFAR_IMPL_TCGEN05_QS) return MFAR_ERR_ARG;
   if (int rc = check_arch()) return rc;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
@@ -315,6 +332,11 @@ static int score_topk_core(ScoreArgs a, int64_t n_docs, int corpus_fields, int f
   a.n_docs = n_docs; a.n_tiles = int((n_docs + kTileDocs - 1) / kTileDocs);
   a.corpus_fields = corpus_fields; a.field_begin = field_begin; a.n_dense = n_dense; a.dim = dim;
   a.Q = Q; a.w = w; a.w_ld = n_dense + n_sparse; a.doc_id_base = doc_id_base; a.k = k;
+  if (filt.on) {
+    a.filter_bits = filt.bits;
+    a.filter_stride = filt.rows == 1 ? 0 : filt.ld;
+    a.filter_words = int((doc_id_base + n_docs + 31) / 32);    // unchanged by skip_tiles
+  }
   if (n_dense > 0 && impl == MFAR_IMPL_TCGEN05 && !score_tc_supported(a)) return MFAR_ERR_SHAPE;
   if (n_dense > 0 && impl == MFAR_IMPL_TCGEN05_QS && !score_qs_supported(a)) return MFAR_ERR_SHAPE;
   const Geometry g = resolve_geometry(a, impl);
@@ -596,6 +618,90 @@ int mfar_score_topk_bm25_e4m3(const void* corpus, const float* corpus_scales, in
                          field_begin, n_dense, dim, Q, w,
                          bm25_input(indptr_host, indices_host, data_host, vocab_host, n_sparse, entries, n_entries),
                          doc_id_base, k, out_keys, out_scores, out_ids, workspace, workspace_bytes, impl, stream);
+}
+
+// The six scoring entry points with a doc filter (filter_bits / filter_rows / filter_ld after doc_id_base): the same
+// pass, in which a doc whose bit is clear never enters a candidate list.  No reference counterpart (DESIGN §4.5).
+int mfar_score_topk_filtered(const void* corpus, int64_t n_docs, int corpus_fields, int field_begin, int n_dense,
+                             int dim, const void* q_vecs, int Q, const float* w, const void* sparse, int n_sparse,
+                             int sparse_dtype, int64_t sparse_ld, int64_t doc_id_base, const uint32_t* filter_bits,
+                             int filter_rows, int64_t filter_ld, int k, uint64_t* out_keys, float* out_scores,
+                             int64_t* out_ids, void* workspace, size_t workspace_bytes, int impl, void* stream) {
+  return score_topk_core(dense_operands(MFAR_BF16, corpus, nullptr, q_vecs, nullptr), n_docs, corpus_fields,
+                         field_begin, n_dense, dim, Q, w, rows_input(sparse, n_sparse, sparse_dtype, sparse_ld),
+                         doc_id_base, k, out_keys, out_scores, out_ids, workspace, workspace_bytes, impl, stream,
+                         filter_input(filter_bits, filter_rows, filter_ld));
+}
+
+int mfar_score_topk_e4m3_filtered(const void* corpus, const float* corpus_scales, int64_t n_docs, int corpus_fields,
+                                  int field_begin, int n_dense, int dim, const void* q_vecs, const float* q_scales,
+                                  int Q, const float* w, const void* sparse, int n_sparse, int sparse_dtype,
+                                  int64_t sparse_ld, int64_t doc_id_base, const uint32_t* filter_bits,
+                                  int filter_rows, int64_t filter_ld, int k, uint64_t* out_keys, float* out_scores,
+                                  int64_t* out_ids, void* workspace, size_t workspace_bytes, int impl, void* stream) {
+  return score_topk_core(dense_operands(MFAR_E4M3, corpus, corpus_scales, q_vecs, q_scales), n_docs, corpus_fields,
+                         field_begin, n_dense, dim, Q, w, rows_input(sparse, n_sparse, sparse_dtype, sparse_ld),
+                         doc_id_base, k, out_keys, out_scores, out_ids, workspace, workspace_bytes, impl, stream,
+                         filter_input(filter_bits, filter_rows, filter_ld));
+}
+
+int mfar_score_topk_coo_filtered(const void* corpus, int64_t n_docs, int corpus_fields, int field_begin, int n_dense,
+                                 int dim, const void* q_vecs, int Q, const float* w, const int32_t* coo_keys,
+                                 const void* coo_vals, int coo_dtype, const int64_t* field_offsets_host, int n_sparse,
+                                 int64_t doc_id_base, const uint32_t* filter_bits, int filter_rows, int64_t filter_ld,
+                                 int k, uint64_t* out_keys, float* out_scores, int64_t* out_ids, void* workspace,
+                                 size_t workspace_bytes, int impl, void* stream) {
+  return score_topk_core(dense_operands(MFAR_BF16, corpus, nullptr, q_vecs, nullptr), n_docs, corpus_fields,
+                         field_begin, n_dense, dim, Q, w,
+                         coo_input(coo_keys, coo_vals, coo_dtype, field_offsets_host, n_sparse), doc_id_base, k,
+                         out_keys, out_scores, out_ids, workspace, workspace_bytes, impl, stream,
+                         filter_input(filter_bits, filter_rows, filter_ld));
+}
+
+int mfar_score_topk_coo_e4m3_filtered(const void* corpus, const float* corpus_scales, int64_t n_docs,
+                                      int corpus_fields, int field_begin, int n_dense, int dim, const void* q_vecs,
+                                      const float* q_scales, int Q, const float* w, const int32_t* coo_keys,
+                                      const void* coo_vals, int coo_dtype, const int64_t* field_offsets_host,
+                                      int n_sparse, int64_t doc_id_base, const uint32_t* filter_bits, int filter_rows,
+                                      int64_t filter_ld, int k, uint64_t* out_keys, float* out_scores,
+                                      int64_t* out_ids, void* workspace, size_t workspace_bytes, int impl,
+                                      void* stream) {
+  return score_topk_core(dense_operands(MFAR_E4M3, corpus, corpus_scales, q_vecs, q_scales), n_docs, corpus_fields,
+                         field_begin, n_dense, dim, Q, w,
+                         coo_input(coo_keys, coo_vals, coo_dtype, field_offsets_host, n_sparse), doc_id_base, k,
+                         out_keys, out_scores, out_ids, workspace, workspace_bytes, impl, stream,
+                         filter_input(filter_bits, filter_rows, filter_ld));
+}
+
+int mfar_score_topk_bm25_filtered(const void* corpus, int64_t n_docs, int corpus_fields, int field_begin,
+                                  int n_dense, int dim, const void* q_vecs, int Q, const float* w,
+                                  const void* const* indptr_host, const void* const* indices_host,
+                                  const void* const* data_host, const int32_t* vocab_host, int n_sparse,
+                                  const int32_t* entries, int64_t n_entries, int64_t doc_id_base,
+                                  const uint32_t* filter_bits, int filter_rows, int64_t filter_ld, int k,
+                                  uint64_t* out_keys, float* out_scores, int64_t* out_ids, void* workspace,
+                                  size_t workspace_bytes, int impl, void* stream) {
+  return score_topk_core(dense_operands(MFAR_BF16, corpus, nullptr, q_vecs, nullptr), n_docs, corpus_fields,
+                         field_begin, n_dense, dim, Q, w,
+                         bm25_input(indptr_host, indices_host, data_host, vocab_host, n_sparse, entries, n_entries),
+                         doc_id_base, k, out_keys, out_scores, out_ids, workspace, workspace_bytes, impl, stream,
+                         filter_input(filter_bits, filter_rows, filter_ld));
+}
+
+int mfar_score_topk_bm25_e4m3_filtered(const void* corpus, const float* corpus_scales, int64_t n_docs,
+                                       int corpus_fields, int field_begin, int n_dense, int dim, const void* q_vecs,
+                                       const float* q_scales, int Q, const float* w, const void* const* indptr_host,
+                                       const void* const* indices_host, const void* const* data_host,
+                                       const int32_t* vocab_host, int n_sparse, const int32_t* entries,
+                                       int64_t n_entries, int64_t doc_id_base, const uint32_t* filter_bits,
+                                       int filter_rows, int64_t filter_ld, int k, uint64_t* out_keys,
+                                       float* out_scores, int64_t* out_ids, void* workspace, size_t workspace_bytes,
+                                       int impl, void* stream) {
+  return score_topk_core(dense_operands(MFAR_E4M3, corpus, corpus_scales, q_vecs, q_scales), n_docs, corpus_fields,
+                         field_begin, n_dense, dim, Q, w,
+                         bm25_input(indptr_host, indices_host, data_host, vocab_host, n_sparse, entries, n_entries),
+                         doc_id_base, k, out_keys, out_scores, out_ids, workspace, workspace_bytes, impl, stream,
+                         filter_input(filter_bits, filter_rows, filter_ld));
 }
 
 int mfar_topk_merge(const uint64_t* keys, int L, int Q, int k_in, int k, uint64_t* out_keys, float* out_scores,

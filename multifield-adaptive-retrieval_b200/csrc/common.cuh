@@ -89,6 +89,25 @@ __device__ __forceinline__ float fmax_nan(float a, float b) {
   return d;
 }
 
+// Doc filter of the *_filtered entry points (DESIGN §4.5): a uint32 bitmap over GLOBAL doc ids, bit d of word d >> 5
+// set <=> doc d may enter the top-k.  One row shared by every query (stride 0) or one row of `ld` words per query
+// (stride == ld).  Only the first `words` = ceil((doc_id_base + n_docs) / 32) words of a row hold docs of the shard
+// (<= 2^27, and <= ld): a word index past them reads as 0, so tile tails never read past the row.
+struct DocFilter {
+  const uint32_t* bits;   // nullptr: no filter
+  long long stride;       // words between the rows of consecutive queries: 0 (one shared row) or ld
+  int words;              // words of a row that are read
+};
+__device__ __forceinline__ uint32_t filter_ld_word(const uint32_t* row, int words, long long w) {
+  return w < words ? __ldg(row + w) : 0u;
+}
+// bits [b, b + 32) of a row: bit j of the result is the eligibility of global doc b + j (funnel shift across words)
+__device__ __forceinline__ uint32_t filter_bits32(const uint32_t* row, int words, long long b) {
+  const long long w = b >> 5;
+  const uint32_t lo = filter_ld_word(row, words, w), hi = filter_ld_word(row, words, w + 1);
+  return __funnelshift_r(lo, hi, uint32_t(b & 31));
+}
+
 // Workspace carve-up shared by the scoring kernels and the merge.
 //   cand_keys [G][Qp][kCandCap] u64 | cand_thr [G][Qp] u64 | cand_cnt [G][Qp] i32 | err flag (256 B) |
 //   progress counters (kProgressInts i32) | gthr [Qp] u64 | pool [G][Qp] u64

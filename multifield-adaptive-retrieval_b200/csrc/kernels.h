@@ -110,6 +110,11 @@ struct ScoreArgs {
   // optional per-query admission thresholds known before the pass starts (packed keys, [Q], 0 = none): copied into the
   // workspace's shared threshold words right after they are zeroed (score_topk_core's prefix pass)
   const unsigned long long* gthr_seed;
+  // optional doc filter (bitmap over GLOBAL doc ids, common.cuh): indexed by doc_id_base + local doc, so moving
+  // doc_id_base past a scored prefix (skip_tiles) moves the filter with it
+  const uint32_t* filter_bits;   // nullptr: every doc is eligible
+  int64_t filter_stride;         // words between the rows of consecutive queries: 0 (one shared row) or the row length
+  int filter_words;              // ceil((doc_id_base + n_docs) / 32): the words of a row that hold docs of the shard
 };
 
 // gthr[q] = seed[q] (after the launcher zeroed the workspace tail)

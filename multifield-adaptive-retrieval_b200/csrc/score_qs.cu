@@ -68,6 +68,7 @@ struct QsParams {
   int stages;          // ring depth
   int kc_per_stage;    // 64-element K chunks per stage (divides k_chunks)
   TopkWorkspace ws;
+  DocFilter filt;      // FILT only
 };
 
 // Issue the 4*KC MMAs of one shared-memory stage (KC K-major [rows x 64] blocks) into accumulator d_tmem.
@@ -189,7 +190,10 @@ __device__ unsigned long long g_qs_cluster4_ctas;
 // SP: the epilogue gathers the sparse fields itself (qs_seed_sparse) - a separate instantiation, so the dense-only
 // kernels keep their register allocation.  map_bh: the corpus view of map_b with half its K chunks per box (the
 // multicast loads of a 4-CTA cluster).
-template <int CG, int ES, bool SP>
+// FILT: doc filter.  A thread owns a query over a half-tile of 64 docs: its 64-bit window of the query's row (3 words
+// and a funnel shift at bit doc_id_base + doc0) is loaded at the head of the half-tile and tested next to the key
+// compare.
+template <int CG, int ES, bool SP, bool FILT>
 __global__ void __launch_bounds__(qs_threads(ES, SP), 1)
 score_qs_kernel(const __grid_constant__ CUtensorMap map_b, const __grid_constant__ CUtensorMap map_bh,
                 const __grid_constant__ CUtensorMap map_sp, QsParams p) {
@@ -516,6 +520,13 @@ score_qs_kernel(const __grid_constant__ CUtensorMap map_b, const __grid_constant
         const bool refresh = q_valid && ((n_push++ & refresh_mask) == 0);
         unsigned long long gt_new = 0ull;
         if (refresh) gt_new = ld_relaxed_u64(p.ws.gthr + qrow);
+        uint32_t fx[3] = {0u, 0u, 0u};               // FILT: words of docs doc0 .. doc0 + 63 (padding queries: none)
+        if (FILT && q_valid && doc0 < p.n_docs) {
+          const uint32_t* frow = p.filt.bits + int64_t(qrow) * p.filt.stride;
+          const int64_t w0 = (p.doc_id_base + doc0) >> 5;
+#pragma unroll
+          for (int j = 0; j < 3; ++j) fx[j] = filter_ld_word(frow, p.filt.words, w0 + j);
+        }
         int sp_e = 0;                                // next sparse element of this half-tile to consume
         if (sp_live) {
 #pragma unroll
@@ -569,6 +580,9 @@ score_qs_kernel(const __grid_constant__ CUtensorMap map_b, const __grid_constant
           // one float compare per doc rejects almost everything; the exact (score, id) key is only built for docs
           // whose score reaches the threshold's score (thr == 0: nothing established yet, admit all)
           const float thr_f = thr ? key_score(thr) : -INFINITY;
+          const uint32_t fsh = uint32_t((p.doc_id_base + doc0) & 31);
+          const uint64_t fwin =                                     // FILT: bit c <=> doc doc0 + c is eligible
+              FILT ? (uint64_t(__funnelshift_r(fx[1], fx[2], fsh)) << 32) | __funnelshift_r(fx[0], fx[1], fsh) : 0ull;
           // ... and one compare per GROUP of 8 docs (max tree: 3 FMNMX/FMNMX3 + 1 FSETP instead of 8 FSETP + 8
           // branches) rejects almost every group once a threshold exists - with a single_ scorer this push phase runs
           // after every MMA unit.  (A branch-free 64-bit pass mask was measured too: its 3 instructions per doc cost
@@ -583,7 +597,7 @@ score_qs_kernel(const __grid_constant__ CUtensorMap map_b, const __grid_constant
               for (int c = c0; c < c0 + 8; ++c) {
                 if (c < nd && !(acc[c] < thr_f)) {
                   const uint64_t key = make_key(acc[c], id0 + c);
-                  if (key > thr) { __stcg(my_list + cnt, key); ++cnt; }
+                  if (key > thr && (!FILT || ((fwin >> c) & 1ull))) { __stcg(my_list + cnt, key); ++cnt; }
                 }
               }
             }
@@ -650,7 +664,7 @@ static size_t qs_smem_bytes(int n_weights, int stages, int stage_bytes, int sp_s
 // Q <= 128 the kernel is HBM-bound and the extra warps measured ~3 % slower
 int score_qs_lists_per_worker(int n_dense, int cg) { return (n_dense == 1 && cg == 2) ? 2 : 1; }
 
-template <int CG, int ES, bool SP>
+template <int CG, int ES, bool SP, bool FILT>
 static int launch_qs_impl(const ScoreArgs& a, void* ws_base, int workers, int q_tiles, cudaStream_t st) {
   constexpr int kChunkBytes = (kQsDocs / CG) * kChunkK * 2;
   QsParams p;
@@ -663,6 +677,7 @@ static int launch_qs_impl(const ScoreArgs& a, void* ws_base, int workers, int q_
   if (a.sparse && (a.base || !sparse_rows_fusable(a.sparse, a.sparse_dtype, a.sparse_ld))) return MFAR_ERR_ARG;
   const int n_w = a.n_dense + p.n_sparse;
   p.ws = carve_workspace(ws_base, workers * ES, q_tiles * kQsQ);   // ES candidate lists per (CTA, query)
+  p.filt = DocFilter{a.filter_bits, a.filter_stride, a.filter_words};
   const size_t smem_cap = 227 * 1024;
   // Shared memory: corpus ring + (SP) sparse ring of 16 KB slots + weights + barriers.  The corpus ring is split in two
   // halves, one per MMA-issuing warp (see the producer), so `stages` is even.  Dense-only: stages of up to 48 KB, 192 KB
@@ -716,7 +731,7 @@ static int launch_qs_impl(const ScoreArgs& a, void* ws_base, int workers, int q_
   }
   static PerDeviceOnce attr_once;   // per template instantiation
   MFAR_CUDA_OK(attr_once.run([&] {
-    return cudaFuncSetAttribute(score_qs_kernel<CG, ES, SP>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem_cap));
+    return cudaFuncSetAttribute(score_qs_kernel<CG, ES, SP, FILT>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem_cap));
   }));
   // lockstep counters of the query groups (producer warp) + shared per-query thresholds (epilogue)
   MFAR_CUDA_OK(cudaMemsetAsync(p.ws.progress, 0, workspace_zero_bytes(p.ws.workers, p.ws.q_pad), st));
@@ -733,7 +748,7 @@ static int launch_qs_impl(const ScoreArgs& a, void* ws_base, int workers, int q_
   attr[1].val.preferredClusterDim.x = 4; attr[1].val.preferredClusterDim.y = 1; attr[1].val.preferredClusterDim.z = 1;
   cfg.attrs = attr;
   cfg.numAttrs = cluster4 ? 2 : 1;
-  MFAR_CUDA_OK(cudaLaunchKernelEx(&cfg, score_qs_kernel<CG, ES, SP>, map_b, map_bh, map_sp, p));
+  MFAR_CUDA_OK(cudaLaunchKernelEx(&cfg, score_qs_kernel<CG, ES, SP, FILT>, map_b, map_bh, map_sp, p));
   return MFAR_OK;
 }
 
@@ -746,17 +761,23 @@ long long qs_cluster4_ctas_collect() {
   return static_cast<long long>(n);
 }
 
-int launch_score_qs(const ScoreArgs& a, void* ws_base, int workers, int q_tiles, int cg, cudaStream_t st) {
-  if (!score_qs_supported(a)) return MFAR_ERR_SHAPE;
+template <bool FILT>
+static int launch_qs_filt(const ScoreArgs& a, void* ws_base, int workers, int q_tiles, int cg, cudaStream_t st) {
   const bool sp = a.sparse != nullptr;
   if (score_qs_lists_per_worker(a.n_dense, cg) == 2)
-    return sp ? launch_qs_impl<2, 2, true>(a, ws_base, workers, q_tiles, st)
-              : launch_qs_impl<2, 2, false>(a, ws_base, workers, q_tiles, st);
+    return sp ? launch_qs_impl<2, 2, true, FILT>(a, ws_base, workers, q_tiles, st)
+              : launch_qs_impl<2, 2, false, FILT>(a, ws_base, workers, q_tiles, st);
   if (cg == 2)
-    return sp ? launch_qs_impl<2, 1, true>(a, ws_base, workers, q_tiles, st)
-              : launch_qs_impl<2, 1, false>(a, ws_base, workers, q_tiles, st);
-  return sp ? launch_qs_impl<1, 1, true>(a, ws_base, workers, q_tiles, st)
-            : launch_qs_impl<1, 1, false>(a, ws_base, workers, q_tiles, st);
+    return sp ? launch_qs_impl<2, 1, true, FILT>(a, ws_base, workers, q_tiles, st)
+              : launch_qs_impl<2, 1, false, FILT>(a, ws_base, workers, q_tiles, st);
+  return sp ? launch_qs_impl<1, 1, true, FILT>(a, ws_base, workers, q_tiles, st)
+            : launch_qs_impl<1, 1, false, FILT>(a, ws_base, workers, q_tiles, st);
+}
+
+int launch_score_qs(const ScoreArgs& a, void* ws_base, int workers, int q_tiles, int cg, cudaStream_t st) {
+  if (!score_qs_supported(a)) return MFAR_ERR_SHAPE;
+  return a.filter_bits ? launch_qs_filt<true>(a, ws_base, workers, q_tiles, cg, st)
+                       : launch_qs_filt<false>(a, ws_base, workers, q_tiles, cg, st);
 }
 
 }  // namespace mfar

@@ -34,6 +34,7 @@ struct SimtParams {
   int64_t doc_id_base;
   int k;
   TopkWorkspace ws;
+  DocFilter filt;               // FILT only
 };
 
 __device__ __forceinline__ void bf16x8_to_f32(const uint4& v, float (&f)[8]) {
@@ -51,7 +52,8 @@ __device__ __forceinline__ uint4 ld_stream(const uint4* p) {
 }
 
 // QB = queries handled per corpus pass (their slices live in registers)
-template <int QB, bool E8>
+// FILT: doc filter; the lane's filter word of each query is loaded at the tile's start and tested after the key compare
+template <int QB, bool E8, bool FILT>
 __global__ void __launch_bounds__(kSimtThreads) score_simt_kernel(SimtParams p) {
   extern __shared__ float s_w[];                      // [QB][n_dense]
   __shared__ unsigned long long s_thr[QB];
@@ -97,6 +99,13 @@ __global__ void __launch_bounds__(kSimtThreads) score_simt_kernel(SimtParams p) 
     __syncthreads();
 
     for (int t = g; t < p.n_tiles; t += gridDim.x) {
+      const int64_t fbit = p.doc_id_base + int64_t(t) * kTileDocs + warp * 32 + lane;   // global id of the lane's doc
+      uint32_t fw[QB];
+#pragma unroll
+      for (int qi = 0; qi < QB; ++qi) {
+        const uint32_t* frow = p.filt.bits + int64_t(q0 + qi) * p.filt.stride;
+        fw[qi] = (FILT && qi < nq) ? filter_ld_word(frow, p.filt.words, fbit >> 5) : 0u;
+      }
       float mine[QB];
 #pragma unroll
       for (int qi = 0; qi < QB; ++qi) mine[qi] = 0.f;
@@ -175,7 +184,7 @@ __global__ void __launch_bounds__(kSimtThreads) score_simt_kernel(SimtParams p) 
             float s = mine[qi];
             if (p.base) s += p.base[int64_t(q0 + qi) * p.base_ld + doc_local];
             const uint64_t key = make_key(s, uint32_t(p.doc_id_base + doc_local));
-            if (key > s_thr[qi]) {
+            if (key > s_thr[qi] && (!FILT || ((fw[qi] >> (fbit & 31)) & 1u))) {
               const int pos = atomicAdd(&s_cnt[qi], 1);
               __stcg(p.ws.cand_keys + (int64_t(g) * p.ws.q_pad + q0 + qi) * kCandCap + pos, key);
             }
@@ -208,14 +217,14 @@ void score_simt_geometry(int Q, int n_tiles, int* q_pad, int* workers) {
   *workers = w;
 }
 
-template <bool E8>
+template <bool E8, bool FILT>
 static void launch_simt_qb(const SimtParams& p, int Q, int n_dense, int workers, cudaStream_t st) {
   if (Q == 1) {
-    score_simt_kernel<1, E8><<<workers, kSimtThreads, 1 * n_dense * sizeof(float) + 16, st>>>(p);
+    score_simt_kernel<1, E8, FILT><<<workers, kSimtThreads, 1 * n_dense * sizeof(float) + 16, st>>>(p);
   } else if (Q == 2) {
-    score_simt_kernel<2, E8><<<workers, kSimtThreads, 2 * n_dense * sizeof(float) + 16, st>>>(p);
+    score_simt_kernel<2, E8, FILT><<<workers, kSimtThreads, 2 * n_dense * sizeof(float) + 16, st>>>(p);
   } else {
-    score_simt_kernel<4, E8><<<workers, kSimtThreads, 4 * n_dense * sizeof(float) + 16, st>>>(p);
+    score_simt_kernel<4, E8, FILT><<<workers, kSimtThreads, 4 * n_dense * sizeof(float) + 16, st>>>(p);
   }
 }
 
@@ -231,8 +240,11 @@ int launch_score_simt(const ScoreArgs& a, void* ws_base, int workers, int q_pad,
   p.n_dense = a.n_dense; p.dim = a.dim; p.q_vecs = a.q_vecs; p.Q = a.Q;
   p.w = a.w; p.w_ld = a.w_ld; p.base = a.base; p.base_ld = a.base_ld; p.doc_id_base = a.doc_id_base; p.k = a.k;
   p.ws = carve_workspace(ws_base, workers, q_pad);
-  if (e8) launch_simt_qb<true>(p, a.Q, a.n_dense, workers, st);
-  else launch_simt_qb<false>(p, a.Q, a.n_dense, workers, st);
+  p.filt = DocFilter{a.filter_bits, a.filter_stride, a.filter_words};
+  const bool f = a.filter_bits != nullptr;
+  auto launch = e8 ? (f ? launch_simt_qb<true, true> : launch_simt_qb<true, false>)
+                   : (f ? launch_simt_qb<false, true> : launch_simt_qb<false, false>);
+  launch(p, a.Q, a.n_dense, workers, st);
   MFAR_CUDA_OK(cudaGetLastError());
   return MFAR_OK;
 }

@@ -51,6 +51,7 @@ struct TcParams {
   int k;
   int stages;
   TopkWorkspace ws;
+  DocFilter filt;               // FILT only
 };
 
 // Sparse term of one corpus tile for the CTA's QP queries, gathered from the per-field score rows (index.py:111-118)
@@ -142,11 +143,14 @@ __device__ __forceinline__ void tc_stage_sparse(float* base_s, const TcParams& p
 // E8: E4M3 corpus and queries.  A K-chunk is still one 128-byte swizzled row span (128 elements instead of 64), so the
 // ring, the descriptors and the producer are those of bf16; the MMA is kind::f8f6f4 (K = 32), and the epilogue applies
 // the query scale (shared memory) and the doc's row scale (one coalesced 512-byte load per (tile, field)) to D_f.
-template <int QP, bool SP, bool E8>   // SP: sparse fields gathered in-kernel (tc_stage_sparse, 2 more warps)
+// FILT: doc filter.  A thread owns a doc and tests QP queries' bits for it, so the tile's words of every query are
+// staged in shared memory (s_filt, one tile ahead) and a pushed pair reads one of them next to the key compare.
+template <int QP, bool SP, bool E8, bool FILT>   // SP: sparse fields gathered in-kernel (tc_stage_sparse, 2 more warps)
 __global__ void __launch_bounds__(SP ? kTcThreads + kStagerThreads : kTcThreads, 1)
 score_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ CUtensorMap map_b, TcParams p) {
   extern __shared__ __align__(1024) uint8_t smem_raw[];
-  // carve: [A stages][B resident][w_s][s_q (E8)][thr as float][thr][cnt][flags][barriers][tmem ptr]
+  // carve: [A stages][B resident][w_s][s_q (E8)][thr as float][thr][cnt][flags][base_s (SP)][s_filt (FILT)][barriers]
+  // [tmem ptr]
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
   uint8_t* smem_a = smem;
   uint8_t* smem_b = smem_a + size_t(p.stages) * kABytes;
@@ -160,8 +164,10 @@ score_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant
   int* s_cnt = reinterpret_cast<int*>(s_thr + QP);
   int* s_flags = s_cnt + QP;                       // reserved (keeps the shared-memory layout)
   float* base_s = reinterpret_cast<float*>((reinterpret_cast<uintptr_t>(s_flags + QP) + 15) & ~uintptr_t(15));   // [QP][128]
+  constexpr int kFiltWords = QP * (kTileDocs / 32);   // one tile's filter words: [QP queries][4 x 32 docs]
+  uint32_t* s_filt = reinterpret_cast<uint32_t*>(base_s + (SP ? QP * kTileDocs : 0));   // [2][kFiltWords]
   uint64_t* bars = reinterpret_cast<uint64_t*>(
-      (reinterpret_cast<uintptr_t>(base_s + (SP ? QP * kTileDocs : 0)) + 7) & ~uintptr_t(7));
+      (reinterpret_cast<uintptr_t>(s_filt + (FILT ? 2 * kFiltWords : 0)) + 7) & ~uintptr_t(7));
   uint64_t* full_bar = bars;                       // [stages]
   uint64_t* empty_bar = bars + p.stages;           // [stages]
   uint64_t* tfull_bar = bars + 2 * p.stages;       // [2]
@@ -290,6 +296,29 @@ score_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant
       const unsigned long long gt = ld_relaxed_u64(p.ws.gthr + q0 + cq);
       if (gt > s_thr[cq]) { s_thr[cq] = gt; s_thrf[cq] = key_score(gt); }
     }
+    // FILT: s_filt[b][c * 4 + w] = bits of docs 32w .. 32w + 31 of a tile for query c (0 for padding queries).  Tile
+    // i + 1's words are loaded at the head of tile i and stored after its last accumulator drain into buffer (i + 1) & 1;
+    // tile i's push reads buffer i & 1.  The block barriers that end tile i order those stores before tile i + 1's
+    // reads, and tile i - 1's reads of the same buffer before them.
+    constexpr int kFiltPer = (kFiltWords + kEpiThreads - 1) / kEpiThreads;
+    const int fe0 = int(threadIdx.x) - 64;           // epilogue thread index 0 .. 127
+    uint32_t fnext[kFiltPer];
+    auto filt_load = [&](int tile) {
+#pragma unroll
+      for (int j = 0; j < kFiltPer; ++j) {
+        const int e = fe0 + j * kEpiThreads, c = e >> 2;
+        fnext[j] = (e < kFiltWords && c < nq)
+                       ? filter_bits32(p.filt.bits + int64_t(q0 + c) * p.filt.stride, p.filt.words,
+                                       p.doc_id_base + int64_t(tile) * kTileDocs + (e & 3) * 32)
+                       : 0u;
+      }
+    };
+    auto filt_store = [&](int b) {
+#pragma unroll
+      for (int j = 0; j < kFiltPer; ++j)
+        if (fe0 + j * kEpiThreads < kFiltWords) s_filt[b * kFiltWords + fe0 + j * kEpiThreads] = fnext[j];
+    };
+    if (FILT && my_tiles > 0) { filt_load(g); filt_store(0); }
     epi_bar_sync();
     for (int i = 0; i < my_tiles; ++i) {
       const int t = g + i * gridDim.x;
@@ -302,6 +331,7 @@ score_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant
       // round of compactions, so the value is applied BEFORE this tile's pushes (one more block barrier, nothing next
       // to a 100 us tile); short tiles apply it after the pushes, for the next tile.
       const bool adopt_before_push = p.n_dense >= 8 || my_tiles <= 32;
+      if (FILT && i + 1 < my_tiles) filt_load(t + int(gridDim.x));   // consumed after the field loop
       // The accumulators start from the pre-mixed sparse term: its QP loads per doc (coalesced across the warp's
       // 32 docs) are issued here, ahead of the wait for the tile's first accumulator, instead of serialising with
       // the push loop after the last field.
@@ -351,12 +381,14 @@ score_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant
         mbar_arrive(&tempty_bar[buf]);             // 128 arrivals free the accumulator buffer
       }
       // ---- tile done: filter, push
+      if (FILT && i + 1 < my_tiles) filt_store((i + 1) & 1);
       if (adopt_before_push) {
         if (cq_live && gt_next > s_thr[cq]) { s_thr[cq] = gt_next; s_thrf[cq] = key_score(gt_next); }
         epi_bar_sync();
       }
       if (doc_local < p.n_docs) {
         const uint32_t doc_id = uint32_t(p.doc_id_base + doc_local);
+        const uint32_t* fw = s_filt + (i & 1) * kFiltWords + lane_grp;   // FILT: word c * 4 holds this warp's 32 docs
         // Float pre-filter per GROUP of 8 queries: max_j(score[c0+j] - score of query c0+j's threshold) >= 0 decides
         // with 8 FADD + 3 FMNMX3/FMNMX + 1 FSETP + 1 branch whether any of the 8 (doc, query) pairs can be admitted;
         // the exact (score, id) key is only built inside live groups.  With one epilogue warp per scheduler every
@@ -375,7 +407,7 @@ score_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant
             for (int j = 0; j < 8; ++j) {
               const int c = c0 + j;
               const uint64_t key = make_key(acc[c], doc_id);
-              if (key > s_thr[c] && c < nq) {
+              if (key > s_thr[c] && c < nq && (!FILT || ((fw[c * 4] >> lane) & 1u))) {
                 const int pos = atomicAdd(&s_cnt[c], 1);
                 __stcg(p.ws.cand_keys + (int64_t(g) * p.ws.q_pad + q0 + c) * kCandCap + pos, key);
               }
@@ -443,13 +475,14 @@ void score_tc_geometry(int Q, int n_tiles, int* q_pad, int* q_tiles, int* worker
   *q_pad = qp; *q_tiles = qt; *workers = w;
 }
 
-// n_weights: rows of [QP] floats next to the weights (E8: + the query scales)
-static size_t tc_smem_bytes(int qp, int n_weights, bool sparse, int k_chunks, int stages) {
+// n_weights: rows of [QP] floats next to the weights (E8: + the query scales); filt: two tiles of filter words
+static size_t tc_smem_bytes(int qp, int n_weights, bool sparse, int k_chunks, int stages, bool filt) {
   return 1024 + size_t(stages) * kABytes + size_t(k_chunks) * qp * 128 + size_t(n_weights) * qp * 4 +
-         size_t(qp) * 20 + 16 + (sparse ? size_t(qp) * kTileDocs * 4 : 0) + 8 + (2 * stages + 7) * 8 + 16;
+         size_t(qp) * 20 + 16 + (sparse ? size_t(qp) * kTileDocs * 4 : 0) + (filt ? size_t(qp) * kTileDocs / 4 : 0) + 8 +
+         (2 * stages + 7) * 8 + 16;
 }
 
-template <int QP, bool SP, bool E8>
+template <int QP, bool SP, bool E8, bool FILT>
 static int launch_tc_impl(const ScoreArgs& a, void* ws_base, int workers, int q_tiles, cudaStream_t st) {
   TcParams p;
   p.n_docs = a.n_docs; p.n_tiles = a.n_tiles; p.corpus_fields = a.corpus_fields; p.field_begin = a.field_begin;
@@ -462,12 +495,13 @@ static int launch_tc_impl(const ScoreArgs& a, void* ws_base, int workers, int q_
   if (a.sparse && (a.base || !sparse_rows_fusable(a.sparse, a.sparse_dtype, a.sparse_ld))) return MFAR_ERR_ARG;
   const int n_w = a.n_dense + p.n_sparse + (E8 ? 1 : 0);
   p.ws = carve_workspace(ws_base, workers, q_tiles * QP);
+  p.filt = DocFilter{a.filter_bits, a.filter_stride, a.filter_words};
   int stages = 8;
   const size_t smem_cap = 227 * 1024;
-  while (stages > 2 && tc_smem_bytes(QP, n_w, a.sparse != nullptr, p.k_chunks, stages) > smem_cap) --stages;
-  if (tc_smem_bytes(QP, n_w, a.sparse != nullptr, p.k_chunks, stages) > smem_cap) return MFAR_ERR_SHAPE;
+  while (stages > 2 && tc_smem_bytes(QP, n_w, a.sparse != nullptr, p.k_chunks, stages, FILT) > smem_cap) --stages;
+  if (tc_smem_bytes(QP, n_w, a.sparse != nullptr, p.k_chunks, stages, FILT) > smem_cap) return MFAR_ERR_SHAPE;
   p.stages = stages;
-  const size_t smem = tc_smem_bytes(QP, n_w, a.sparse != nullptr, p.k_chunks, stages);
+  const size_t smem = tc_smem_bytes(QP, n_w, a.sparse != nullptr, p.k_chunks, stages, FILT);
 
   CUtensorMap map_a, map_b;
   int rc = make_tensor_map_2d(&map_a, a.corpus, uint64_t(a.n_tiles) * a.corpus_fields * kTileDocs, a.dim, kTileDocs,
@@ -478,25 +512,25 @@ static int launch_tc_impl(const ScoreArgs& a, void* ws_base, int workers, int q_
 
   static PerDeviceOnce attr_once;   // per template instantiation
   MFAR_CUDA_OK(attr_once.run([&] {
-    return cudaFuncSetAttribute(score_tc_kernel<QP, SP, E8>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem_cap));
+    return cudaFuncSetAttribute(score_tc_kernel<QP, SP, E8, FILT>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem_cap));
   }));
   MFAR_CUDA_OK(cudaMemsetAsync(p.ws.progress, 0, workspace_zero_bytes(p.ws.workers, p.ws.q_pad), st));   // shared thresholds
   if (a.gthr_seed) { if (int rc2 = launch_seed_gthr(p.ws.gthr, a.gthr_seed, a.Q, st)) return rc2; }
   dim3 grid(workers, q_tiles);
-  score_tc_kernel<QP, SP, E8><<<grid, SP ? kTcThreads + kStagerThreads : kTcThreads, smem, st>>>(map_a, map_b, p);
+  score_tc_kernel<QP, SP, E8, FILT><<<grid, SP ? kTcThreads + kStagerThreads : kTcThreads, smem, st>>>(map_a, map_b, p);
   MFAR_CUDA_OK(cudaGetLastError());
   return MFAR_OK;
 }
 
-template <bool E8>
+template <bool E8, bool FILT>
 static int launch_tc_qp(const ScoreArgs& a, void* ws_base, int workers, int q_tiles, int q_pad, cudaStream_t st) {
   switch (q_pad) {
-    case 16: return a.sparse ? launch_tc_impl<16, true, E8>(a, ws_base, workers, q_tiles, st)
-                             : launch_tc_impl<16, false, E8>(a, ws_base, workers, q_tiles, st);
-    case 32: return a.sparse ? launch_tc_impl<32, true, E8>(a, ws_base, workers, q_tiles, st)
-                             : launch_tc_impl<32, false, E8>(a, ws_base, workers, q_tiles, st);
-    case 64: return a.sparse ? launch_tc_impl<64, true, E8>(a, ws_base, workers, q_tiles, st)
-                             : launch_tc_impl<64, false, E8>(a, ws_base, workers, q_tiles, st);
+    case 16: return a.sparse ? launch_tc_impl<16, true, E8, FILT>(a, ws_base, workers, q_tiles, st)
+                             : launch_tc_impl<16, false, E8, FILT>(a, ws_base, workers, q_tiles, st);
+    case 32: return a.sparse ? launch_tc_impl<32, true, E8, FILT>(a, ws_base, workers, q_tiles, st)
+                             : launch_tc_impl<32, false, E8, FILT>(a, ws_base, workers, q_tiles, st);
+    case 64: return a.sparse ? launch_tc_impl<64, true, E8, FILT>(a, ws_base, workers, q_tiles, st)
+                             : launch_tc_impl<64, false, E8, FILT>(a, ws_base, workers, q_tiles, st);
     default: return MFAR_ERR_SHAPE;
   }
 }
@@ -505,9 +539,11 @@ int launch_score_tc(const ScoreArgs& a, void* ws_base, int workers, int q_tiles,
   if (!score_tc_supported(a)) return MFAR_ERR_SHAPE;
   if (a.corpus_dtype == MFAR_E4M3) {
     if (!a.corpus_scales || !a.q_scales) return MFAR_ERR_ARG;
-    return launch_tc_qp<true>(a, ws_base, workers, q_tiles, q_pad, st);
+    return a.filter_bits ? launch_tc_qp<true, true>(a, ws_base, workers, q_tiles, q_pad, st)
+                         : launch_tc_qp<true, false>(a, ws_base, workers, q_tiles, q_pad, st);
   }
-  return launch_tc_qp<false>(a, ws_base, workers, q_tiles, q_pad, st);
+  return a.filter_bits ? launch_tc_qp<false, true>(a, ws_base, workers, q_tiles, q_pad, st)
+                       : launch_tc_qp<false, false>(a, ws_base, workers, q_tiles, q_pad, st);
 }
 
 }  // namespace mfar

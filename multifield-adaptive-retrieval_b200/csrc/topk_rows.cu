@@ -27,30 +27,36 @@ constexpr int kRowsStepDocs = 512;     // docs per warp step: 4 float4 per lane
 constexpr int kSeedThreads = 256;
 constexpr int kSeedPerThread = 32;     // float4 subsets per thread: prefix = 256 * 32 * 4 = 32768 docs
 
+// FILT: ineligible docs count as absent (-inf) in their subset's maximum, so every maximum above -inf is still an
+// eligible doc and the bound stays one that k eligible docs reach.
+template <bool FILT>
 __global__ void __launch_bounds__(kSeedThreads)
 topk_rows_seed_kernel(const float* __restrict__ base, long long base_ld, long long n_docs, int k,
-                      unsigned long long* __restrict__ gthr) {
+                      unsigned long long* __restrict__ gthr, long long doc_id_base, DocFilter filt) {
   __shared__ int part[kSeedThreads / 32];
   __shared__ int total_s;
   const int q = blockIdx.x, tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
   const float* row = base + (long long)q * base_ld;
+  const uint32_t* frow = FILT ? filt.bits + (long long)q * filt.stride : nullptr;
   uint32_t hi[kSeedPerThread];
   const long long last_vec = ((n_docs - 1) / 4) * 4;       // base_ld is a multiple of 128: this 16-byte read is in bounds
 #pragma unroll
   for (int i0 = 0; i0 < kSeedPerThread; i0 += 8) {         // 8 unconditional loads in flight, then the masking
     float4 v[8];
+    uint32_t fb[8];                                        // FILT: eligibility of the subset's 4 docs (bits 0..3)
 #pragma unroll
     for (int j = 0; j < 8; ++j) {
       const long long d = ((long long)(i0 + j) * kSeedThreads + tid) * 4;
       v[j] = __ldg(reinterpret_cast<const float4*>(row + (d < n_docs ? d : last_vec)));
+      fb[j] = FILT ? filter_bits32(frow, filt.words, doc_id_base + d) : 0xFu;
     }
 #pragma unroll
     for (int j = 0; j < 8; ++j) {
       const long long d = ((long long)(i0 + j) * kSeedThreads + tid) * 4;
-      float m = d < n_docs ? v[j].x : -INFINITY;
-      m = d + 1 < n_docs ? fmaxf(m, v[j].y) : m;
-      m = d + 2 < n_docs ? fmaxf(m, v[j].z) : m;
-      m = d + 3 < n_docs ? fmaxf(m, v[j].w) : m;
+      float m = d < n_docs && (fb[j] & 1u) ? v[j].x : -INFINITY;
+      m = d + 1 < n_docs && (fb[j] & 2u) ? fmaxf(m, v[j].y) : m;
+      m = d + 2 < n_docs && (fb[j] & 4u) ? fmaxf(m, v[j].z) : m;
+      m = d + 3 < n_docs && (fb[j] & 8u) ? fmaxf(m, v[j].w) : m;
       hi[i0 + j] = float_to_ordered(m);
     }
   }
@@ -85,15 +91,18 @@ __device__ __forceinline__ void rows_load_step(const float* __restrict__ row, lo
   }
 }
 
+// FILT: a doc whose bit is clear is never pushed; its bits are read on the rare path, after the sub-step's ballot.
+template <bool FILT>
 __global__ void __launch_bounds__(kRowsWarps * 32, 3)
 topk_rows_kernel(const float* __restrict__ base, long long base_ld, long long n_docs, int Q, int segments,
-                 long long seg_docs, long long doc_id_base, int k, TopkWorkspace ws) {
+                 long long seg_docs, long long doc_id_base, int k, TopkWorkspace ws, DocFilter filt) {
   const int lane = threadIdx.x & 31;
   const long long task = (long long)blockIdx.x * kRowsWarps + (threadIdx.x >> 5);   // = seg * Q + q (q fastest)
   if (task >= (long long)segments * Q) return;
   const int seg = int(task / Q), q = int(task - (long long)seg * Q);
   const long long d0 = seg * seg_docs, d1 = min(n_docs, d0 + seg_docs);
   const float* row = base + (long long)q * base_ld;
+  const uint32_t* frow = FILT ? filt.bits + (long long)q * filt.stride : nullptr;
   uint64_t* list = ws.cand_keys + ((long long)seg * ws.q_pad + q) * kCandCap;
   unsigned long long thr = 0ull;
   float thr_f = -INFINITY;
@@ -115,10 +124,11 @@ topk_rows_kernel(const float* __restrict__ base, long long base_ld, long long n_
       if (__ballot_sync(0xffffffffu, !(m < thr_f)) == 0u) continue;
       const long long d = s0 + j * 128 + lane * 4;
       const float x[4] = {cur[j].x, cur[j].y, cur[j].z, cur[j].w};
+      const uint32_t fb = FILT ? filter_bits32(frow, filt.words, doc_id_base + d) : 0xFu;
 #pragma unroll
       for (int e = 0; e < 4; ++e) {
         const unsigned long long key = make_key(x[e], uint32_t(doc_id_base + d + e));
-        const bool pass = (d + e < d1) && !(x[e] < thr_f) && key > thr;
+        const bool pass = (d + e < d1) && !(x[e] < thr_f) && key > thr && ((fb >> e) & 1u);
         const unsigned b = __ballot_sync(0xffffffffu, pass);
         if (b) {
           if (pass) __stcg(list + cnt + __popc(b & lt_mask), key);
@@ -164,12 +174,17 @@ int launch_topk_rows(const ScoreArgs& a, void* ws_base, int segments, long long 
   if (!a.base || a.base_ld % 4 != 0 || reinterpret_cast<uintptr_t>(a.base) % 16 != 0) return MFAR_ERR_ARG;
   TopkWorkspace ws = carve_workspace(ws_base, segments, round_up(a.Q, 4));
   MFAR_CUDA_OK(cudaMemsetAsync(ws.progress, 0, workspace_zero_bytes(ws.workers, ws.q_pad), st));   // gthr
-  if (a.n_docs >= 4096)                                    // tiny shards: a few steps per warp, nothing to seed
-    topk_rows_seed_kernel<<<a.Q, kSeedThreads, 0, st>>>(a.base, a.base_ld, a.n_docs, a.k, ws.gthr);
+  const DocFilter filt{a.filter_bits, a.filter_stride, a.filter_words};
+  const bool f = filt.bits != nullptr;
+  if (a.n_docs >= 4096) {                                  // tiny shards: a few steps per warp, nothing to seed
+    auto seed = f ? topk_rows_seed_kernel<true> : topk_rows_seed_kernel<false>;
+    seed<<<a.Q, kSeedThreads, 0, st>>>(a.base, a.base_ld, a.n_docs, a.k, ws.gthr, a.doc_id_base, filt);
+  }
   const long long tasks = (long long)segments * a.Q;
   const unsigned blocks = unsigned((tasks + kRowsWarps - 1) / kRowsWarps);
-  topk_rows_kernel<<<blocks, kRowsWarps * 32, 0, st>>>(a.base, a.base_ld, a.n_docs, a.Q, segments, seg_docs,
-                                                      a.doc_id_base, a.k, ws);
+  auto rows = f ? topk_rows_kernel<true> : topk_rows_kernel<false>;
+  rows<<<blocks, kRowsWarps * 32, 0, st>>>(a.base, a.base_ld, a.n_docs, a.Q, segments, seg_docs, a.doc_id_base, a.k,
+                                           ws, filt);
   MFAR_CUDA_OK(cudaGetLastError());
   return MFAR_OK;
 }

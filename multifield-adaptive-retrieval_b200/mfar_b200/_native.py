@@ -44,6 +44,19 @@ PROTOTYPES = {
                                       _vp, _vp, _vp, _vp, _sz, _i, _vp]),
     "mfar_score_topk_bm25_e4m3": (_i, [_vp, _vp, _i64, _i, _i, _i, _i, _vp, _vp, _i, _vp, _vp, _vp, _vp, _vp, _i, _vp,
                                        _i64, _i64, _i, _vp, _vp, _vp, _vp, _sz, _i, _vp]),
+    # *_filtered: the twin's arguments with (filter_bits, filter_rows, filter_ld) after doc_id_base
+    "mfar_score_topk_filtered": (_i, [_vp, _i64, _i, _i, _i, _i, _vp, _i, _vp, _vp, _i, _i, _i64, _i64, _vp, _i, _i64, _i,
+                                      _vp, _vp, _vp, _vp, _sz, _i, _vp]),
+    "mfar_score_topk_coo_filtered": (_i, [_vp, _i64, _i, _i, _i, _i, _vp, _i, _vp, _vp, _vp, _i, _vp, _i, _i64, _vp, _i,
+                                          _i64, _i, _vp, _vp, _vp, _vp, _sz, _i, _vp]),
+    "mfar_score_topk_bm25_filtered": (_i, [_vp, _i64, _i, _i, _i, _i, _vp, _i, _vp, _vp, _vp, _vp, _vp, _i, _vp, _i64,
+                                           _i64, _vp, _i, _i64, _i, _vp, _vp, _vp, _vp, _sz, _i, _vp]),
+    "mfar_score_topk_e4m3_filtered": (_i, [_vp, _vp, _i64, _i, _i, _i, _i, _vp, _vp, _i, _vp, _vp, _i, _i, _i64, _i64,
+                                           _vp, _i, _i64, _i, _vp, _vp, _vp, _vp, _sz, _i, _vp]),
+    "mfar_score_topk_coo_e4m3_filtered": (_i, [_vp, _vp, _i64, _i, _i, _i, _i, _vp, _vp, _i, _vp, _vp, _vp, _i, _vp, _i,
+                                               _i64, _vp, _i, _i64, _i, _vp, _vp, _vp, _vp, _sz, _i, _vp]),
+    "mfar_score_topk_bm25_e4m3_filtered": (_i, [_vp, _vp, _i64, _i, _i, _i, _i, _vp, _vp, _i, _vp, _vp, _vp, _vp, _vp, _i,
+                                                _vp, _i64, _i64, _vp, _i, _i64, _i, _vp, _vp, _vp, _vp, _sz, _i, _vp]),
     "mfar_score_candidates_e4m3": (_i, [_vp, _vp, _i64, _i, _i, _i, _i, _vp, _vp, _i, _vp, _i, _vp, _vp]),
     "mfar_topk_merge": (_i, [_vp, _i, _i, _i, _i, _vp, _vp, _vp, _vp]),
     "mfar_exchange_buffer_bytes": (_sz, [_i, _i, _i]),

@@ -216,13 +216,17 @@ class ShardedRetriever:
         self._k = None
 
     @torch.no_grad()
-    def search(self, q_vecs, q_emb=None, sparse_local=None, top_k: Optional[int] = None, sparse_tokens=None):
+    def search(self, q_vecs, q_emb=None, sparse_local=None, top_k: Optional[int] = None, sparse_tokens=None,
+               doc_filter=None):
         """``sparse_local``: this shard's columns of the precomputed sparse scores; ``sparse_tokens``: the (replicated)
-        query tokens when the local retriever holds this shard's BM25 postings (``DeviceBM25.shard``)."""
+        query tokens when the local retriever holds this shard's BM25 postings (``DeviceBM25.shard``).
+        ``doc_filter``: the GLOBAL doc bitmap of ``MultiFieldRetriever.search`` (the same tensor on every rank: its
+        bits are indexed by global doc id, so each shard reads its own range)."""
         k = top_k or self.local.top_k
         k_local = min(k, self.local.n_docs)
+        extra = {} if doc_filter is None else {"doc_filter": doc_filter}
         _, _, keys = self.local.search(q_vecs, q_emb, sparse_local, top_k=k_local, return_keys=True,
-                                       sparse_tokens=sparse_tokens)
+                                       sparse_tokens=sparse_tokens, **extra)
         if k_local < k:                                   # tiny shard: pad with empty keys
             keys = torch.nn.functional.pad(keys, (0, k - k_local))
         if not dist.is_initialized() or dist.get_world_size(self.group) == 1:

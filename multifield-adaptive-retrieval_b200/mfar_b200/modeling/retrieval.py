@@ -285,12 +285,41 @@ class MultiFieldRetriever:
             cv = cv.float()
         return ck.contiguous(), cv.contiguous(), off
 
+    def _check_filter(self, doc_filter, Q: int) -> Optional[Tuple[torch.Tensor, int, int]]:
+        """(bitmap, rows, words per row) of a ``doc_filter`` argument, or None.  The bitmap is used in place (a
+        ``GraphedSearch`` replays with whatever it holds), so it must already be a contiguous device tensor."""
+        if doc_filter is None:
+            return None
+        dev = self.device                                  # "cuda" (no index) accepts the current device's tensors
+        if not torch.is_tensor(doc_filter) or doc_filter.device.type != dev.type or (
+                dev.index is not None and doc_filter.device.index != dev.index):
+            raise ValueError(f"doc_filter must be a tensor on {self.device}")
+        if doc_filter.dtype not in (torch.int32, torch.uint32):
+            raise ValueError(f"doc_filter must be int32 or uint32 (a bitmap over global doc ids), got {doc_filter.dtype}")
+        if doc_filter.dim() == 1:
+            rows = 1
+        elif doc_filter.dim() == 2 and doc_filter.shape[0] == Q:
+            rows = Q
+        else:
+            raise ValueError(f"doc_filter must be [W] (shared) or [{Q},W] (one row per query), "
+                             f"got {tuple(doc_filter.shape)}")
+        if not doc_filter.is_contiguous():
+            raise ValueError("doc_filter must be contiguous")
+        ld = int(doc_filter.shape[-1])
+        need = (self.doc_id_base + self.n_docs + 31) // 32
+        if ld < need:
+            raise ValueError(f"doc_filter rows hold {ld} words; docs [{self.doc_id_base}, "
+                             f"{self.doc_id_base + self.n_docs}) need {need}")
+        return doc_filter, rows, ld
+
     def _score_topk(self, q: Tuple[Optional[torch.Tensor], Optional[torch.Tensor]], w: torch.Tensor, sparse: tuple,
                     k: int, field_begin: int, n_dense: int, n_sparse: int, want_keys: bool = False,
-                    impl: Optional[str] = None, n_docs: Optional[int] = None, doc_id_base: Optional[int] = None):
+                    impl: Optional[str] = None, n_docs: Optional[int] = None, doc_id_base: Optional[int] = None,
+                    doc_filter: Optional[Tuple[torch.Tensor, int, int]] = None):
         """``q``: the query operand of ``_queries`` (rows, scales).  ``sparse``: the sparse fields' input in one of
         the layouts of the scoring entry points - ("rows", [Q,Fs,ld] tensor or None, dtype code),
-        ("coo", keys, vals, field_offsets) or ("bm25", int32 [n,3] token entries)."""
+        ("coo", keys, vals, field_offsets) or ("bm25", int32 [n,3] token entries).  ``doc_filter``: the output of
+        ``_check_filter`` - the call then runs the ``*_filtered`` twin."""
         Q = w.shape[0]
         n_docs = self.n_docs if n_docs is None else n_docs
         doc_id_base = self.doc_id_base if doc_id_base is None else doc_id_base
@@ -317,11 +346,16 @@ class MultiFieldRetriever:
         ws = self._workspace(Q, k, n_sparse, n_docs, n_entries)
         c = self.corpus
         e8 = c is not None and c.e4m3
-        name = "score_topk" if layout == "rows" else "score_topk_" + layout
-        fn = getattr(nv.lib(), f"mfar_{name}_e4m3" if e8 else f"mfar_{name}")
+        name = ("score_topk" if layout == "rows" else "score_topk_" + layout) + ("_e4m3" if e8 else "")
+        filt_args = ()
+        if doc_filter is not None:
+            name += "_filtered"
+            bits, rows, ld = doc_filter
+            filt_args = (nv.ptr(bits), rows, ld)
+        fn = getattr(nv.lib(), "mfar_" + name)
         nv.check(fn(*_operand(c.data if c else None, c.scales if c else None, e8), n_docs, c.n_fields if c else 0,
                     field_begin, n_dense, c.dim_pad if c else 0, *_operand(*q, e8), Q, nv.ptr(w), *sparse_args,
-                    doc_id_base, k, nv.ptr(keys), nv.ptr(scores), nv.ptr(ids), nv.ptr(ws), ws.numel(),
+                    doc_id_base, *filt_args, k, nv.ptr(keys), nv.ptr(scores), nv.ptr(ids), nv.ptr(ws), ws.numel(),
                     nv.IMPL[impl or self.impl], nv.stream()), name)
         self.last_launches = nv.lib().mfar_last_launch_count()
         return scores, ids, keys
@@ -366,7 +400,7 @@ class MultiFieldRetriever:
     @torch.no_grad()
     def search(self, q_vecs, q_emb: Optional[torch.Tensor] = None, sparse: Optional[torch.Tensor] = None,
                top_k: Optional[int] = None, return_keys: bool = False, impl: Optional[str] = None, sparse_coo=None,
-               sparse_tokens=None, batch: Optional[int] = None):
+               sparse_tokens=None, batch: Optional[int] = None, doc_filter: Optional[torch.Tensor] = None):
         """Exhaustive multi-field top-k.
 
         q_vecs [Q,dim]: query vectors for the dense dots (rounded to bf16);
@@ -384,6 +418,11 @@ class MultiFieldRetriever:
                         field j, or the prebuilt int32 [n,3] entry tensor of ``BM25FieldSet.entries`` - the sparse
                         fields are then scored on the device (bm25s ``get_scores``, index.py:72-76).
         batch          : number of queries, needed only for a sparse-only retriever fed with an entry tensor.
+        doc_filter     : restrict the top-k to eligible docs: an int32/uint32 device bitmap over GLOBAL doc ids (bit d
+                        of word d >> 5 set <=> doc d is eligible; ``data.bm25.safe_docs_bitmap`` builds one row), either
+                        one row [W] for every query or one row per query [Q,W], with 32*W >= doc_id_base + n_docs.
+                        Ineligible docs never enter the top-k, inside the scoring pass; a query with fewer than k
+                        eligible docs gets (-inf, -1) in the remaining slots.
         Returns (scores [Q,k] fp32, ids [Q,k] int64) sorted by (score desc, id asc), NaN scores first (as
         ``torch.topk`` ranks them), then +inf, finite, -inf; with
         return_keys also the packed uint64 keys (as int64) used for cross-shard merging."""
@@ -402,7 +441,8 @@ class MultiFieldRetriever:
         else:
             sp = ("rows", *self._check_sparse(sparse, Q))
         scores, ids, keys = self._score_topk((q_bf16, q_sc), w, sp, k, 0, self.n_dense, self.n_sparse,
-                                             want_keys=return_keys, impl=impl)
+                                             want_keys=return_keys, impl=impl,
+                                             doc_filter=self._check_filter(doc_filter, Q))
         return (scores, ids, keys) if return_keys else (scores, ids)
 
     # ------------------------------------------------------------------ field-masking sweep in one corpus pass
@@ -683,10 +723,13 @@ class GraphedSearch:
 
     def __init__(self, retriever: "MultiFieldRetriever", batch: int, sparse: str = "none", max_entries: int = 0,
                  top_k: Optional[int] = None, sparse_dtype=torch.float16, sparse_ld: Optional[int] = None,
-                 sharded=None, sparse_buffer: Optional[torch.Tensor] = None):
+                 sharded=None, sparse_buffer: Optional[torch.Tensor] = None,
+                 doc_filter: Optional[torch.Tensor] = None):
         """``sharded``: the ``mfar_b200.dist.ShardedRetriever`` wrapping ``retriever`` - the captured step then also holds
         the cross-GPU exchange + merge (its call counter lives in device memory, so the replayed launch is identical on
-        every call); every rank must construct and call its GraphedSearch the same number of times."""
+        every call); every rank must construct and call its GraphedSearch the same number of times.
+        ``doc_filter``: a bitmap as ``MultiFieldRetriever.search`` takes it, adopted as a static input (not copied):
+        every replay filters with its contents at that time, so the caller may rewrite them between replays."""
         r = self.r = retriever
         self.sharded = sharded
         dev = r.device
@@ -703,6 +746,9 @@ class GraphedSearch:
         E = r.mixture.weight.shape[0] if r.mixture.query_cond else 0
         self.q_emb = torch.zeros((self.Q, E), dtype=torch.float32, device=dev) if E else None
         self.sparse = self.entries = None
+        self.doc_filter = doc_filter
+        if doc_filter is not None:
+            r._check_filter(doc_filter, self.Q)            # fail here rather than inside the capture
         if sparse == "dense":
             if sparse_buffer is not None:                 # adopt the caller's [Q,Fs,ld] tensor as the static input: a
                 self.sparse = sparse_buffer               # corpus-sized score tensor is not copied per replay
@@ -732,9 +778,10 @@ class GraphedSearch:
 
     def _run(self):
         if self.sharded is not None:
-            return self.sharded.search(self.q_vecs, self.q_emb, self.sparse, top_k=self.k, sparse_tokens=self.entries)
+            return self.sharded.search(self.q_vecs, self.q_emb, self.sparse, top_k=self.k, sparse_tokens=self.entries,
+                                       doc_filter=self.doc_filter)
         return self.r.search(self.q_vecs, self.q_emb, self.sparse, top_k=self.k, sparse_tokens=self.entries,
-                             batch=self.Q)
+                             batch=self.Q, doc_filter=self.doc_filter)
 
     def __call__(self, q_vecs=None, q_emb=None, sparse=None, entries=None):
         if self.q_vecs is not None:
