@@ -36,58 +36,48 @@ static size_t seed_scratch_bytes(int Q, int k) {      // two [Q,k] key buffers (
   return 2 * align_up(size_t(Q) * k * 8, 256) + align_up(size_t(Q) * 8, 256);
 }
 
-struct Geometry {
-  int impl;       // resolved: MFAR_IMPL_SIMT, MFAR_IMPL_TCGEN05 or MFAR_IMPL_TCGEN05_QS
-  int workers;
-  int q_tiles;
-  int q_pad;      // per tile (tc, qs) or total (simt)
-  int q_pad_total;
-  int cg;         // qs: CTAs per MMA group (1 or 2)
-  int lists;      // candidate lists per query the scoring kernel fills (workers, or 2 x workers: qs single-field)
-  long long seg_docs;   // rows kernel: docs per segment
-};
-
-constexpr int kImplRows = 100;    // internal: sparse-only scorers (no dense field) -> streaming top-k of the base rows
-
 constexpr int kQsMinBatch = 65;   // AUTO: batches above 64 queries take the query-stationary kernel
 
 #ifdef MFAR_DEBUG_SEED
 static const unsigned long long* g_debug_seed = nullptr;
 #endif
 
-static Geometry resolve_geometry(const ScoreArgs& a, int impl) {
-  Geometry g{};
-  if (a.n_dense == 0) {                                        // every impl request: there is nothing to contract
-    g.impl = kImplRows;
-    g.cg = 1;
-    g.q_tiles = 1;
-    topk_rows_geometry(a.Q, a.n_docs, &g.workers, &g.seg_docs);
-    g.q_pad = g.q_pad_total = round_up(a.Q, 4);
-    g.lists = g.workers;
-    return g;
-  }
+// The pass `impl` asks for (AUTO resolved), planned for `a`.
+static PassPlan plan_pass(const ScoreArgs& a, int impl) {
+  if (a.n_dense == 0) return plan_topk_rows(a.Q, a.n_docs);   // every impl request: there is nothing to contract
   if (impl == MFAR_IMPL_AUTO) {
     if (a.Q >= kQsMinBatch && score_qs_supported(a)) impl = MFAR_IMPL_TCGEN05_QS;
     else impl = score_tc_supported(a) ? MFAR_IMPL_TCGEN05 : MFAR_IMPL_SIMT;
   }
-  g.impl = impl;
-  g.cg = 1;
-  if (impl == MFAR_IMPL_TCGEN05_QS) {
-    score_qs_geometry(a.Q, a.n_tiles, &g.q_tiles, &g.workers, &g.cg);
-    g.q_pad = 128;
-    g.q_pad_total = g.q_pad * g.q_tiles;
-    g.lists = g.workers * score_qs_lists_per_worker(a.n_dense, g.cg);
-    return g;
-  } else if (impl == MFAR_IMPL_TCGEN05) {
-    score_tc_geometry(a.Q, a.n_tiles, &g.q_pad, &g.q_tiles, &g.workers);
-    g.q_pad_total = g.q_pad * g.q_tiles;
-  } else {
-    score_simt_geometry(a.Q, a.n_tiles, &g.q_pad, &g.workers);
-    g.q_tiles = 1;
-    g.q_pad_total = g.q_pad;
+  if (impl == MFAR_IMPL_TCGEN05_QS) return plan_score_qs(a.Q, a.n_tiles, a.n_dense);
+  if (impl == MFAR_IMPL_TCGEN05) return plan_score_tc(a.Q, a.n_tiles);
+  return plan_score_simt(a.Q, a.n_tiles);
+}
+
+static size_t plan_workspace_bytes(const PassPlan& p) { return topk_workspace_bytes(p.lists, p.q_pad_total); }
+
+// One scoring pass: carves the candidate lists of `plan` from `workspace` into *ws (the merge reads the same carve),
+// zeroes the workspace tail and copies a.gthr_seed into the shared thresholds for the kinds that read them, and
+// launches the pass.  Counts every kernel it enqueued in t_last_launches.
+static int launch_pass(const ScoreArgs& a, const PassPlan& plan, void* workspace, cudaStream_t st,
+                       TopkWorkspace* ws) {
+  *ws = carve_workspace(workspace, plan.lists, plan.q_pad_total);
+  int launches = 0;
+  if (plan.impl != MFAR_IMPL_SIMT) {      // progress counters (score_qs lockstep), shared thresholds, pooled bounds
+    MFAR_CUDA_OK(cudaMemsetAsync(ws->progress, 0, workspace_zero_bytes(ws->workers, ws->q_pad), st));
+    if (a.gthr_seed) {
+      if (int rc = launch_seed_gthr(ws->gthr, a.gthr_seed, a.Q, st)) return rc;
+      ++launches;
+    }
   }
-  g.lists = g.workers;
-  return g;
+  int rc;
+  if (plan.impl == kImplRows) rc = launch_topk_rows(a, plan, *ws, st, &launches);
+  else if (plan.impl == MFAR_IMPL_TCGEN05_QS) rc = launch_score_qs(a, plan, *ws, st, &launches);
+  else if (plan.impl == MFAR_IMPL_TCGEN05) rc = launch_score_tc(a, plan, *ws, st, &launches);
+  else rc = launch_score_simt(a, plan, *ws, st, &launches);
+  if (rc) return rc;
+  t_last_launches += launches;
+  return MFAR_OK;
 }
 
 extern "C" {
@@ -179,28 +169,12 @@ int mfar_mixture_apply(const float* x, const float* w, int B, int S, int F, int 
 size_t mfar_score_topk_workspace_bytes(int Q, int k, int64_t n_docs, int n_sparse) {
   if (Q <= 0 || n_docs < 0) return 0;
   (void)k;
-  const int n_tiles = int((n_docs + kTileDocs - 1) / kTileDocs);
-  size_t best = 0;
-  {
-    int qp, qt, w;
-    score_tc_geometry(Q, std::max(n_tiles, 1), &qp, &qt, &w);
-    best = std::max(best, topk_workspace_bytes(w, qp * qt));
-  }
-  {
-    int qp, w;
-    score_simt_geometry(Q, std::max(n_tiles, 1), &qp, &w);
-    best = std::max(best, topk_workspace_bytes(w, qp));
-  }
-  if (n_sparse > 0) {
-    int segs; long long per;
-    topk_rows_geometry(Q, std::max<int64_t>(n_docs, 1), &segs, &per);
-    best = std::max(best, topk_workspace_bytes(segs, round_up(Q, 4)));
-  }
-  {
-    int qt, w, cg;
-    score_qs_geometry(Q, std::max(n_tiles, 1), &qt, &w, &cg);
-    best = std::max(best, topk_workspace_bytes(2 * w, qt * 128));   // single-field scorers keep 2 lists per CTA
-  }
+  const int n_tiles = std::max(int((n_docs + kTileDocs - 1) / kTileDocs), 1);
+  // the largest pass any call of this shape may plan; n_dense is not known here (plan_score_qs)
+  size_t best = std::max({plan_workspace_bytes(plan_score_tc(Q, n_tiles)),
+                          plan_workspace_bytes(plan_score_simt(Q, n_tiles)),
+                          plan_workspace_bytes(plan_score_qs(Q, n_tiles, 0))});
+  if (n_sparse > 0) best = std::max(best, plan_workspace_bytes(plan_topk_rows(Q, std::max<int64_t>(n_docs, 1))));
   size_t total = align_up(best, 256);
   if (n_sparse > 0) total += align_up(size_t(Q) * size_t(align_up(size_t(n_docs), kTileDocs)) * 4, 256);
   total += seed_scratch_bytes(Q, MFAR_MAX_K);         // threshold-seeding prefix pass
@@ -339,9 +313,9 @@ static int score_topk_core(ScoreArgs a, int64_t n_docs, int corpus_fields, int f
   }
   if (n_dense > 0 && impl == MFAR_IMPL_TCGEN05 && !score_tc_supported(a)) return MFAR_ERR_SHAPE;
   if (n_dense > 0 && impl == MFAR_IMPL_TCGEN05_QS && !score_qs_supported(a)) return MFAR_ERR_SHAPE;
-  const Geometry g = resolve_geometry(a, impl);
+  const PassPlan g = plan_pass(a, impl);
 
-  const size_t ws_topk = align_up(topk_workspace_bytes(g.lists, g.q_pad_total), 256);
+  const size_t ws_topk = align_up(plan_workspace_bytes(g), 256);
   const int64_t base_ld = int64_t(align_up(size_t(n_docs), kTileDocs));   // tile-wide vector reads stay in bounds
   // Dense [Q,Fs,ld] score rows are gathered and mixed INSIDE the tensor-core scoring epilogues (no [Q,N] intermediate
   // in HBM) when their rows are 32-byte aligned; COO pairs / BM25 postings scatter into the fp32 base block, and the
@@ -390,6 +364,7 @@ static int score_topk_core(ScoreArgs a, int64_t n_docs, int corpus_fields, int f
     a.base_ld = base_ld;
   }
   int rc;
+  TopkWorkspace ws;
   // Threshold seeding (tensor-core kernels, shards of >= 16 tiles per CTA): the same kernel first scores a PREFIX of one
   // tile per CTA, the merge ranks it, and the k-th best key of the prefix (a valid lower bound of the shard's k-th key)
   // becomes every query's initial admission threshold.  Without it every candidate list fills unfiltered and is
@@ -427,20 +402,17 @@ static int score_topk_core(ScoreArgs a, int64_t n_docs, int corpus_fields, int f
       ScoreArgs ap = a;                                 // `a` already starts behind the previous level
       ap.n_tiles = g.workers * level_tiles[lv];
       ap.n_docs = int64_t(ap.n_tiles) * kTileDocs;
-      const Geometry gp = resolve_geometry(ap, g.impl);
-      if (g.impl == MFAR_IMPL_TCGEN05_QS) rc = launch_score_qs(ap, workspace, gp.workers, gp.q_tiles, gp.cg, st);
-      else rc = launch_score_tc(ap, workspace, gp.workers, gp.q_tiles, gp.q_pad, st);
-      if (rc) return rc;
-      TopkWorkspace wp = carve_workspace(workspace, gp.lists, gp.q_pad_total);
+      const PassPlan gp = plan_pass(ap, g.impl);
+      if ((rc = launch_pass(ap, gp, workspace, st, &ws))) return rc;
       uint64_t* pref_keys = pref_buf[lv & 1];           // ranked top k of everything scored so far
-      rc = launch_merge(wp.cand_keys, wp.cand_cnt, wp.cand_thr, gp.lists, gp.q_pad_total, kCandCap, Q, k, pref_keys,
+      rc = launch_merge(ws.cand_keys, ws.cand_cnt, ws.cand_thr, ws.workers, ws.q_pad, kCandCap, Q, k, pref_keys,
                         nullptr, nullptr, st, prefix_keys, prefix_keys ? k : 0);
       if (rc) return rc;
       if ((rc = launch_seed_from_keys(pref_keys, Q, k, seed_thr, st))) return rc;
 #ifdef MFAR_DEBUG_SEED   // experiment builds only: replace the prefix seed by thresholds the caller supplies
       if (g_debug_seed) MFAR_CUDA_OK(cudaMemcpyAsync(seed_thr, g_debug_seed, size_t(Q) * 8, cudaMemcpyDeviceToDevice, st));
 #endif
-      t_last_launches += 4;                             // prefix scoring + merge + seed, and the copy into the next pass
+      t_last_launches += 2;                             // merge + seed
       // A prefix is not scored twice: the next pass starts behind it and the next merge takes the prefix's ranked top
       // k as one more list.
       skip_tiles(a, ap.n_tiles);
@@ -448,20 +420,9 @@ static int score_topk_core(ScoreArgs a, int64_t n_docs, int corpus_fields, int f
       prefix_keys = pref_keys;
     }
   }
-  if (g.impl == kImplRows)
-    rc = launch_topk_rows(a, workspace, g.workers, g.seg_docs, st);
-  else if (g.impl == MFAR_IMPL_TCGEN05_QS)
-    rc = launch_score_qs(a, workspace, g.workers, g.q_tiles, g.cg, st);
-  else if (g.impl == MFAR_IMPL_TCGEN05)
-    rc = launch_score_tc(a, workspace, g.workers, g.q_tiles, g.q_pad, st);
-  else
-    rc = launch_score_simt(a, workspace, g.workers, g.q_pad, st);
-  if (rc) return rc;
+  if ((rc = launch_pass(a, g, workspace, st, &ws))) return rc;
   if (prof) { MFAR_CUDA_OK(cudaEventRecord(g_prof_ev[g_prof_n][1], st)); ++g_prof_n; }
-  ++t_last_launches;
-  if (g.impl == kImplRows && n_docs >= 4096) ++t_last_launches;   // + the threshold-seed kernel
-  TopkWorkspace ws = carve_workspace(workspace, g.lists, g.q_pad_total);
-  rc = launch_merge(ws.cand_keys, ws.cand_cnt, ws.cand_thr, g.lists, g.q_pad_total, kCandCap, Q, k, out_keys,
+  rc = launch_merge(ws.cand_keys, ws.cand_cnt, ws.cand_thr, ws.workers, ws.q_pad, kCandCap, Q, k, out_keys,
                     out_scores, out_ids, st, prefix_keys, prefix_keys ? k : 0);
   if (rc) return rc;
   ++t_last_launches;

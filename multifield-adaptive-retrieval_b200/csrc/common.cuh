@@ -111,7 +111,7 @@ __device__ __forceinline__ uint32_t filter_bits32(const uint32_t* row, int words
 // Workspace carve-up shared by the scoring kernels and the merge.
 //   cand_keys [G][Qp][kCandCap] u64 | cand_thr [G][Qp] u64 | cand_cnt [G][Qp] i32 | err flag (256 B) |
 //   progress counters (kProgressInts i32) | gthr [Qp] u64 | pool [G][Qp] u64
-//   (the tail from the progress counters on is zeroed by the scoring-kernel launcher)
+//   (the tail from the progress counters on is zeroed before every scoring pass that reads it)
 // gthr[q] = best admission threshold any CTA has established for query q (atomicMax of a k-th key).  The k-th key
 // of ANY subset of the shard is a lower bound of the shard's k-th key, so every CTA may filter with it: the
 // admitted-candidate count (and with it the list compactions) drops from k*ln(N_cta/k) per CTA to ~that in total.

@@ -117,25 +117,47 @@ struct ScoreArgs {
   int filter_words;              // ceil((doc_id_base + n_docs) / 32): the words of a row that hold docs of the shard
 };
 
-// gthr[q] = seed[q] (after the launcher zeroed the workspace tail)
+// gthr[q] = seed[q] (after the workspace tail was zeroed)
 int launch_seed_gthr(unsigned long long* gthr, const unsigned long long* seed, int Q, cudaStream_t st);
 // seed[q] = keys[q, k-1] - 1 (the k-th best key of a prefix, made exclusive), 0 when the prefix holds fewer than k docs
 int launch_seed_from_keys(const uint64_t* keys, int Q, int k, unsigned long long* seed, cudaStream_t st);
 
-// SIMT (CUDA-core) scoring pass.  workers = grid size; fills ws candidate lists.
-int launch_score_simt(const ScoreArgs& a, void* ws_base, int workers, int q_pad, cudaStream_t st);
+constexpr int kImplRows = 100;    // pass kind of sparse-only scorers (no dense field): streaming top-k of the base rows
+
+// One scoring pass's launch geometry and candidate-list layout, filled completely by its kind's plan_* function.  The
+// workspace is carved for (lists, q_pad_total) once per pass: the kernel writes its lists there and the merge reads them.
+struct PassPlan {
+  int impl;           // MFAR_IMPL_SIMT, MFAR_IMPL_TCGEN05, MFAR_IMPL_TCGEN05_QS or kImplRows
+  int workers;        // doc-side grid size (rows: segments per query)
+  int q_tiles;
+  int q_pad;          // queries per tile (tc, qs), or all queries padded (simt, rows)
+  int q_pad_total;    // q_pad * q_tiles
+  int cg;             // qs: CTAs per MMA group (1 or 2)
+  int lists;          // candidate lists per query: workers, or 2 x workers (qs: two epilogue sets)
+  long long seg_docs; // rows: docs per segment
+};
+PassPlan plan_score_simt(int Q, int n_tiles);
+PassPlan plan_score_tc(int Q, int n_tiles);
+PassPlan plan_score_qs(int Q, int n_tiles, int n_dense);
+PassPlan plan_topk_rows(int Q, long long n_docs);
+
+// The scoring passes.  Each fills the candidate lists of `ws` (carved from `plan`, its tail zeroed and seeded by the
+// caller where the kind reads it) and adds the kernels it enqueued to *launches.
+struct TopkWorkspace;
+// SIMT (CUDA-core) scoring pass.
+int launch_score_simt(const ScoreArgs& a, const PassPlan& plan, const TopkWorkspace& ws, cudaStream_t st,
+                      int* launches);
 // TMA + tcgen05 scoring pass.
-int launch_score_tc(const ScoreArgs& a, void* ws_base, int workers, int q_tiles, int q_pad, cudaStream_t st);
+int launch_score_tc(const ScoreArgs& a, const PassPlan& plan, const TopkWorkspace& ws, cudaStream_t st,
+                    int* launches);
 // Query-stationary tcgen05 pass for large batches (queries resident in TMEM, CTA pairs when cg == 2).
-int launch_score_qs(const ScoreArgs& a, void* ws_base, int workers, int q_tiles, int cg, cudaStream_t st);
+int launch_score_qs(const ScoreArgs& a, const PassPlan& plan, const TopkWorkspace& ws, cudaStream_t st,
+                    int* launches);
+// Streaming top-k of the pre-mixed fp32 score rows (sparse-only scorers: no dense field).
+int launch_topk_rows(const ScoreArgs& a, const PassPlan& plan, const TopkWorkspace& ws, cudaStream_t st,
+                     int* launches);
 long long qs_cluster4_ctas_collect();   // CTAs that ran in 4-CTA clusters since the last call (resets); -1: CUDA error
 bool score_qs_supported(const ScoreArgs& a);
-void score_qs_geometry(int Q, int n_tiles, int* q_tiles, int* workers, int* cg);
-// candidate lists per (worker CTA, query): 2 for a single-field scorer in CTA-pair mode (two epilogue sets), else 1
-int score_qs_lists_per_worker(int n_dense, int cg);
-// Streaming top-k of the pre-mixed fp32 score rows (sparse-only scorers: no dense field).
-void topk_rows_geometry(int Q, long long n_docs, int* segments, long long* seg_docs);
-int launch_topk_rows(const ScoreArgs& a, void* ws_base, int segments, long long seg_docs, cudaStream_t st);
 // rows of a dense sparse-score tensor can be gathered by the scoring epilogues (32-byte vector loads)
 inline bool sparse_rows_fusable(const void* sparse, int dtype, int64_t ld) {
   const int es = dtype == MFAR_F32 ? 4 : 2;
@@ -144,8 +166,5 @@ inline bool sparse_rows_fusable(const void* sparse, int dtype, int64_t ld) {
 }
 // Shape envelope of the tcgen05 path.
 bool score_tc_supported(const ScoreArgs& a);
-// geometry chosen for (Q): q_pad per tile, number of q tiles, workers
-void score_tc_geometry(int Q, int n_tiles, int* q_pad, int* q_tiles, int* workers);
-void score_simt_geometry(int Q, int n_tiles, int* q_pad, int* workers);
 
 }  // namespace mfar

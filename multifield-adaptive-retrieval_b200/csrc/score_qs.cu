@@ -645,14 +645,24 @@ bool score_qs_supported(const ScoreArgs& a) {
          int64_t(a.n_tiles) * a.corpus_fields * kTileDocs < (int64_t(1) << 31);
 }
 
-void score_qs_geometry(int Q, int n_tiles, int* q_tiles, int* workers, int* cg) {
-  int qt = (Q + kQsQ - 1) / kQsQ;
-  const int c = qt >= 2 ? 2 : 1;
-  qt = round_up(qt, c);
-  int w = kNumSmsB200 / qt;
+// n_dense = 0 plans the reservation of mfar_score_topk_workspace_bytes, which does not know n_dense: two lists per
+// worker at every batch size
+PassPlan plan_score_qs(int Q, int n_tiles, int n_dense) {
+  PassPlan p{};
+  p.impl = MFAR_IMPL_TCGEN05_QS;
+  const int qt = (Q + kQsQ - 1) / kQsQ;
+  p.cg = qt >= 2 ? 2 : 1;
+  p.q_tiles = round_up(qt, p.cg);
+  p.q_pad = kQsQ;
+  p.q_pad_total = p.q_pad * p.q_tiles;
+  int w = kNumSmsB200 / p.q_tiles;
   if (w > n_tiles) w = n_tiles;
   if (w < 1) w = 1;
-  *q_tiles = qt; *workers = w; *cg = c;
+  p.workers = w;
+  // two epilogue sets, each with its own lists, only where the epilogue is the bound: single-field scorers in CTA-pair
+  // mode (Q > 128); at Q <= 128 the kernel is HBM-bound and the extra warps measured ~3 % slower
+  p.lists = (n_dense == 0 || (n_dense == 1 && p.cg == 2)) ? 2 * w : w;
+  return p;
 }
 
 static size_t qs_smem_bytes(int n_weights, int stages, int stage_bytes, int sp_slots) {
@@ -660,12 +670,8 @@ static size_t qs_smem_bytes(int n_weights, int stages, int stage_bytes, int sp_s
          (2 * stages + 4 + 2 * kSpMaxSlots) * 8 + 16;
 }
 
-// two epilogue sets only where the epilogue is the bound: single-field scorers in CTA-pair mode (Q > 128); at
-// Q <= 128 the kernel is HBM-bound and the extra warps measured ~3 % slower
-int score_qs_lists_per_worker(int n_dense, int cg) { return (n_dense == 1 && cg == 2) ? 2 : 1; }
-
 template <int CG, int ES, bool SP, bool FILT>
-static int launch_qs_impl(const ScoreArgs& a, void* ws_base, int workers, int q_tiles, cudaStream_t st) {
+static int launch_qs_impl(const ScoreArgs& a, const PassPlan& plan, const TopkWorkspace& ws, cudaStream_t st) {
   constexpr int kChunkBytes = (kQsDocs / CG) * kChunkK * 2;
   QsParams p;
   p.n_docs = a.n_docs; p.n_tiles = a.n_tiles; p.corpus_fields = a.corpus_fields; p.field_begin = a.field_begin;
@@ -674,9 +680,8 @@ static int launch_qs_impl(const ScoreArgs& a, void* ws_base, int workers, int q_
   p.doc_id_base = a.doc_id_base; p.k = a.k;
   p.sparse = a.sparse; p.sparse_ld = a.sparse_ld; p.n_sparse = a.sparse ? a.n_sparse : 0;
   p.sparse_f16 = a.sparse_dtype == MFAR_F16;
-  if (a.sparse && (a.base || !sparse_rows_fusable(a.sparse, a.sparse_dtype, a.sparse_ld))) return MFAR_ERR_ARG;
   const int n_w = a.n_dense + p.n_sparse;
-  p.ws = carve_workspace(ws_base, workers * ES, q_tiles * kQsQ);   // ES candidate lists per (CTA, query)
+  p.ws = ws;
   p.filt = DocFilter{a.filter_bits, a.filter_stride, a.filter_words};
   const size_t smem_cap = 227 * 1024;
   // Shared memory: corpus ring + (SP) sparse ring of 16 KB slots + weights + barriers.  The corpus ring is split in two
@@ -710,7 +715,7 @@ static int launch_qs_impl(const ScoreArgs& a, void* ws_base, int workers, int q_
   // of one worker column) and a stage splits into two K halves: each doc tile then crosses from L2 to the SMs once per
   // column instead of once per pair.  A preferred cluster, not a required one: GPCs with no room for 4 CTAs get
   // 2-CTA clusters, so every SM stays busy.
-  const bool cluster4 = CG == 2 && q_tiles % 4 == 0 && kc % 2 == 0;
+  const bool cluster4 = CG == 2 && plan.q_tiles % 4 == 0 && kc % 2 == 0;
   const uint64_t corpus_rows = uint64_t(a.n_tiles) * a.corpus_fields * kTileDocs;
   CUtensorMap map_b;
   int rc = make_tensor_map_kchunked(&map_b, a.corpus, corpus_rows, a.dim, kQsDocs / CG, kc,
@@ -733,11 +738,8 @@ static int launch_qs_impl(const ScoreArgs& a, void* ws_base, int workers, int q_
   MFAR_CUDA_OK(attr_once.run([&] {
     return cudaFuncSetAttribute(score_qs_kernel<CG, ES, SP, FILT>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem_cap));
   }));
-  // lockstep counters of the query groups (producer warp) + shared per-query thresholds (epilogue)
-  MFAR_CUDA_OK(cudaMemsetAsync(p.ws.progress, 0, workspace_zero_bytes(p.ws.workers, p.ws.q_pad), st));
-  if (a.gthr_seed) { if (int rc2 = launch_seed_gthr(p.ws.gthr, a.gthr_seed, a.Q, st)) return rc2; }
   cudaLaunchConfig_t cfg{};
-  cfg.gridDim = dim3(q_tiles, workers);
+  cfg.gridDim = dim3(plan.q_tiles, plan.workers);
   cfg.blockDim = dim3(qs_threads(ES, SP));
   cfg.dynamicSmemBytes = smem;
   cfg.stream = st;
@@ -762,22 +764,20 @@ long long qs_cluster4_ctas_collect() {
 }
 
 template <bool FILT>
-static int launch_qs_filt(const ScoreArgs& a, void* ws_base, int workers, int q_tiles, int cg, cudaStream_t st) {
+static int launch_qs_filt(const ScoreArgs& a, const PassPlan& plan, const TopkWorkspace& ws, cudaStream_t st) {
   const bool sp = a.sparse != nullptr;
-  if (score_qs_lists_per_worker(a.n_dense, cg) == 2)
-    return sp ? launch_qs_impl<2, 2, true, FILT>(a, ws_base, workers, q_tiles, st)
-              : launch_qs_impl<2, 2, false, FILT>(a, ws_base, workers, q_tiles, st);
-  if (cg == 2)
-    return sp ? launch_qs_impl<2, 1, true, FILT>(a, ws_base, workers, q_tiles, st)
-              : launch_qs_impl<2, 1, false, FILT>(a, ws_base, workers, q_tiles, st);
-  return sp ? launch_qs_impl<1, 1, true, FILT>(a, ws_base, workers, q_tiles, st)
-            : launch_qs_impl<1, 1, false, FILT>(a, ws_base, workers, q_tiles, st);
+  if (plan.lists == 2 * plan.workers)               // two epilogue sets (CTA pairs only)
+    return sp ? launch_qs_impl<2, 2, true, FILT>(a, plan, ws, st) : launch_qs_impl<2, 2, false, FILT>(a, plan, ws, st);
+  if (plan.cg == 2)
+    return sp ? launch_qs_impl<2, 1, true, FILT>(a, plan, ws, st) : launch_qs_impl<2, 1, false, FILT>(a, plan, ws, st);
+  return sp ? launch_qs_impl<1, 1, true, FILT>(a, plan, ws, st) : launch_qs_impl<1, 1, false, FILT>(a, plan, ws, st);
 }
 
-int launch_score_qs(const ScoreArgs& a, void* ws_base, int workers, int q_tiles, int cg, cudaStream_t st) {
-  if (!score_qs_supported(a)) return MFAR_ERR_SHAPE;
-  return a.filter_bits ? launch_qs_filt<true>(a, ws_base, workers, q_tiles, cg, st)
-                       : launch_qs_filt<false>(a, ws_base, workers, q_tiles, cg, st);
+int launch_score_qs(const ScoreArgs& a, const PassPlan& plan, const TopkWorkspace& ws, cudaStream_t st,
+                    int* launches) {
+  const int rc = a.filter_bits ? launch_qs_filt<true>(a, plan, ws, st) : launch_qs_filt<false>(a, plan, ws, st);
+  if (rc == MFAR_OK) ++*launches;
+  return rc;
 }
 
 }  // namespace mfar

@@ -209,12 +209,16 @@ __global__ void __launch_bounds__(kSimtThreads) score_simt_kernel(SimtParams p) 
   }
 }
 
-void score_simt_geometry(int Q, int n_tiles, int* q_pad, int* workers) {
-  *q_pad = round_up(Q, 4);
+PassPlan plan_score_simt(int Q, int n_tiles) {
+  PassPlan p{};
+  p.impl = MFAR_IMPL_SIMT;
+  p.q_tiles = p.cg = 1;
+  p.q_pad = p.q_pad_total = round_up(Q, 4);
   int w = (Q <= 8) ? kNumSmsB200 * 4 : kNumSmsB200;   // bounded so the candidate workspace stays small
   if (w > n_tiles) w = n_tiles;
   if (w < 1) w = 1;
-  *workers = w;
+  p.workers = p.lists = w;
+  return p;
 }
 
 template <bool E8, bool FILT>
@@ -228,24 +232,25 @@ static void launch_simt_qb(const SimtParams& p, int Q, int n_dense, int workers,
   }
 }
 
-int launch_score_simt(const ScoreArgs& a, void* ws_base, int workers, int q_pad, cudaStream_t st) {
+int launch_score_simt(const ScoreArgs& a, const PassPlan& plan, const TopkWorkspace& ws, cudaStream_t st,
+                      int* launches) {
   if (a.dim % 8 != 0 || a.dim > kSimtMaxVec * 32 * 8) return MFAR_ERR_SHAPE;
   const bool e8 = a.corpus_dtype == MFAR_E4M3;
-  if (e8 && a.n_dense > 0 && (!a.corpus_scales || !a.q_scales || reinterpret_cast<uintptr_t>(a.corpus) % 8 ||
-                             reinterpret_cast<uintptr_t>(a.q_vecs) % 8))
+  if (e8 && (reinterpret_cast<uintptr_t>(a.corpus) % 8 || reinterpret_cast<uintptr_t>(a.q_vecs) % 8))
     return MFAR_ERR_ARG;
   SimtParams p;
   p.corpus = a.corpus; p.corpus_scales = a.corpus_scales; p.q_scales = a.q_scales;
   p.n_docs = a.n_docs; p.n_tiles = a.n_tiles; p.corpus_fields = a.corpus_fields; p.field_begin = a.field_begin;
   p.n_dense = a.n_dense; p.dim = a.dim; p.q_vecs = a.q_vecs; p.Q = a.Q;
   p.w = a.w; p.w_ld = a.w_ld; p.base = a.base; p.base_ld = a.base_ld; p.doc_id_base = a.doc_id_base; p.k = a.k;
-  p.ws = carve_workspace(ws_base, workers, q_pad);
+  p.ws = ws;
   p.filt = DocFilter{a.filter_bits, a.filter_stride, a.filter_words};
   const bool f = a.filter_bits != nullptr;
   auto launch = e8 ? (f ? launch_simt_qb<true, true> : launch_simt_qb<true, false>)
                    : (f ? launch_simt_qb<false, true> : launch_simt_qb<false, false>);
-  launch(p, a.Q, a.n_dense, workers, st);
+  launch(p, a.Q, a.n_dense, plan.workers, st);
   MFAR_CUDA_OK(cudaGetLastError());
+  ++*launches;
   return MFAR_OK;
 }
 

@@ -465,14 +465,19 @@ bool score_tc_supported(const ScoreArgs& a) {
          int64_t(a.n_tiles) * a.corpus_fields * kTileDocs < (int64_t(1) << 31);
 }
 
-void score_tc_geometry(int Q, int n_tiles, int* q_pad, int* q_tiles, int* workers) {
-  int qp = Q <= 16 ? 16 : (Q <= 32 ? 32 : 64);
-  int qt = (Q + qp - 1) / qp;
-  int w = kNumSmsB200 / qt;
+PassPlan plan_score_tc(int Q, int n_tiles) {
+  PassPlan p{};
+  p.impl = MFAR_IMPL_TCGEN05;
+  p.q_pad = Q <= 16 ? 16 : (Q <= 32 ? 32 : 64);
+  p.q_tiles = (Q + p.q_pad - 1) / p.q_pad;
+  p.q_pad_total = p.q_pad * p.q_tiles;
+  int w = kNumSmsB200 / p.q_tiles;
   if (w < 1) w = 1;
   if (w > n_tiles) w = n_tiles;
   if (w < 1) w = 1;
-  *q_pad = qp; *q_tiles = qt; *workers = w;
+  p.workers = p.lists = w;
+  p.cg = 1;
+  return p;
 }
 
 // n_weights: rows of [QP] floats next to the weights (E8: + the query scales); filt: two tiles of filter words
@@ -483,7 +488,7 @@ static size_t tc_smem_bytes(int qp, int n_weights, bool sparse, int k_chunks, in
 }
 
 template <int QP, bool SP, bool E8, bool FILT>
-static int launch_tc_impl(const ScoreArgs& a, void* ws_base, int workers, int q_tiles, cudaStream_t st) {
+static int launch_tc_impl(const ScoreArgs& a, const PassPlan& plan, const TopkWorkspace& ws, cudaStream_t st) {
   TcParams p;
   p.n_docs = a.n_docs; p.n_tiles = a.n_tiles; p.corpus_fields = a.corpus_fields; p.field_begin = a.field_begin;
   p.n_dense = a.n_dense; p.k_chunks = a.dim / (E8 ? kChunkK8 : kChunkK);
@@ -492,9 +497,8 @@ static int launch_tc_impl(const ScoreArgs& a, void* ws_base, int workers, int q_
   p.sparse = a.sparse; p.sparse_ld = a.sparse_ld; p.n_sparse = a.sparse ? a.n_sparse : 0;
   p.sparse_cols = a.sparse_cols ? a.sparse_cols : a.sparse_ld;
   p.sparse_f16 = a.sparse_dtype == MFAR_F16;
-  if (a.sparse && (a.base || !sparse_rows_fusable(a.sparse, a.sparse_dtype, a.sparse_ld))) return MFAR_ERR_ARG;
   const int n_w = a.n_dense + p.n_sparse + (E8 ? 1 : 0);
-  p.ws = carve_workspace(ws_base, workers, q_tiles * QP);
+  p.ws = ws;
   p.filt = DocFilter{a.filter_bits, a.filter_stride, a.filter_words};
   int stages = 8;
   const size_t smem_cap = 227 * 1024;
@@ -514,36 +518,34 @@ static int launch_tc_impl(const ScoreArgs& a, void* ws_base, int workers, int q_
   MFAR_CUDA_OK(attr_once.run([&] {
     return cudaFuncSetAttribute(score_tc_kernel<QP, SP, E8, FILT>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem_cap));
   }));
-  MFAR_CUDA_OK(cudaMemsetAsync(p.ws.progress, 0, workspace_zero_bytes(p.ws.workers, p.ws.q_pad), st));   // shared thresholds
-  if (a.gthr_seed) { if (int rc2 = launch_seed_gthr(p.ws.gthr, a.gthr_seed, a.Q, st)) return rc2; }
-  dim3 grid(workers, q_tiles);
+  dim3 grid(plan.workers, plan.q_tiles);
   score_tc_kernel<QP, SP, E8, FILT><<<grid, SP ? kTcThreads + kStagerThreads : kTcThreads, smem, st>>>(map_a, map_b, p);
   MFAR_CUDA_OK(cudaGetLastError());
   return MFAR_OK;
 }
 
 template <bool E8, bool FILT>
-static int launch_tc_qp(const ScoreArgs& a, void* ws_base, int workers, int q_tiles, int q_pad, cudaStream_t st) {
-  switch (q_pad) {
-    case 16: return a.sparse ? launch_tc_impl<16, true, E8, FILT>(a, ws_base, workers, q_tiles, st)
-                             : launch_tc_impl<16, false, E8, FILT>(a, ws_base, workers, q_tiles, st);
-    case 32: return a.sparse ? launch_tc_impl<32, true, E8, FILT>(a, ws_base, workers, q_tiles, st)
-                             : launch_tc_impl<32, false, E8, FILT>(a, ws_base, workers, q_tiles, st);
-    case 64: return a.sparse ? launch_tc_impl<64, true, E8, FILT>(a, ws_base, workers, q_tiles, st)
-                             : launch_tc_impl<64, false, E8, FILT>(a, ws_base, workers, q_tiles, st);
+static int launch_tc_qp(const ScoreArgs& a, const PassPlan& plan, const TopkWorkspace& ws, cudaStream_t st) {
+  switch (plan.q_pad) {
+    case 16: return a.sparse ? launch_tc_impl<16, true, E8, FILT>(a, plan, ws, st)
+                             : launch_tc_impl<16, false, E8, FILT>(a, plan, ws, st);
+    case 32: return a.sparse ? launch_tc_impl<32, true, E8, FILT>(a, plan, ws, st)
+                             : launch_tc_impl<32, false, E8, FILT>(a, plan, ws, st);
+    case 64: return a.sparse ? launch_tc_impl<64, true, E8, FILT>(a, plan, ws, st)
+                             : launch_tc_impl<64, false, E8, FILT>(a, plan, ws, st);
     default: return MFAR_ERR_SHAPE;
   }
 }
 
-int launch_score_tc(const ScoreArgs& a, void* ws_base, int workers, int q_tiles, int q_pad, cudaStream_t st) {
-  if (!score_tc_supported(a)) return MFAR_ERR_SHAPE;
-  if (a.corpus_dtype == MFAR_E4M3) {
-    if (!a.corpus_scales || !a.q_scales) return MFAR_ERR_ARG;
-    return a.filter_bits ? launch_tc_qp<true, true>(a, ws_base, workers, q_tiles, q_pad, st)
-                         : launch_tc_qp<true, false>(a, ws_base, workers, q_tiles, q_pad, st);
-  }
-  return a.filter_bits ? launch_tc_qp<false, true>(a, ws_base, workers, q_tiles, q_pad, st)
-                       : launch_tc_qp<false, false>(a, ws_base, workers, q_tiles, q_pad, st);
+int launch_score_tc(const ScoreArgs& a, const PassPlan& plan, const TopkWorkspace& ws, cudaStream_t st,
+                    int* launches) {
+  int rc;
+  if (a.corpus_dtype == MFAR_E4M3)
+    rc = a.filter_bits ? launch_tc_qp<true, true>(a, plan, ws, st) : launch_tc_qp<true, false>(a, plan, ws, st);
+  else
+    rc = a.filter_bits ? launch_tc_qp<false, true>(a, plan, ws, st) : launch_tc_qp<false, false>(a, plan, ws, st);
+  if (rc == MFAR_OK) ++*launches;
+  return rc;
 }
 
 }  // namespace mfar

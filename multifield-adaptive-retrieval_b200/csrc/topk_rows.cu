@@ -156,7 +156,7 @@ topk_rows_kernel(const float* __restrict__ base, long long base_ld, long long n_
 }
 
 // segments per row: enough warps to fill the machine (148 SMs x 64 warps), at least 2048 docs each
-void topk_rows_geometry(int Q, long long n_docs, int* segments, long long* seg_docs) {
+PassPlan plan_topk_rows(int Q, long long n_docs) {
   long long want = (long long)kNumSmsB200 * 64 / (Q > 0 ? Q : 1);
   if (want < 1) want = 1;
   long long cap = (n_docs + 2047) / 2048;
@@ -166,26 +166,32 @@ void topk_rows_geometry(int Q, long long n_docs, int* segments, long long* seg_d
   long long per = (n_docs + s - 1) / s;
   per = (per + kRowsStepDocs - 1) / kRowsStepDocs * kRowsStepDocs;     // whole steps: 16-byte aligned segment starts
   s = (n_docs + per - 1) / per;
-  *segments = int(s < 1 ? 1 : s);
-  *seg_docs = per;
+  PassPlan p{};
+  p.impl = kImplRows;
+  p.workers = p.lists = int(s < 1 ? 1 : s);
+  p.seg_docs = per;
+  p.q_tiles = p.cg = 1;
+  p.q_pad = p.q_pad_total = round_up(Q, 4);
+  return p;
 }
 
-int launch_topk_rows(const ScoreArgs& a, void* ws_base, int segments, long long seg_docs, cudaStream_t st) {
+int launch_topk_rows(const ScoreArgs& a, const PassPlan& plan, const TopkWorkspace& ws, cudaStream_t st,
+                     int* launches) {
   if (!a.base || a.base_ld % 4 != 0 || reinterpret_cast<uintptr_t>(a.base) % 16 != 0) return MFAR_ERR_ARG;
-  TopkWorkspace ws = carve_workspace(ws_base, segments, round_up(a.Q, 4));
-  MFAR_CUDA_OK(cudaMemsetAsync(ws.progress, 0, workspace_zero_bytes(ws.workers, ws.q_pad), st));   // gthr
   const DocFilter filt{a.filter_bits, a.filter_stride, a.filter_words};
   const bool f = filt.bits != nullptr;
-  if (a.n_docs >= 4096) {                                  // tiny shards: a few steps per warp, nothing to seed
+  const bool seeded = a.n_docs >= 4096;                    // tiny shards: a few steps per warp, nothing to seed
+  if (seeded) {
     auto seed = f ? topk_rows_seed_kernel<true> : topk_rows_seed_kernel<false>;
     seed<<<a.Q, kSeedThreads, 0, st>>>(a.base, a.base_ld, a.n_docs, a.k, ws.gthr, a.doc_id_base, filt);
   }
-  const long long tasks = (long long)segments * a.Q;
+  const long long tasks = (long long)plan.workers * a.Q;
   const unsigned blocks = unsigned((tasks + kRowsWarps - 1) / kRowsWarps);
   auto rows = f ? topk_rows_kernel<true> : topk_rows_kernel<false>;
-  rows<<<blocks, kRowsWarps * 32, 0, st>>>(a.base, a.base_ld, a.n_docs, a.Q, segments, seg_docs, a.doc_id_base, a.k,
-                                           ws, filt);
+  rows<<<blocks, kRowsWarps * 32, 0, st>>>(a.base, a.base_ld, a.n_docs, a.Q, plan.workers, plan.seg_docs,
+                                           a.doc_id_base, a.k, ws, filt);
   MFAR_CUDA_OK(cudaGetLastError());
+  *launches += seeded ? 2 : 1;
   return MFAR_OK;
 }
 
